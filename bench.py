@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — CSTR env-steps/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--math strict|fast]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--math strict|fast] [--dump-outputs DIR]
 
 Workload at N=1 = BASELINE.json configs[1]: "TwoSeriesCSTR step-only, 65,536 batched envs, random
 actions, fp32", one *step* = one pass of the hot path over one batch = ONE launch of the tape kernel
@@ -26,6 +26,9 @@ Keys beyond the base contract:
                BCQ / MADDPG update timings) — reported, not the headline; N=1 only.
   config / run `config` is the workload and is the same dictionary in both arms; `run` holds what varies with the run (math flavour,
                per-rank times, host placement).
+
+--dump-outputs DIR writes what the last timed step returned (rewards, dones, final state, step and episode counters) for a fixed, seeded
+sample of 8,192 reactors over all ranks as DIR/<name>.npy: all inputs are seeded, so two builds can be compared output for output.
 
 Order: headline -> e2e -> cpu_baseline -> [hard stop armed] rollout / dp_update -> extras -> the ONE JSON line.  The optional sections
 run under a hard stop (CSTR_BENCH_SECTION_LIMIT_S, default 300 s): if one of them hangs, rank 0 prints the line it already has (plus
@@ -99,10 +102,18 @@ def bind_to_gpu_numa_node(torch, local_rank: int) -> dict:
     return info
 
 
+FAILED_SECTIONS = []  # the exceptions of failed sections, kept until the process leaves (describe_error)
+
+
 def describe_error(exc: BaseException) -> str:
-    """repr(exc) plus the innermost frames, so that an error key in the JSON line says where it happened."""
+    """repr(exc) plus the innermost frames, so that an error key in the JSON line says where it happened.  The exception is kept in
+    FAILED_SECTIONS: its traceback holds the failed section's frames and with them its tensors.  Dropping it would free them, and after a
+    device error that free can abort the process (a pinned host buffer used in a non_blocking copy records a CUDA event when it is freed;
+    with the error pending the record throws inside a destructor) before the JSON line is printed.  run_ours leaves through os._exit once
+    a section has failed, so they are never freed."""
     import traceback
 
+    FAILED_SECTIONS.append(exc)
     frames = traceback.extract_tb(exc.__traceback__)[-3:]
     return repr(exc) + " @ " + " <- ".join(f"{os.path.basename(f.filename)}:{f.lineno}" for f in reversed(frames))
 
@@ -216,8 +227,8 @@ def cpu_port_rate(n_envs: int, target_seconds: float, seed: int = 0):
 
 
 def reference_python_rates(budget_s: float = 24.0) -> dict:
-    """The UNMODIFIED reference (pure Python) timed on this box's host cores, when its tree is staged (oracle/refload.py: /root/reference in
-    the build container, the git-ignored baseline/_ref on a GPU box): BASELINE.md §3's C1 / C2 / C4 / C5.  Reported beside the C port, never
+    """The UNMODIFIED reference (pure Python) timed on this box's host cores, when its tree is available (oracle/refload.py: CSTR_REFERENCE_ROOT, or
+    a git-ignored copy in oracle/_ref or baseline/_ref): BASELINE.md §3's C1 / C2 / C4 / C5.  Reported beside the C port, never
     as the arm's value: the port is the strongest CPU statement of the same arithmetic, the Python original is what a user of the reference
     actually runs.  Bounded to ~budget_s seconds in total."""
     import numpy as np
@@ -225,8 +236,8 @@ def reference_python_rates(budget_s: float = 24.0) -> dict:
     import refload
 
     if not refload.available():
-        return {"unavailable": "reference tree not staged on this box (baseline/_ref)"}
-    out = {"cpu_count": os.cpu_count(), "reference_root": "staged copy" if "baseline" in (refload.reference_root() or "") else "in place"}
+        return {"unavailable": "reference tree not available (CSTR_REFERENCE_ROOT, oracle/_ref or baseline/_ref)"}
+    out = {"cpu_count": os.cpu_count(), "reference_root": "staged copy" if os.path.basename(refload.reference_root()) == "_ref" else "in place"}
     try:
         refload.install_shims()
         core = refload.load_core()
@@ -394,6 +405,37 @@ def time_launches(torch, fn, k: int):
     return evs[0].elapsed_time(evs[-1]), per
 
 
+DUMP_REACTORS = 8192  # reactors sampled over ALL ranks: 8192 x (400 x (4 + 4) + 16 + 8 + 8) B = 26.5 MB per dump, whatever the rank count
+
+
+def dump_columns(n: int, world: int):
+    """The reactors of one rank's shard that --dump-outputs writes: sorted indices of default_rng(0).choice(n, k, replace=False) with
+    k = min(n, DUMP_REACTORS // world), so that the ranks together write at most DUMP_REACTORS reactors."""
+    import numpy as np
+
+    return np.sort(np.random.default_rng(0).choice(n, size=min(n, max(1, DUMP_REACTORS // world)), replace=False))
+
+
+def dump_outputs(out_dir: str, env, rewards, dones, rank: int, world: int) -> None:
+    """--dump-outputs: what the caller of the timed step receives after the last timed launch, as float32 / float64 .npy files, for the
+    reactors of dump_columns(): rewards / dones (T, k), state (k, 4), step_count and episode (k).  With more than one rank each writes
+    its own shard's sample under a _rank<r> suffix."""
+    import numpy as np
+    import torch
+
+    cols = dump_columns(rewards.shape[1], world)
+    idx = torch.as_tensor(cols, device=rewards.device)
+    arrays = {"rewards": rewards.index_select(1, idx).cpu().numpy(),
+              "dones": dones.index_select(1, idx).to(torch.float32).cpu().numpy(),
+              "state": env.state.index_select(0, idx).cpu().numpy(),
+              "step_count": env.step_count.index_select(0, idx).cpu().numpy().astype(np.float64),
+              "episode": env.episode.index_select(0, idx).cpu().numpy().astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def run_ours(args) -> None:
     import numpy as np
     import torch
@@ -469,6 +511,8 @@ def run_ours(args) -> None:
     ev1.record()
     ev1.synchronize()
     total_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:  # before the per-launch pass below steps the reactors on
+        dump_outputs(args.dump_outputs, env, rewards, dones, rank, world)
     barrier()
     _, per = time_launches(torch, step, args.steps)
     tmax = torch.tensor([total_ms], dtype=torch.float64, device=device)
@@ -597,6 +641,7 @@ def run_ours(args) -> None:
             sticky = sticky or any(k.endswith("error") for k in extras) or any(k.endswith("error") for k in extras.get("td3_update", {}))
             with stop.lock:
                 line["extras"] = extras
+    sticky = sticky or bool(FAILED_SECTIONS)
     stop.emit(line)
     if sticky:  # a failed section may have left a sticky CUDA error or a rank out of step: no teardown that could abort or wait
         sys.stdout.flush()
@@ -810,6 +855,7 @@ def run_extras(pkg, torch, device, lib, env, tape, rewards, dones, args) -> dict
                 Kr = 2 if mode_name == "fp32" else 16
                 ex[f"fused_rollout_{mode_name}_transitions_per_s"] = rate_of(lambda: roll.collect(Kr), ne * Kr, reps=3)
             except Exception as exc:
+                FAILED_SECTIONS.append(exc)  # kept, see describe_error
                 ex[f"fused_rollout_{mode_name}_transitions_per_s"] = f"unavailable: {exc}"
 
     def updates():
@@ -930,7 +976,12 @@ def main() -> None:
     ap.add_argument("--math", choices=["strict", "fast"], default="fast",
                     help="headline kernel: fast = the throughput variant (FMA contraction, MUFU; documented tolerance), strict = bit-exact vs the oracle; the other one is timed too and reported under \"other_math\"")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,7 +1,7 @@
 """Loader for the UNMODIFIED reference (TEST INFRASTRUCTURE ONLY — never imported by the product).
 
-Only usable where the reference tree exists (this build container: ``/root/reference``;
-override with ``CSTR_REFERENCE_ROOT``).  It is used by
+Only usable where the reference tree exists: ``CSTR_REFERENCE_ROOT``, or a copy of it under the git-ignored ``oracle/_ref`` or
+``baseline/_ref``.  The repository does not contain it.  It is used by
   * ``oracle/make_golden.py``   – to generate the committed fixtures under ``tests/golden/``;
   * ``tests/test_oracle_vs_reference.py`` – to pin the oracle restatement (skipped when absent);
   * ``oracle/run_reference_algos.py`` – reference TD3/SAC/BCQ/... on top of the GPU classes (staged for ``gpurun``).
@@ -30,9 +30,8 @@ _scratch: Optional[str] = None
 
 
 def reference_root() -> Optional[str]:
-    """``CSTR_REFERENCE_ROOT``, else /root/reference (the build container), else the git-ignored staging copy ``baseline/_ref`` that
-    travels to a GPU box with the repository snapshot."""
-    for root in (os.environ.get("CSTR_REFERENCE_ROOT"), "/root/reference", os.path.join(os.path.dirname(_HERE), "baseline", "_ref")):
+    """``CSTR_REFERENCE_ROOT``, else a git-ignored copy of the reference tree in ``oracle/_ref`` or ``baseline/_ref``."""
+    for root in (os.environ.get("CSTR_REFERENCE_ROOT"), os.path.join(_HERE, "_ref"), os.path.join(os.path.dirname(_HERE), "baseline", "_ref")):
         if root and os.path.isfile(os.path.join(root, "twoseriescstr.py")):
             return root
     return None

@@ -202,6 +202,70 @@ def test_both_arms_report_the_same_config(bench, monkeypatch, capsys):
     assert ours["rollout"] is None and ours["extras"] == {}  # --no-extras
 
 
+class _CountingLib(_FakeLib):
+    """The tape call numbers its launches: every reward is 1000 x (launch number) + the reactor's index, every state row the index."""
+
+    def __init__(self):
+        self.launches = 0
+
+    def cstr_tape_f32(self, params, n, T, mode, actions, t_base, state, sc, ep, static_base, rewards, dones, obs, rsum, stream):
+        self.launches += 1
+        self._fill(n, T, rewards, dones)
+        np.ctypeslib.as_array((ctypes.c_float * (T * n)).from_address(rewards)).reshape(T, n)[:] = 1000 * self.launches + np.arange(n)
+        np.ctypeslib.as_array((ctypes.c_float * (n * 4)).from_address(state)).reshape(n, 4)[:] = np.arange(n)[:, None]
+        return 0
+
+
+def test_dump_outputs_writes_what_the_last_timed_step_returned(bench, monkeypatch, capsys, tmp_path):
+    """--dump-outputs DIR: the arrays the caller of the LAST TIMED tape launch receives (not those of the per-launch pass after it), for the
+    seeded sample of reactors, float32 / float64 .npy; the JSON line is unchanged."""
+    lib = _CountingLib()
+    monkeypatch.setattr(importlib.import_module(PKG)._lib, "load", lambda *a, **kw: lib)
+    monkeypatch.setattr(bench, "DUMP_REACTORS", 64)  # below the fake batch of 256: a real sample
+    monkeypatch.delenv("WORLD_SIZE", raising=False)
+    monkeypatch.delenv("RANK", raising=False)
+    out_dir = tmp_path / "dump"
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "2", "--warmup", "3", "--no-extras", "--dump-outputs", str(out_dir)])
+    bench.main()
+    assert len([ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]) == 1
+    last_timed = 3 + 10 + 3 + 2  # the other math flavour (3 warm-up + 10 timed), the warm-up, the 2 timed steps
+    assert lib.launches == last_timed + 2  # then the per-launch timing pass
+    got = {f.stem: np.load(f) for f in out_dir.iterdir()}
+    n, T = bench.N_ENVS, bench.T_STEPS
+    cols = np.sort(np.random.default_rng(0).choice(n, size=64, replace=False))
+    assert np.array_equal(bench.dump_columns(n, 1), cols)
+    assert {k: v.shape for k, v in got.items()} == {"rewards": (T, 64), "dones": (T, 64), "state": (64, 4), "step_count": (64,), "episode": (64,)}
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    assert np.array_equal(got["rewards"], np.broadcast_to(1000 * last_timed + cols, (T, 64)).astype(np.float32))
+    assert np.array_equal(got["state"], np.broadcast_to(cols[:, None], (64, 4)).astype(np.float32))
+    assert got["dones"][T - 1].all() and not got["dones"][: T - 1].any()  # the fake tape's one truncation row
+
+
+def test_failed_section_keeps_its_objects_until_the_process_leaves(bench, monkeypatch, capsys):
+    """A section that fails with a device error: the error is in the line, and what the failed section's frames held is not freed before
+    bench.py leaves through os._exit(0) — after a device error such a free can abort the process before the line is printed."""
+    freed, exits = [], []
+
+    class Held:
+        def __del__(self):
+            freed.append(True)
+
+    def failing(*a, **kw):
+        held = Held()  # noqa: F841  (a tensor of the section in a real failure)
+        raise RuntimeError("CUDA error: an illegal memory access was encountered")
+
+    monkeypatch.setattr(bench, "td3_update_extras", failing)
+    monkeypatch.setattr(bench, "FAILED_SECTIONS", [])
+    monkeypatch.setattr(os, "_exit", lambda code: exits.append((code, list(freed))))
+    monkeypatch.delenv("WORLD_SIZE", raising=False)
+    monkeypatch.delenv("RANK", raising=False)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "2", "--warmup", "3"])
+    bench.main()
+    out = [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]
+    assert len(out) == 1 and "illegal memory access" in json.loads(out[0])["extras"]["updates_error"]
+    assert exits == [(0, [])]  # left through os._exit(0), nothing of the failed section freed before
+
+
 def test_hard_stop_prints_the_line_and_leaves_with_zero(bench, monkeypatch, capsys):
     """A section that never returns: the timer prints the line already assembled (with sections_timeout_s) and exits 0."""
     left = []
@@ -245,7 +309,8 @@ def test_two_ranks_one_line(tmp_path):
         f"sys.path.insert(0, {os.path.join(ROOT, 'tests')!r})\n"
         "import test_bench_dryrun as T\n"
         "b = T.install_fakes(pytest.MonkeyPatch())\n"
-        "sys.argv = ['bench.py', '--gpus', '2', '--steps', '3', '--warmup', '3']\n"
+        "b.DUMP_REACTORS = 64\n"
+        f"sys.argv = ['bench.py', '--gpus', '2', '--steps', '3', '--warmup', '3', '--dump-outputs', {str(tmp_path / 'dump')!r}]\n"
         "b.main()\n")
     env = dict(os.environ, CSTR_BENCH_BACKEND="gloo", OMP_NUM_THREADS="1")
     import socket
@@ -267,3 +332,7 @@ def test_two_ranks_one_line(tmp_path):
     row = line["dp_update"]["per_rank_batch_4096"]
     assert {"local_ms_per_update", "peer_ms_per_update", "nccl_eager_ms_per_update", "peer_over_local", "nccl_eager_over_local"} <= set(row)
     assert row["global_batch"] == 8192
+    # --dump-outputs: each rank writes its own shard's sample, DUMP_REACTORS reactors over both ranks together
+    dumped = {f.name: np.load(f) for f in (tmp_path / "dump").iterdir()}
+    assert set(dumped) == {f"{k}_rank{r}.npy" for k in ("rewards", "dones", "state", "step_count", "episode") for r in (0, 1)}
+    assert sum(dumped[f"state_rank{r}.npy"].shape[0] for r in (0, 1)) == 64 and dumped["rewards_rank1.npy"].shape == (8, 32)
