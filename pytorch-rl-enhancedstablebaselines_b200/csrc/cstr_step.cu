@@ -154,21 +154,23 @@ __device__ __forceinline__ void block_sum_to(double v, double *dst) {
 constexpr int TAPE_PF = 8;  // action loads in flight per thread
 
 // Per-thread cursor of the tape kernel: everything one control interval touches, passed by reference so the
-// unrolled loops below share one definition of "a step".
+// unrolled loops below share one definition of "a step".  The tapes are addressed by element index t*n + i: a 32-bit
+// index (IDX = uint32_t, when n*T < 2^31) makes each per-step address one IMAD.WIDE.U32 off the base and the advance one
+// 32-bit add, where 64-bit pointers cost two adds per pointer and step.
+template <typename IDX>
 struct TapeCursor {
     float4 s;        // strict: normalised state; fast: RAW state
     int sc, ep;
     bool bad_state, unboxed;
     double acc;
-    const float2 *pa;  // next action to prefetch for this thread
-    float *pr;         // this step's reward slot
-    uint8_t *pd;       // this step's done slot
-    float4 *po;        // this step's obs slot
+    IDX ia;  // element index of the next action to prefetch for this thread
+    IDX io;  // element index of this step's reward / done / obs slot
 };
 
-template <int MODE, bool CHECK, bool SUM, bool OBS>
-__device__ __forceinline__ void tape_step(const cstr_env_params &p, int64_t i, int64_t n, float target, double *static_base, float2 a,
-                                          TapeCursor &c, bool has_r, bool has_d) {
+template <int MODE, bool CHECK, bool SUM, bool OBS, bool REW, bool DONE, typename IDX>
+__device__ __forceinline__ void tape_step(const cstr_env_params &p, int64_t i, IDX n, float target, double *static_base, float2 a,
+                                          float *__restrict__ rewards, uint8_t *__restrict__ dones, float4 *__restrict__ obs_tape,
+                                          TapeCursor<IDX> &c) {
     StepResult r;
     if (MODE == MODE_STRICT) {
         // a state that did not come out of step_strict_core may lie outside the box (caller-injected, or a static-mode
@@ -178,27 +180,27 @@ __device__ __forceinline__ void tape_step(const cstr_env_params &p, int64_t i, i
         r = step_strict_core<CHECK>(c.s, sx, a, c.bad_state, c.sc, target, p.max_steps);
         c.unboxed = r.bad;  // a bad row keeps its (possibly unboxed) state
     } else {
+        // no commit: a bad row is truncated, so the reset below overwrites whatever state it computed
         r = step_fast_raw<CHECK>(c.s, a, c.bad_state, c.sc, target, p.max_steps);
     }
     c.bad_state = false;
-    if (has_r) *c.pr = r.reward;
-    if (has_d) *c.pd = (uint8_t)r.truncated;
+    if (REW) rewards[c.io] = r.reward;
+    if (DONE) dones[c.io] = (uint8_t)r.truncated;
     if (SUM) c.acc += (double)r.reward;
     bool wrote_obs = false;
     if (r.truncated) {
         c.s = reset_f32_env(p, i, c.ep, static_base);
-        if (OBS && MODE != MODE_STRICT) { *c.po = c.s; wrote_obs = true; }
+        if (OBS && MODE != MODE_STRICT) { obs_tape[c.io] = c.s; wrote_obs = true; }
         if (MODE != MODE_STRICT) c.s = fast_denorm(c.s);
         c.unboxed = p.init_mode != CSTR_INIT_RANDOM;
         c.sc = 0;
     }
-    if (OBS && !wrote_obs) *c.po = (MODE == MODE_STRICT) ? c.s : fast_norm(c.s);
-    c.pr += n;
-    c.pd += n;
-    if (OBS) c.po += n;
+    if (OBS && !wrote_obs) obs_tape[c.io] = (MODE == MODE_STRICT) ? c.s : fast_norm(c.s);
+    c.io += n;
 }
 
-// SUM / OBS are compile-time so the common launch (rewards + dones only) carries no dead work.
+// SUM / OBS / REW / DONE are compile-time so the common launch (rewards + dones only) carries no dead work and no
+// per-step pointer tests.
 // After the first step the register state is always "in the box" (it is either this kernel's own
 // output or a fresh reset: a bad/NaN row truncates and is reset at once), so the loop runs the
 // clamp-free cores; strict keeps the normalised state, fast keeps the RAW state across steps.
@@ -208,15 +210,16 @@ __device__ __forceinline__ void tape_step(const cstr_env_params &p, int64_t i, i
 // unconditional refills, which makes every ring slot a fixed register (a rolled loop with predicated refills made
 // ptxas copy each freshly loaded value at once and exposed the full HBM latency: 70 % long-scoreboard stalls);
 // the last <= 2*TAPE_PF-1 steps run through a guarded copy of the same body.
-template <int MODE, bool PHILOX, bool SUM, bool OBS>
+template <int MODE, bool PHILOX, bool SUM, bool OBS, bool REW, bool DONE, typename IDX>
 __global__ void __launch_bounds__(256, 2)
-tape_f32_kernel(cstr_env_params p, int64_t n, int64_t T64, const float2 *__restrict__ actions, uint32_t t_base,
+tape_f32_kernel(cstr_env_params p, int64_t n64, int64_t T64, const float2 *__restrict__ actions, uint32_t t_base,
                 float4 *__restrict__ state, int32_t *__restrict__ step_count, int32_t *__restrict__ episode, double *static_base,
                 float *__restrict__ rewards, uint8_t *__restrict__ dones, float4 *__restrict__ obs_tape, double *reward_sum, float target) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool live = i < n;
+    const bool live = i < n64;
     const int T = (int)T64;
-    TapeCursor c;
+    const IDX n = (IDX)n64;
+    TapeCursor<IDX> c;
     c.acc = 0.0;
     if (live) {
         c.s = state[i];
@@ -225,25 +228,22 @@ tape_f32_kernel(cstr_env_params p, int64_t n, int64_t T64, const float2 *__restr
         c.unboxed = true;
         c.sc = step_count[i];
         c.ep = episode[i];
-        const bool has_r = rewards != nullptr, has_d = dones != nullptr;
-        c.pr = rewards + i;
-        c.pd = dones + i;
-        c.po = obs_tape + i;
+        c.io = (IDX)i;
         if (PHILOX) {
             const uint64_t env = (uint64_t)(p.env_offset + i);
             uint4 cache = make_uint4(0, 0, 0, 0);
             for (int t = 0; t < T; ++t) {
                 const uint32_t g = t_base + (uint32_t)t;
                 const float2 a = philox_action(p.seed, env, g, cache, t == 0 || (g & 1u) == 0);
-                tape_step<MODE, false, SUM, OBS>(p, i, n, target, static_base, a, c, has_r, has_d);
+                tape_step<MODE, false, SUM, OBS, REW, DONE>(p, i, n, target, static_base, a, rewards, dones, obs_tape, c);
             }
         } else {
             float2 ring[TAPE_PF];
-            c.pa = actions + i;
+            c.ia = (IDX)i;
 #pragma unroll
             for (int j = 0; j < TAPE_PF; ++j) {
-                ring[j] = (j < T) ? *c.pa : make_float2(0.f, 0.f);
-                if (j + 1 < T) c.pa += n;  // ends up pointing at step min(TAPE_PF, T-1)... only dereferenced when in range
+                ring[j] = (j < T) ? actions[c.ia] : make_float2(0.f, 0.f);
+                if (j + 1 < T) c.ia += n;  // ends up at step min(TAPE_PF, T-1)... only dereferenced when in range
             }
             int t = 0;
             // full groups: every refill t+TAPE_PF+j (j < TAPE_PF) is in range  <=>  t + 2*TAPE_PF <= T.
@@ -256,11 +256,12 @@ tape_f32_kernel(cstr_env_params p, int64_t n, int64_t T64, const float2 *__restr
                 for (int j = 0; j < TAPE_PF; ++j) cur[j] = ring[j];
 #pragma unroll
                 for (int j = 0; j < TAPE_PF; ++j) {
-                    ring[j] = *c.pa;  // action of step t + TAPE_PF + j
-                    c.pa += n;
+                    ring[j] = actions[c.ia];  // action of step t + TAPE_PF + j
+                    c.ia += n;
                 }
 #pragma unroll
-                for (int j = 0; j < TAPE_PF; ++j) tape_step<MODE, true, SUM, OBS>(p, i, n, target, static_base, cur[j], c, has_r, has_d);
+                for (int j = 0; j < TAPE_PF; ++j)
+                    tape_step<MODE, true, SUM, OBS, REW, DONE>(p, i, n, target, static_base, cur[j], rewards, dones, obs_tape, c);
             }
             // tail: fewer than 2*TAPE_PF steps left; refills are guarded
             for (; t < T; t += TAPE_PF) {
@@ -269,10 +270,10 @@ tape_f32_kernel(cstr_env_params p, int64_t n, int64_t T64, const float2 *__restr
                     if (t + j < T) {
                         const float2 a = ring[j];
                         if (t + TAPE_PF + j < T) {
-                            ring[j] = *c.pa;
-                            if (t + TAPE_PF + j + 1 < T) c.pa += n;
+                            ring[j] = actions[c.ia];
+                            if (t + TAPE_PF + j + 1 < T) c.ia += n;
                         }
-                        tape_step<MODE, true, SUM, OBS>(p, i, n, target, static_base, a, c, has_r, has_d);
+                        tape_step<MODE, true, SUM, OBS, REW, DONE>(p, i, n, target, static_base, a, rewards, dones, obs_tape, c);
                     }
                 }
             }
@@ -449,9 +450,27 @@ int cstr_tape_f32(const cstr_env_params *p, int64_t n, int64_t T, int math_mode,
     int grid, block;
     env_launch_geometry(n, grid, block);
     cudaStream_t st = (cudaStream_t)stream;
-#define CSTR_LAUNCH_TAPE(MODE, PH, SUM, OBS)                                                                                     \
-    tape_f32_kernel<MODE, PH, SUM, OBS><<<grid, block, 0, st>>>(*p, n, T, (const float2 *)actions, t_base, (float4 *)state, step_count, \
-                                                                episode, static_base, rewards, dones, (float4 *)obs_tape, reward_sum, (float)p->target_c2)
+    const bool idx32 = n <= INT32_MAX / T;  // every tape element index t*n + i fits in 31 bits
+#define CSTR_LAUNCH_TAPE_IDX(MODE, PH, SUM, OBS, REW, DONE, IDX)                                                                 \
+    tape_f32_kernel<MODE, PH, SUM, OBS, REW, DONE, IDX><<<grid, block, 0, st>>>(*p, n, T, (const float2 *)actions, t_base,            \
+                                                                                (float4 *)state, step_count, episode, static_base,   \
+                                                                                rewards, dones, (float4 *)obs_tape, reward_sum,     \
+                                                                                (float)p->target_c2)
+#define CSTR_LAUNCH_TAPE_RD(MODE, PH, SUM, OBS, REW, DONE)                                   \
+    do {                                                                                     \
+        if (idx32) CSTR_LAUNCH_TAPE_IDX(MODE, PH, SUM, OBS, REW, DONE, uint32_t);            \
+        else CSTR_LAUNCH_TAPE_IDX(MODE, PH, SUM, OBS, REW, DONE, int64_t);                   \
+    } while (0)
+#define CSTR_LAUNCH_TAPE(MODE, PH, SUM, OBS)                                                       \
+    do {                                                                                           \
+        if (rewards) {                                                                             \
+            if (dones) CSTR_LAUNCH_TAPE_RD(MODE, PH, SUM, OBS, true, true);                        \
+            else CSTR_LAUNCH_TAPE_RD(MODE, PH, SUM, OBS, true, false);                             \
+        } else {                                                                                   \
+            if (dones) CSTR_LAUNCH_TAPE_RD(MODE, PH, SUM, OBS, false, true);                       \
+            else CSTR_LAUNCH_TAPE_RD(MODE, PH, SUM, OBS, false, false);                            \
+        }                                                                                          \
+    } while (0)
 #define CSTR_TAPE_FLAGS(MODE, PH)                                         \
     do {                                                                  \
         if (reward_sum) {                                                 \
@@ -469,6 +488,8 @@ int cstr_tape_f32(const cstr_env_params *p, int64_t n, int64_t T, int math_mode,
     }
 #undef CSTR_TAPE_FLAGS
 #undef CSTR_LAUNCH_TAPE
+#undef CSTR_LAUNCH_TAPE_RD
+#undef CSTR_LAUNCH_TAPE_IDX
     return check_launch("tape_f32_kernel");
 }
 
