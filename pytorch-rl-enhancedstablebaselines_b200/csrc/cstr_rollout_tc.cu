@@ -461,7 +461,16 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
             for (int64_t k = 0; k < K; ++k) {
                 // the first two layer-1 MMAs of the step go to the threads that own chunks 0 and 1
                 const uint32_t own0 = gc & 1u, own1 = own0 ^ 1u;
+                bool ordered = false;  // this thread already holds the ORDER token for its first chunk of the step
                 if (me == own0 || (g.NKC > 1 && me == own1)) {
+                    if (g.NKC == 1 && gc > 0) {
+                        // One chunk per step: the threads take alternate steps, so this one skipped the previous step's A1_FULL phase,
+                        // and parity k&1 also matches the phase two steps back, which has completed long ago.  Waiting first for
+                        // the other thread's chunk gc-1 (issued after it waited for the previous phase) leaves only this step's phase.
+                        mbar_wait(bars + 8 * (BAR_ORDER + me), order_waits & 1u);
+                        order_waits += 1;
+                        ordered = true;
+                    }
                     mbar_wait(bars + 8 * BAR_A1_FULL, (uint32_t)(k & 1));  // this step's observation rows are in shared memory
                     tc_fence_after();
                     if (me == own0) issue_l1(k, 0);
@@ -472,7 +481,7 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
                     const uint32_t wb = gc % TC_WSTAGES, wuse = gc / TC_WSTAGES, ab = gc & 1u, ause = gc >> 1;  // A_FULL phase = use count of the A buffer
                     mbar_wait(bars + 8 * (BAR_W_FULL + wb), wuse & 1u);
                     mbar_wait(bars + 8 * (BAR_A_FULL + ab), ause & 1u);
-                    if (gc > 0) {  // the other thread has issued chunk gc-1: keeps the accumulation order (chunk 0 overwrites)
+                    if (gc > 0 && !ordered) {  // the other thread has issued chunk gc-1: keeps the accumulation order (chunk 0 overwrites)
                         mbar_wait(bars + 8 * (BAR_ORDER + me), order_waits & 1u);
                         order_waits += 1;
                     }
@@ -529,7 +538,7 @@ int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int m
                            double *reward_sum, const cstr_episode_stats *stats, void *stream) {
     (void)warmup;
     TcGeometry g;
-    if (!make_geometry(actor->H1, actor->H2, g)) return fail_arg(CSTR_EINVAL, "rollout(tc): H1 must be a multiple of 16 (<=1024), H2 <= 512, and fit in shared memory");
+    if (!make_geometry(actor->H1, actor->H2, g)) return fail_arg(CSTR_EINVAL, "rollout(tc): H1 must be a multiple of 16 (<=1024), H2 rounded up to 16 plus two layer-1 K-chunks must fit 512 TMEM columns (H2 <= 480), and the operands must fit in shared memory");
     if (!packed_bf16) return fail_arg(CSTR_EINVAL, "rollout(tc): packed bf16 weights missing (cstr_actor_pack_bf16)");
     if (!aligned(packed_bf16, 16)) return fail_arg(CSTR_EALIGN, "rollout(tc): packed weights must be 16-byte aligned");
     if ((int64_t)K * g.NKC >= (int64_t)1 << 31) return fail_arg(CSTR_EINVAL, "rollout(tc): K too large");

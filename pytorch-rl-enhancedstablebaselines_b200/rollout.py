@@ -15,6 +15,25 @@ from . import _lib
 from .buffer import GpuReplayBuffer
 from .env import _MATH, GpuCSTRVecEnv
 
+# rollout_f32_kernel keeps h1 of its 128 reactors in shared memory: 128 * max(H1, 64) floats + 128 float4 <= 227 KB
+FP32_MAX_H1 = 448
+
+
+def actor_shape_error(H1: int, H2: int, actor_mode: str) -> Optional[str]:
+    """Why the rollout kernel of ``actor_mode`` cannot run a 4 -> H1 -> H2 actor — or None when it can."""
+    if H1 <= 0 or H2 <= 0 or H1 % 4:
+        return f"H1={H1}, H2={H2}: the rollout kernels need positive widths and H1 a multiple of 4"
+    if actor_mode != "tc":
+        return None if H1 <= FP32_MAX_H1 else f"H1={H1}: the float32 actor keeps h1 in shared memory, H1 <= {FP32_MAX_H1}"
+    if H1 % 16 or H1 > 1024:
+        return f"H1={H1}: the tensor-core actor needs H1 a multiple of 16 and <= 1024"
+    # the size query of the W2 packer reads the shape only (W2 need not point anywhere) and returns <= 0 for a shape it rejects
+    probe = _lib.ActorF32(W1=None, b1=None, W2=1, b2=None, W3=None, b3=None, H1=H1, H2=H2, kind=_lib.ACTOR_TANH, reserved=0)
+    if _lib.load().cstr_actor_pack_bf16(byref(probe), None, None) <= 0:
+        return (f"H1={H1}, H2={H2}: the tensor-core actor needs H2 rounded up to 16 plus two layer-1 K-chunks within 512 TMEM columns "
+                "(H2 <= 480) and its operand buffers within 227 KB of shared memory")
+    return None
+
 
 class ActorWeights:
     """fp32 weights of a 4 -> H1 -> H2 -> head actor on the device, torch Linear layout (out,in).
@@ -101,6 +120,9 @@ class ActorWeights:
     def pack_bf16(self):
         """Build the bf16 UMMA image of W2 for the tensor-core path (cstr_actor_pack_bf16)."""
         torch = _lib.require_cuda()
+        why = actor_shape_error(self.H1, self.H2, "tc")
+        if why:
+            raise ValueError(why)
         lib = _lib.load()
         with torch.cuda.device(self.device):
             nbytes = lib.cstr_actor_pack_bf16(byref(self._struct), None, None)
@@ -205,6 +227,9 @@ class FusedRollout:
         self.env, self.buffer, self.actor, self.sigma = env, buffer, actor, float(sigma)
         if isinstance(actor, AgentActorWeights) and actor_mode != "fp32":
             raise ValueError("the multi-agent rollout runs the float32 actor (actor_mode='fp32')")
+        why = actor_shape_error(actor.H1, actor.H2, actor_mode) if actor is not None else None
+        if why:
+            raise ValueError(why)
         self.actor_mode = actor_mode
         self.t = 0  # global step counter: the Philox counter of the noise / warm-up action streams
         self._lib = _lib.load()
@@ -276,8 +301,51 @@ def _noise_sigma(action_noise):
     return float(sigma[0])
 
 
-def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_noise) -> Optional[str]:
-    """Why ``cstr_rollout_fused`` can NOT stand in for this ``collect_rollouts`` call — or None when it can."""
+def _leaf_types(module):
+    return [type(m) for m in module.modules() if not any(True for _ in m.children())]
+
+
+def _actor_unsupported(actor, actor_mode: str) -> Optional[str]:
+    """Why the rollout kernels cannot evaluate this actor (the kernels are ReLU, ReLU, then a tanh or squashed-Gaussian head on a flat
+    4-value observation) — or None when they can."""
+    import torch.nn as nn
+
+    relu_trunk = [nn.Linear, nn.ReLU, nn.Linear, nn.ReLU]
+    if hasattr(actor, "mu_list"):  # MADDPG / IDDPG: per-agent 2 -> H1 -> H2 -> 1, run by the float32 kernel
+        shapes = set()
+        for i, mu in enumerate(actor.mu_list):
+            if _leaf_types(mu) != relu_trunk + [nn.Linear, nn.Tanh]:
+                return f"agent {i}'s actor is not Linear, ReLU, Linear, ReLU, Linear, Tanh: {[t.__name__ for t in _leaf_types(mu)]}"
+            lin = [m for m in mu.modules() if type(m) is nn.Linear]
+            if lin[0].in_features != 2 or lin[2].out_features != 1:
+                return f"agent {i}'s actor is {lin[0].in_features} -> {lin[2].out_features}, not 2 -> 1"
+            shapes.add((lin[0].out_features, lin[1].out_features))
+        if len(shapes) != 1:
+            return f"the agents' hidden widths differ: {sorted(shapes)}"
+        return actor_shape_error(*shapes.pop(), "fp32")
+    if type(getattr(actor, "features_extractor", None)).__name__ != "FlattenExtractor":
+        return f"features extractor {type(getattr(actor, 'features_extractor', None)).__name__} (the kernels read the raw observation)"
+    if hasattr(actor, "latent_pi"):  # SAC
+        if _leaf_types(actor.latent_pi) != relu_trunk:
+            return f"actor.latent_pi is not Linear, ReLU, Linear, ReLU: {[t.__name__ for t in _leaf_types(actor.latent_pi)]}"
+        if type(getattr(actor, "mu", None)) is not nn.Linear or type(getattr(actor, "log_std", None)) is not nn.Linear:
+            return "actor.mu / actor.log_std are not single Linear layers"
+        lin = [m for m in actor.latent_pi.modules() if type(m) is nn.Linear] + [actor.mu, actor.log_std]
+        outs = (actor.mu.out_features, actor.log_std.out_features)
+    else:  # TD3 / DDPG
+        if _leaf_types(actor.mu) != relu_trunk + [nn.Linear, nn.Tanh]:
+            return f"actor.mu is not Linear, ReLU, Linear, ReLU, Linear, Tanh: {[t.__name__ for t in _leaf_types(actor.mu)]}"
+        lin = [m for m in actor.mu.modules() if type(m) is nn.Linear]
+        outs = (lin[2].out_features,)
+    H1, H2 = lin[0].out_features, lin[1].out_features
+    if lin[0].in_features != 4 or any(o != 2 for o in outs) or lin[1].in_features != H1 or any(m.in_features != H2 for m in lin[2:]):
+        return f"actor is {lin[0].in_features} -> {H1} -> {H2} -> {outs}, not 4 -> H1 -> H2 -> 2"
+    return actor_shape_error(H1, H2, actor_mode)
+
+
+def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_noise, actor_mode: str = "fp32") -> Optional[str]:
+    """Why ``cstr_rollout_fused`` can NOT stand in for this ``collect_rollouts`` call — or None when it can.  ``actor_mode`` is the
+    kernel that would run the actor (``"fp32"`` or ``"tc"``; the two-agent actors always run on ``"fp32"``)."""
     if not isinstance(env, GpuCSTRVecEnv):
         return f"env is a {type(env).__name__}, not a GpuCSTRVecEnv (wrappers step through the NumPy protocol)"
     if env.dtype != "fp32" or env.reset_rng != "philox":
@@ -295,12 +363,12 @@ def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_nois
         splits = ([list(s) for s in getattr(model, "observation_splits", [])], [list(s) for s in getattr(model, "action_splits", [])])
         if len(actor.mu_list) != 2 or splits != ([[0, 1], [2, 3]], [[0], [1]]):
             return "agents are not the two reactors (observation_splits [[0,1],[2,3]], action_splits [[0],[1]])"
-        return None
+        return _actor_unsupported(actor, "fp32")
     if _noise_sigma(action_noise) is None:
         return f"action noise {action_noise!r} is not a zero-mean NormalActionNoise with one sigma"
     if actor is None or not (hasattr(actor, "mu") and (hasattr(actor.mu, "__len__") or hasattr(actor, "latent_pi"))):
         return "the policy has no TD3/DDPG `actor.mu` Sequential or SAC `actor.latent_pi/mu/log_std`"
-    return None
+    return _actor_unsupported(actor, actor_mode)
 
 
 def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
@@ -373,7 +441,7 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
 
         def collect_rollouts(self, env, callback, train_freq, replay_buffer, action_noise=None, learning_starts: int = 0, log_interval=None):
             noise = action_noise if action_noise is not None else self.action_noise
-            why = fused_rollout_unsupported(self, env, replay_buffer, train_freq, noise)
+            why = fused_rollout_unsupported(self, env, replay_buffer, train_freq, noise, actor_mode=actor_mode)
             if why:
                 if not self._fused_rollout_warned:
                     warnings.warn(f"fused rollout not used, the reference's collect_rollouts runs instead: {why}", RuntimeWarning, stacklevel=2)
