@@ -123,7 +123,7 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
     const Net g_critic = net_at(stt->grads, T.critic_off[0], T.critic);
     const float *dev_sc = stt->counters ? w.scalars : nullptr;
     if (stt->counters) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, actor_step_now ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, 0.0, 0.0);
+        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, actor_step_now ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
         if (int rc = check_launch("td3_tick_kernel")) return rc;
     }
     Workspace tw = as_workspace(w.sc);  // what the TD3-shaped critic helpers read

@@ -117,7 +117,7 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
     Workspace tw = as_workspace(w.sc);
     tw.n_row_blocks = rb;
     for (int i = 0; i < MA_AGENTS; ++i)
-        if (!(cfg->actor_lr[i] > 0.f) || !(cfg->critic_lr[i] > 0.f)) return fail_arg(CSTR_EINVAL, "ma_update: learning rates must be positive");
+        if (!(cfg->actor_lr[i] >= 0.f) || !(cfg->critic_lr[i] >= 0.f)) return fail_arg(CSTR_EINVAL, "ma_update: learning rates must be >= 0");
     auto adam = [&](ApplyArgs &a, int64_t step, float lr, bool actor_scalars, int agent) {
         a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
         const double bc1 = 1.0 - pow((double)cfg->beta1, (double)step), bc2 = 1.0 - pow((double)cfg->beta2, (double)step);

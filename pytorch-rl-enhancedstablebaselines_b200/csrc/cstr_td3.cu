@@ -793,7 +793,8 @@ __global__ void __launch_bounds__(256) td3_finalize_kernel(FinJobs J) {
 // graph mode: the per-update scalars (Philox counter of the smoothing noise, Adam bias corrections) cannot be baked into a captured
 // launch, so they live on the device.  counters = {n_updates, critic_step, actor_step, sample_draw}; one thread advances them at the
 // start of an update and derives scalars = {step_size_c, bc2_sqrt_c, step_size_a, bc2_sqrt_a, bits(n_updates)} (double math as torch).
-// lr_c2 / lr_a2 > 0 (multi-agent: a second critic / actor optimiser with its own rate): their {step_size, bc2_sqrt} pairs go to scalars[8..11].
+// lr_c2 / lr_a2 >= 0 (multi-agent: a second critic / actor optimiser with its own rate, which may be 0 as torch's Adam allows): their
+// {step_size, bc2_sqrt} pairs go to scalars[8..11]; -1 = no second optimiser.
 __global__ void td3_tick_kernel(int64_t *counters, float *scalars, int policy_step, double lr, double beta1, double beta2, double lr_a, double lr_c2,
                                 double lr_a2) {
     pdl_enter();
@@ -804,11 +805,11 @@ __global__ void td3_tick_kernel(int64_t *counters, float *scalars, int policy_st
     if (lr_a < 0.0) lr_a = lr;
     scalars[0] = (float)(lr / (1.0 - pow(beta1, (double)cs)));
     scalars[1] = (float)sqrt(1.0 - pow(beta2, (double)cs));
-    if (lr_c2 > 0.0) scalars[8] = (float)(lr_c2 / (1.0 - pow(beta1, (double)cs))), scalars[9] = scalars[1];
+    if (lr_c2 >= 0.0) scalars[8] = (float)(lr_c2 / (1.0 - pow(beta1, (double)cs))), scalars[9] = scalars[1];
     if (as > 0) {
         scalars[2] = (float)(lr_a / (1.0 - pow(beta1, (double)as)));
         scalars[3] = (float)sqrt(1.0 - pow(beta2, (double)as));
-        if (lr_a2 > 0.0) scalars[10] = (float)(lr_a2 / (1.0 - pow(beta1, (double)as))), scalars[11] = scalars[3];
+        if (lr_a2 >= 0.0) scalars[10] = (float)(lr_a2 / (1.0 - pow(beta1, (double)as))), scalars[11] = scalars[3];
     }
     scalars[4] = __uint_as_float((uint32_t)n);
 }
@@ -1309,7 +1310,7 @@ int cstr_td3_update(const cstr_td3_config *cfg, const cstr_td3_state *stt, const
     const int ZC = cfg->n_critics == 1 ? 1 : 2;  // DDPG = TD3 with one critic (core/ddpg/ddpg.py:100-109); its block 1 stays unused
     const float *dev_sc = stt->counters ? w.scalars : nullptr;  // graph mode (see td3_tick_kernel)
     if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD)) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, policy_step ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, 0.0, 0.0);
+        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, policy_step ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
         if (int rc = check_launch("td3_tick_kernel")) return rc;
     }
 
@@ -1458,7 +1459,7 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
         return check_launch("sac_ent_coef_kernel");
     };
     if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD)) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, 1, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, 0.0, 0.0);
+        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, 1, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
         if (int rc = check_launch("td3_tick_kernel")) return rc;
     }
     if (phases & CSTR_TD3_CRITIC_GRAD) {
