@@ -79,13 +79,10 @@ int cstr_bcq_layout(const cstr_bcq_config *cfg, int64_t *offsets) {
     if (int rc = check_bcq_cfg(cfg)) return rc;
     if (!offsets) return fail_arg(CSTR_EINVAL, "bcq_layout: null output");
     const BcqLayout T = bcq_layout(cfg);
-    const int64_t base[5] = {T.enc_off, T.dec_off, T.pert_off, T.critic_off[0], T.critic_off[1]};
-    const NetLayout *nets[5] = {&T.enc, &T.dec, &T.pert, &T.critic, &T.critic};
-    for (int n = 0; n < 5; ++n) {
-        const NetLayout &L = *nets[n];
-        const int64_t o[6] = {L.w1, L.b1, L.w2, L.b2, L.w3, L.b3};
-        for (int k = 0; k < 6; ++k) offsets[n * 6 + k] = base[n] + o[k];
-    }
+    put_offsets(offsets, 0, T.enc_off, T.enc);
+    put_offsets(offsets, 1, T.dec_off, T.dec);
+    put_offsets(offsets, 2, T.pert_off, T.pert);
+    for (int n = 3; n < 5; ++n) put_offsets(offsets, n, T.critic_off[n - 3], T.critic);
     offsets[30] = T.total;
     return 0;
 }
@@ -99,16 +96,10 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
                     const float *dones, const float *rewards, const float *eps_vae, const float *z_next, const float *z_actor, int64_t n_updates,
                     int64_t critic_step, int64_t actor_step, void *stream) {
     if (int rc = check_bcq_cfg(cfg)) return rc;
-    if (!stt || !stt->params || !stt->targets || !stt->grads || !stt->adam_m || !stt->adam_v || !stt->workspace)
-        return fail_arg(CSTR_EINVAL, "bcq_update: null state pointer");
-    if (!obs || !actions || !next_obs || !dones || !rewards) return fail_arg(CSTR_EINVAL, "bcq_update: null batch pointer");
-    if (!aligned(obs, 16) || !aligned(next_obs, 16) || !aligned(actions, 8) || (eps_vae && !aligned(eps_vae, 16)) || (z_next && !aligned(z_next, 16)) ||
-        (z_actor && !aligned(z_actor, 16)) || !aligned(stt->params, 16) || !aligned(stt->targets, 16) || !aligned(stt->grads, 16) ||
-        !aligned(stt->adam_m, 16) || !aligned(stt->adam_v, 16) || !aligned(stt->workspace, 16))
-        return fail_arg(CSTR_EALIGN, "bcq_update: 16 B (obs, latent draws, params, workspace) / 8 B (actions) alignment");
-    if (n_updates < 1 || critic_step < 1 || actor_step < 0) return fail_arg(CSTR_EINVAL, "bcq_update: counters are 1-based (value after this update)");
+    if (int rc = check_update("bcq", stt, cstr_bcq_workspace_bytes(cfg), obs, actions, next_obs, dones, rewards, n_updates, critic_step, actor_step)) return rc;
+    if ((eps_vae && !aligned(eps_vae, 16)) || (z_next && !aligned(z_next, 16)) || (z_actor && !aligned(z_actor, 16)))
+        return fail_arg(CSTR_EALIGN, "bcq_update: latent draws need 16 B alignment");
     BcqWorkspace w = bcq_carve(stt->workspace, cfg);
-    if (stt->workspace_bytes < w.floats * (int64_t)sizeof(float)) return fail_arg(CSTR_EINVAL, "bcq_update: workspace too small (cstr_bcq_workspace_bytes)");
     w.sc.tensor = cfg->gemm_mode;
     const BcqLayout T = bcq_layout(cfg);
     cudaStream_t st = (cudaStream_t)stream;
@@ -122,18 +113,8 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
     const Net g_enc = net_at(stt->grads, T.enc_off, T.enc), g_dec = net_at(stt->grads, T.dec_off, T.dec), g_pert = net_at(stt->grads, T.pert_off, T.pert);
     const Net g_critic = net_at(stt->grads, T.critic_off[0], T.critic);
     const float *dev_sc = stt->counters ? w.scalars : nullptr;
-    if (stt->counters) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, actor_step_now ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
-        if (int rc = check_launch("td3_tick_kernel")) return rc;
-    }
-    Workspace tw = as_workspace(w.sc);  // what the TD3-shaped critic helpers read
-    tw.n_row_blocks = rb;
-    auto adam = [&](ApplyArgs &a, int64_t step, bool actor_scalars) {
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
-        const double bc1 = 1.0 - pow((double)cfg->beta1, (double)step), bc2 = 1.0 - pow((double)cfg->beta2, (double)step);
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = (float)((double)cfg->lr / bc1), a.bc2_sqrt = (float)sqrt(bc2), a.tau = cfg->tau;
-        a.dev_scalars = dev_sc ? dev_sc + (actor_scalars ? 2 : 0) : nullptr;
-    };
+    if (stt->counters)
+        if (int rc = launch_tick(stt, w.scalars, actor_step_now, cfg->lr, cfg->beta1, cfg->beta2, -1.0, -1.0, -1.0, st)) return rc;
 
     // ---- VAE (bcq.py:142-155) ----
     Src s_enc{};
@@ -148,16 +129,15 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
     launch_k(bcq_vae_loss_kernel, tb, 256, 0, st, B, L, (const float2 *)w.recon, (const float2 *)actions, (const float *)w.e_y, (const float *)w.std, (float2 *)w.d_dy,
              w.loss_partial);
     if (int rc = check_launch("bcq_vae_loss_kernel")) return rc;
-    if (int rc = backward_mlp(B, T.dec, s_dec, w.xdec, dec, g_dec, w.d_h1, w.d_h2, w.d_dy, w.v_dz2, w.v_dz1, w.sc, true, st)) return rc;
+    if (int rc = backward_mlp(B, T.dec, s_dec, w.xdec, dec, g_dec, w.d_h1, w.d_h2, w.d_dy, w.v_dz2, w.v_dz1, w.sc, st)) return rc;
     launch_k(mlp_dx_kernel, rb, 256, 0, st, B, T.dec.h1, OBS + L, (const float *)w.v_dz1, (const float *)dec.w1, OBS, L, w.dzl);
     if (int rc = check_launch("mlp_dx_kernel<latent>")) return rc;
     launch_k(bcq_enc_grad_kernel, (unsigned)(((int64_t)B * L + 255) / 256), 256, 0, st, B, L, (const float *)w.dzl, (const float *)w.e_y, (const float *)w.std,
              (const float *)w.eps, w.e_dy);
     if (int rc = check_launch("bcq_enc_grad_kernel")) return rc;
-    if (int rc = backward_mlp(B, T.enc, s_enc, nullptr, enc, g_enc, w.e_h1, w.e_h2, w.e_dy, w.v_dz2, w.v_dz1, w.sc, true, st)) return rc;
+    if (int rc = backward_mlp(B, T.enc, s_enc, nullptr, enc, g_enc, w.e_h1, w.e_h2, w.e_dy, w.v_dz2, w.v_dz1, w.sc, st)) return rc;
     {
-        ApplyArgs a{};
-        adam(a, critic_step, false);
+        ApplyArgs a = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, critic_step, dev_sc, 0);
         a.adam_lo = T.enc_off, a.adam_hi = T.pert_off, a.polyak_lo = a.polyak_hi = 0;
         a.loss_partial = w.loss_partial, a.n_loss_partial = tb, a.loss_scale = 1.f, a.loss_acc = stt->losses;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<bcq vae>")) return rc;
@@ -182,20 +162,12 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
     if (int rc = check_launch("bcq_target_kernel")) return rc;
 
     // ---- critics (bcq.py:174-186): TD3's twin-critic step ----
-    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, 2, w.h1, w.h2, w.sc.tensor, st, w.sc.slabs, w.sc.slab_cap)) return rc;
-    launch_k(td3_critic_head_kernel<false>, dim3(rb, 2), 256, 0, st, B, H2, (const float *)w.h2, (int64_t)B * H2, (const float *)critic.w3, (const float *)critic.b3, cz,
-             (const float *)w.target, 2.f / (float)B, w.dq, w.dz2, w.loss_partial);
-    if (int rc = check_launch("td3_critic_head_kernel<bcq>")) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, 2, w.h1, w.h2, w.sc, st)) return rc;
+    if (int rc = critic_loss_backward(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, 2, w.h1, w.h2, w.target, 2.f / (float)B, w.dq, w.dz2, w.dz1,
+                                      w.loss_partial, w.sc, st))
+        return rc;
     {
-        SkinnyArgs s{};  // dW3 = dq^T @ h2, db3 = sum dq
-        s.X = w.h2, s.x_z = (int64_t)B * H2, s.ldx = H2, s.H = H2, s.B = B;
-        s.Y0 = w.dq, s.n0 = 1, s.ld0 = 1, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = B;
-        s.out_w = g_critic.w3, s.out_b = g_critic.b3, s.out_z = cz, s.transposed = 1;
-        FinJobs J{};
-        if (int rc = launch_skinny<1, true>(s, 2, tw.skinny + 2 * tw.skinny_region, st, "td3_skinny_wgrad_kernel<w3>", &J)) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, 2, w.h1, w.dz2, w.dz1, tw, true, st, &J)) return rc;
-        ApplyArgs a{};
-        adam(a, critic_step, false);
+        ApplyArgs a = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, critic_step, dev_sc, 0);
         a.adam_lo = T.critic_off[0], a.adam_hi = T.total, a.polyak_lo = a.polyak_hi = 0;
         a.loss_partial = w.loss_partial, a.n_loss_partial = 2 * rb, a.loss_scale = 1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 2 : nullptr;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<bcq critic>")) return rc;
@@ -215,18 +187,14 @@ int cstr_bcq_update(const cstr_bcq_config *cfg, const cstr_td3_state *stt, const
     if (int rc = forward_mlp(B, T.pert, s_apert, pert, 0, 1, w.p_h1, w.p_h2, w.xi, true, w.sc, st)) return rc;
     launch_k(bcq_perturb_kernel, tb, 256, 0, st, (int64_t)B, (const float2 *)w.a0, (const float2 *)w.xi, cfg->max_perturbation, (float2 *)w.a, (float2 *)w.pre);
     if (int rc = check_launch("bcq_perturb_kernel<actor>")) return rc;
-    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a, critic, cz, 1, w.h1, w.h2, w.sc.tensor, st, w.sc.slabs, w.sc.slab_cap)) return rc;
-    launch_k(td3_critic_head_kernel<true>, dim3(rb, 1), 256, 0, st, B, H2, (const float *)w.h2, (int64_t)B * H2, (const float *)critic.w3, (const float *)critic.b3, cz,
-             (const float *)nullptr, 0.f, w.dq, w.dz2, w.loss_partial);
-    if (int rc = check_launch("td3_critic_head_kernel<bcq policy>")) return rc;
-    if (int rc = backward_hidden(B, H1, H2, td3_src(obs, w.a, OBS + ACT), critic, g_critic, cz, 1, w.h1, w.dz2, w.dz1, tw, false, st)) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a, critic, cz, 1, w.h1, w.h2, w.sc, st)) return rc;
+    if (int rc = policy_critic_backward(B, H1, H2, critic, cz, w.h1, w.h2, w.dq, w.dz2, w.dz1, w.loss_partial, w.sc, st)) return rc;
     launch_k(mlp_dx_kernel, rb, 256, 0, st, B, H1, OBS + ACT, (const float *)w.dz1, (const float *)critic.w1, OBS, ACT, w.da);
     if (int rc = check_launch("mlp_dx_kernel<action>")) return rc;
     launch_k(bcq_pert_grad_kernel, tb, 256, 0, st, B, (const float2 *)w.da, (const float2 *)w.pre, (const float2 *)w.xi, cfg->max_perturbation, (float2 *)w.p_dy);
     if (int rc = check_launch("bcq_pert_grad_kernel")) return rc;
-    if (int rc = backward_mlp(B, T.pert, s_apert, nullptr, pert, g_pert, w.p_h1, w.p_h2, w.p_dy, w.p_dz2, w.p_dz1, w.sc, true, st)) return rc;
-    ApplyArgs a{};
-    adam(a, actor_step, true);
+    if (int rc = backward_mlp(B, T.pert, s_apert, nullptr, pert, g_pert, w.p_h1, w.p_h2, w.p_dy, w.p_dz2, w.p_dz1, w.sc, st)) return rc;
+    ApplyArgs a = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, actor_step, dev_sc, 2);
     a.adam_lo = T.pert_off, a.adam_hi = T.critic_off[0], a.polyak_lo = T.pert_off, a.polyak_hi = T.total;  // pert + both critics: one contiguous range
     a.loss_partial = w.loss_partial, a.n_loss_partial = rb, a.loss_scale = -1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 4 : nullptr;
     return launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<bcq pert+polyak>");

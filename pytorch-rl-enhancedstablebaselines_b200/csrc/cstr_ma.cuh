@@ -70,14 +70,9 @@ int cstr_ma_layout(const cstr_ma_config *cfg, int64_t *offsets) {
     if (!offsets) return fail_arg(CSTR_EINVAL, "ma_layout: null output");
     const MaLayout T = ma_layout(cfg);
     int n = 0;
-    auto put = [&](int64_t base, const NetLayout &L) {
-        const int64_t o[6] = {L.w1, L.b1, L.w2, L.b2, L.w3, L.b3};
-        for (int k = 0; k < 6; ++k) offsets[n * 6 + k] = base + o[k];
-        ++n;
-    };
-    for (int i = 0; i < MA_AGENTS; ++i) put(T.actor_off[i], T.actor);
+    for (int i = 0; i < MA_AGENTS; ++i) put_offsets(offsets, n++, T.actor_off[i], T.actor);
     for (int i = 0; i < MA_AGENTS; ++i)
-        for (int k = 0; k < T.n_critics; ++k) put(T.critic_off[i] + k * T.critic.size, T.critic);
+        for (int k = 0; k < T.n_critics; ++k) put_offsets(offsets, n++, T.critic_off[i] + k * T.critic.size, T.critic);
     offsets[n * 6] = T.total;
     return 0;
 }
@@ -91,15 +86,8 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
                    const float *dones, const float *rewards, const float *noise, int64_t n_updates, int64_t critic_step, int64_t actor_step,
                    void *stream) {
     if (int rc = check_ma_cfg(cfg)) return rc;
-    if (!stt || !stt->params || !stt->targets || !stt->grads || !stt->adam_m || !stt->adam_v || !stt->workspace)
-        return fail_arg(CSTR_EINVAL, "ma_update: null state pointer");
-    if (!obs || !actions || !next_obs || !dones || !rewards) return fail_arg(CSTR_EINVAL, "ma_update: null batch pointer");
-    if (!aligned(obs, 16) || !aligned(next_obs, 16) || !aligned(actions, 8) || !aligned(stt->params, 16) || !aligned(stt->targets, 16) ||
-        !aligned(stt->grads, 16) || !aligned(stt->adam_m, 16) || !aligned(stt->adam_v, 16) || !aligned(stt->workspace, 16))
-        return fail_arg(CSTR_EALIGN, "ma_update: 16 B (obs, params, workspace) / 8 B (actions) alignment");
-    if (n_updates < 1 || critic_step < 1 || actor_step < 0) return fail_arg(CSTR_EINVAL, "ma_update: counters are 1-based (value after this update)");
+    if (int rc = check_update("ma", stt, cstr_ma_workspace_bytes(cfg), obs, actions, next_obs, dones, rewards, n_updates, critic_step, actor_step)) return rc;
     MaWorkspace w = ma_carve(stt->workspace, cfg);
-    if (stt->workspace_bytes < w.floats * (int64_t)sizeof(float)) return fail_arg(CSTR_EINVAL, "ma_update: workspace too small (cstr_ma_workspace_bytes)");
     w.sc.tensor = cfg->gemm_mode;
     const MaLayout T = ma_layout(cfg);
     cudaStream_t st = (cudaStream_t)stream;
@@ -109,21 +97,11 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
     const bool policy_step = (n_updates % cfg->policy_delay) == 0;
     if (policy_step && actor_step < 1) return fail_arg(CSTR_EINVAL, "ma_update: actor_step must be >= 1 on a policy step");
     const float *dev_sc = stt->counters ? w.scalars : nullptr;
-    if (stt->counters) {  // one {step_size, bc2_sqrt} pair per optimiser: critic 0, actor 0 at scalars[0..3], critic 1, actor 1 at scalars[8..11]
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, policy_step ? 1 : 0, (double)cfg->critic_lr[0], (double)cfg->beta1, (double)cfg->beta2,
-                 (double)cfg->actor_lr[0], (double)cfg->critic_lr[1], (double)cfg->actor_lr[1]);
-        if (int rc = check_launch("td3_tick_kernel")) return rc;
-    }
-    Workspace tw = as_workspace(w.sc);
-    tw.n_row_blocks = rb;
+    if (stt->counters)  // one {step_size, bc2_sqrt} pair per optimiser: critic 0, actor 0 at scalars[0..3], critic 1, actor 1 at scalars[8..11]
+        if (int rc = launch_tick(stt, w.scalars, policy_step, cfg->critic_lr[0], cfg->beta1, cfg->beta2, cfg->actor_lr[0], cfg->critic_lr[1], cfg->actor_lr[1], st))
+            return rc;
     for (int i = 0; i < MA_AGENTS; ++i)
         if (!(cfg->actor_lr[i] >= 0.f) || !(cfg->critic_lr[i] >= 0.f)) return fail_arg(CSTR_EINVAL, "ma_update: learning rates must be >= 0");
-    auto adam = [&](ApplyArgs &a, int64_t step, float lr, bool actor_scalars, int agent) {
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
-        const double bc1 = 1.0 - pow((double)cfg->beta1, (double)step), bc2 = 1.0 - pow((double)cfg->beta2, (double)step);
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = (float)((double)lr / bc1), a.bc2_sqrt = (float)sqrt(bc2), a.tau = cfg->tau;
-        a.dev_scalars = dev_sc ? dev_sc + (agent ? 8 : 0) + (actor_scalars ? 2 : 0) : nullptr;
-    };
     // critic input of agent i over (observations X, actions A): all of both (MADDPG) or the agent's own slices (IDDPG)
     auto critic_src = [&](int i, const float *X, const float *A) {
         Src s{};
@@ -152,19 +130,10 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
         if (int rc = check_launch("td3_target_head_kernel<ma>")) return rc;
         const Src s_cur = critic_src(i, obs, actions);
         if (int rc = forward_hidden_g(B, T.critic, s_cur, critic, cz, ZC, w.h1, w.h2, w.sc, st)) return rc;
-        launch_k(td3_critic_head_kernel<false>, dim3(rb, ZC), 256, 0, st, B, H2, (const float *)w.h2, (int64_t)B * H2, (const float *)critic.w3, (const float *)critic.b3, cz,
-                 (const float *)w.target, 2.f / (float)B, w.dq, w.dz2, w.loss_partial);
-        if (int rc = check_launch("td3_critic_head_kernel<ma>")) return rc;
+        if (int rc = critic_loss_backward(B, H1, H2, s_cur, critic, g_critic, cz, ZC, w.h1, w.h2, w.target, 2.f / (float)B, w.dq, w.dz2, w.dz1, w.loss_partial, w.sc, st))
+            return rc;
         {
-            SkinnyArgs s{};
-            s.X = w.h2, s.x_z = (int64_t)B * H2, s.ldx = H2, s.H = H2, s.B = B;
-            s.Y0 = w.dq, s.n0 = 1, s.ld0 = 1, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = B;
-            s.out_w = g_critic.w3, s.out_b = g_critic.b3, s.out_z = cz, s.transposed = 1;
-            FinJobs J{};
-            if (int rc = launch_skinny<1, true>(s, ZC, tw.skinny + 2 * tw.skinny_region, st, "td3_skinny_wgrad_kernel<w3>", &J)) return rc;
-            if (int rc = backward_hidden(B, H1, H2, s_cur, critic, g_critic, cz, ZC, w.h1, w.dz2, w.dz1, tw, true, st, &J)) return rc;
-            ApplyArgs a{};
-            adam(a, critic_step, cfg->critic_lr[i], false, i);
+            ApplyArgs a = adam_args(stt, cfg->critic_lr[i], cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, critic_step, dev_sc, i ? 8 : 0);
             a.adam_lo = T.critic_off[i], a.adam_hi = T.critic_off[i] + ZC * cz, a.polyak_lo = a.polyak_hi = 0;
             a.loss_partial = w.loss_partial, a.n_loss_partial = ZC * rb, a.loss_scale = 1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 4 * i : nullptr;
             if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<ma critic>")) return rc;
@@ -179,10 +148,7 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
         if (int rc = check_launch("ma_joint_kernel")) return rc;
         const Src s_pi = critic_src(i, obs, w.joint);
         if (int rc = forward_hidden_g(B, T.critic, s_pi, critic, cz, 1, w.h1, w.h2, w.sc, st)) return rc;
-        launch_k(td3_critic_head_kernel<true>, dim3(rb, 1), 256, 0, st, B, H2, (const float *)w.h2, (int64_t)B * H2, (const float *)critic.w3, (const float *)critic.b3, cz,
-                 (const float *)nullptr, 0.f, w.dq, w.dz2, w.loss_partial);
-        if (int rc = check_launch("td3_critic_head_kernel<ma policy>")) return rc;
-        if (int rc = backward_hidden(B, H1, H2, s_pi, critic, g_critic, cz, 1, w.h1, w.dz2, w.dz1, tw, false, st)) return rc;
+        if (int rc = policy_critic_backward(B, H1, H2, critic, cz, w.h1, w.h2, w.dq, w.dz2, w.dz1, w.loss_partial, w.sc, st)) return rc;
         const int col = cfg->centralised ? OBS + i * MA_ACT : MA_OBS;  // where agent i's action sits in its critic's input
         launch_k(mlp_dx_kernel, rb, 256, 0, st, B, H1, CI, (const float *)w.dz1, (const float *)critic.w1, col, MA_ACT, w.da);
         if (int rc = check_launch("mlp_dx_kernel<ma action>")) return rc;
@@ -190,10 +156,9 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *stt, const f
         if (int rc = check_launch("ma_actor_grad_kernel")) return rc;
         const Net actor_i = net_at(stt->params, T.actor_off[i], T.actor), g_actor_i = net_at(stt->grads, T.actor_off[i], T.actor);
         if (int rc = backward_mlp(B, T.actor, s_act, nullptr, actor_i, g_actor_i, w.a_h1 + (int64_t)i * B * H1, w.a_h2 + (int64_t)i * B * H2, w.a_dy, w.a_dz2, w.a_dz1,
-                                  w.sc, true, st))
+                                  w.sc, st))
             return rc;
-        ApplyArgs a{};
-        adam(a, actor_step, cfg->actor_lr[i], true, i);
+        ApplyArgs a = adam_args(stt, cfg->actor_lr[i], cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, actor_step, dev_sc, (i ? 8 : 0) + 2);
         a.adam_lo = T.actor_off[i], a.adam_hi = T.actor_off[i] + az, a.polyak_lo = 0, a.polyak_hi = T.total;  // polyak of ALL nets, inside the agent loop (:181-182)
         a.loss_partial = w.loss_partial, a.n_loss_partial = rb, a.loss_scale = -1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 4 * i + 2 : nullptr;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<ma actor+polyak>")) return rc;

@@ -703,36 +703,6 @@ __global__ void __launch_bounds__(256) td3_skinny_wgrad_kernel(SkinnyArgs s) {
     }
 }
 
-// second stage: sum the chunks in order and scatter into the gradient tensors
-template <int NY, bool YBIAS>
-__global__ void __launch_bounds__(256) td3_skinny_reduce_kernel(SkinnyArgs s, int Hp, int Z) {
-    pdl_enter();
-    const int e = blockIdx.x * blockDim.x + threadIdx.x, z = blockIdx.y;
-    if (e >= (NY + 1) * Hp) return;
-    const int i = e / Hp, jj = e % Hp;
-    if (i == NY) {
-        if (!s.out_b || (YBIAS ? jj >= NY : jj >= s.H)) return;
-    } else if (jj >= s.H || !s.out_w) return;
-    const int64_t stride = (int64_t)Z * (NY + 1) * Hp;
-    const float *pp = s.part + (int64_t)z * (NY + 1) * Hp + e;
-    float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;  // four loads in flight; the combination order is fixed
-    int c = 0;
-    for (; c + 4 <= s.chunks; c += 4) {
-        a0 += pp[(c + 0) * stride];
-        a1 += pp[(c + 1) * stride];
-        a2 += pp[(c + 2) * stride];
-        a3 += pp[(c + 3) * stride];
-    }
-    for (; c < s.chunks; ++c) a0 += pp[c * stride];
-    const float v = (a0 + a1) + (a2 + a3);
-    if (i < NY) {
-        if (s.transposed) s.out_w[z * s.out_z + (int64_t)i * s.H + jj] = v;
-        else s.out_w[z * s.out_z + (int64_t)jj * NY + i] = v;
-    } else {
-        s.out_b[z * s.out_z + jj] = v;
-    }
-}
-
 // One node instead of four: the second stages of up to three skinny weight gradients and the dW2 slab sum of a backward pass run as
 // jobs of ONE launch (blockIdx.z = job).  Fewer graph nodes is what the small-batch update time is made of.
 struct FinJob {
@@ -830,25 +800,28 @@ struct ApplyArgs {
     float *loss_acc;  // [0] += scale * sum(partials), [1] += 1
 };
 
+// block 0 of an apply launch: the per-CTA loss partials -> the running loss sums (block-wide tree, fixed order)
+__device__ __forceinline__ void fold_loss_partials(const ApplyArgs &a) {
+    __shared__ float sl[256];
+    float s = 0.f;
+    for (int k = threadIdx.x; k < a.n_loss_partial; k += 256) s += a.loss_partial[k];
+    sl[threadIdx.x] = s;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if ((int)threadIdx.x < o) sl[threadIdx.x] += sl[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        a.loss_acc[0] += sl[0] * a.loss_scale;
+        a.loss_acc[1] += 1.f;
+    }
+}
+
 __global__ void __launch_bounds__(256) td3_apply_kernel(ApplyArgs a) {
     pdl_enter();
     const int64_t lo = min(a.adam_lo, a.polyak_lo < a.polyak_hi ? a.polyak_lo : a.adam_lo);
     const int64_t i = lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (blockIdx.x == 0 && a.loss_acc) {  // per-CTA loss partials -> running sums (block-wide, fixed order)
-        __shared__ float sl[256];
-        float s = 0.f;
-        for (int k = threadIdx.x; k < a.n_loss_partial; k += 256) s += a.loss_partial[k];
-        sl[threadIdx.x] = s;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) {
-            if ((int)threadIdx.x < o) sl[threadIdx.x] += sl[threadIdx.x + o];
-            __syncthreads();
-        }
-        if (threadIdx.x == 0) {
-            a.loss_acc[0] += sl[0] * a.loss_scale;
-            a.loss_acc[1] += 1.f;
-        }
-    }
+    if (blockIdx.x == 0 && a.loss_acc) fold_loss_partials(a);
     float p;
     bool have = false;
     const float step_size = a.dev_scalars ? a.dev_scalars[0] : a.step_size, bc2_sqrt = a.dev_scalars ? a.dev_scalars[1] : a.bc2_sqrt;
@@ -936,21 +909,7 @@ __global__ void __launch_bounds__(256) td3_apply_peer_kernel(ApplyArgs a, PeerAr
     // group is ONE bounded wait, after which the host finds the error word (cstr_peer_error) instead of a hung stream
     const bool broken = *(volatile uint32_t *)(my + PEER_ERROR) != 0u;
     const bool alive = !broken && peer_barrier(pa, 0, epoch);
-    if (blockIdx.x == 0 && a.loss_acc) {  // as td3_apply_kernel: per-CTA loss partials -> running sums (the LOCAL shard's loss)
-        __shared__ float sl[256];
-        float s = 0.f;
-        for (int k = threadIdx.x; k < a.n_loss_partial; k += 256) s += a.loss_partial[k];
-        sl[threadIdx.x] = s;
-        __syncthreads();
-        for (int o = 128; o > 0; o >>= 1) {
-            if ((int)threadIdx.x < o) sl[threadIdx.x] += sl[threadIdx.x + o];
-            __syncthreads();
-        }
-        if (threadIdx.x == 0) {
-            a.loss_acc[0] += sl[0] * a.loss_scale;
-            a.loss_acc[1] += 1.f;
-        }
-    }
+    if (blockIdx.x == 0 && a.loss_acc) fold_loss_partials(a);  // the LOCAL shard's loss
     const float step_size = a.dev_scalars ? a.dev_scalars[0] : a.step_size, bc2_sqrt = a.dev_scalars ? a.dev_scalars[1] : a.bc2_sqrt;
     const int64_t lo = min(a.adam_lo, a.polyak_lo < a.polyak_hi ? a.polyak_lo : a.adam_lo), hi = max(a.adam_hi, a.polyak_hi);
     if (alive)  // every range boundary is a multiple of 4 floats (pad4 layout): one float4 group per thread and trip
@@ -1014,20 +973,6 @@ using namespace cstr;
 // ------------------------------------------------------------------------------------------------------------------
 namespace {
 
-struct Workspace {  // carved out of the caller's workspace buffer (floats)
-    float *h1[2], *h2[2];    // forward activations, [z] slabs contiguous: h1[0] + B*H1 == h1[1]
-    float *dz1, *dz2;        // 2 slabs each
-    float *t_h1, *t_h2;      // target-critic activations (2 slabs)
-    float *a_h1, *a_h2;      // actor / actor-target activations
-    float *next_act, *a_pi, *target, *dq, *dpre, *loss_partial, *slabs, *skinny, *scalars;
-    float *logp, *next_logp, *std_eps, *raw_log_std, *dpre4, *lp_partial;  // SAC
-    int n_row_blocks;
-    int64_t slab_cap;  // floats in `slabs`
-    int64_t skinny_region;
-    int tensor;  // cfg->gemm_mode: 0 FFMA, 1 tcgen05 bf16x3 split, 2 tcgen05 plain bf16
-    int64_t floats;
-};
-
 constexpr int MAX_SPLITS = 16;
 
 // split-K factor of the dW2 GEMM: minimise (CTA rounds per SM) x (k-iterations per CTA) over the 148 SMs
@@ -1044,36 +989,6 @@ int choose_splits(int B, int H1, int H2, int Z, int tc) {
     return best;
 }
 
-Workspace carve(float *base, int B, int H1, int H2) {
-    Workspace w;
-    int64_t o = 0;
-    auto take = [&](int64_t n) {
-        float *p = base ? base + o : nullptr;
-        o += pad4(n);
-        return p;
-    };
-    const int64_t bh1 = (int64_t)B * H1, bh2 = (int64_t)B * H2;
-    w.h1[0] = take(2 * bh1), w.h1[1] = w.h1[0] ? w.h1[0] + bh1 : nullptr;
-    w.h2[0] = take(2 * bh2), w.h2[1] = w.h2[0] ? w.h2[0] + bh2 : nullptr;
-    w.dz1 = take(2 * bh1), w.dz2 = take(2 * bh2);
-    w.t_h1 = take(2 * bh1), w.t_h2 = take(2 * bh2);
-    w.a_h1 = take(bh1), w.a_h2 = take(bh2);
-    w.next_act = take(2 * (int64_t)B), w.a_pi = take(2 * (int64_t)B), w.target = take(B), w.dq = take(2 * (int64_t)B), w.dpre = take(2 * (int64_t)B);
-    w.n_row_blocks = (B + 7) / 8;
-    w.loss_partial = take(2 * (int64_t)w.n_row_blocks);
-    w.slab_cap = (int64_t)MAX_SPLITS * 2 * pad4((int64_t)H1 * H2);
-    w.slabs = take(w.slab_cap);
-    const int64_t hp = ((int64_t)(H1 > H2 ? H1 : H2) + 31) / 32 * 32;
-    w.skinny_region = (int64_t)((B + SKINNY_ROWS - 1) / SKINNY_ROWS) * 2 * (OBS + ACT + 1) * hp;
-    w.skinny = take(3 * w.skinny_region);  // one region per deferred job of a backward pass
-    w.scalars = take(8);
-    w.logp = take(B), w.next_logp = take(B), w.std_eps = take(2 * (int64_t)B), w.raw_log_std = take(2 * (int64_t)B), w.dpre4 = take(4 * (int64_t)B);
-    w.lp_partial = take(w.n_row_blocks);
-    w.tensor = 0;
-    w.floats = o;
-    return w;
-}
-
 int check_cfg(const cstr_td3_config *c) {
     if (!c) return fail_arg(CSTR_EINVAL, "td3: null config");
     if (c->h1 < 4 || c->h2 < 4 || (c->h1 & 3) || (c->h2 & 3) || c->h1 > 4096 || c->h2 > 4096)
@@ -1086,20 +1001,16 @@ int check_cfg(const cstr_td3_config *c) {
 }
 
 template <int NY, bool YBIAS>
-int launch_skinny(SkinnyArgs s, int Z, float *part, cudaStream_t st, const char *what, FinJobs *defer = nullptr) {
+int launch_skinny(SkinnyArgs s, int Z, float *part, cudaStream_t st, const char *what, FinJobs &J) {
     s.part = part;
     s.rows_per_chunk = SKINNY_ROWS;
     s.chunks = (s.B + SKINNY_ROWS - 1) / SKINNY_ROWS;
-    const int cols = (s.H + 31) / 32, Hp = cols * 32;
+    const int cols = (s.H + 31) / 32;
     launch_k(td3_skinny_wgrad_kernel<NY, YBIAS>, dim3(cols, s.chunks, Z), 256, 0, st, s);
     if (int rc = check_launch(what)) return rc;
-    if (defer) {  // the second stage runs as a job of the backward pass's finalize launch
-        FinJob &f = defer->job[defer->n++];
-        f.s = s, f.ny = NY, f.ybias = YBIAS ? 1 : 0, f.hp = Hp, f.Z = Z;
-        return 0;
-    }
-    launch_k(td3_skinny_reduce_kernel<NY, YBIAS>, dim3(((NY + 1) * Hp + 255) / 256, Z), 256, 0, st, s, Hp, Z);
-    return check_launch(what);
+    FinJob &f = J.job[J.n++];  // the second stage runs as a job of the backward pass's finalize launch
+    f.s = s, f.ny = NY, f.ybias = YBIAS ? 1 : 0, f.hp = cols * 32, f.Z = Z;
+    return 0;
 }
 
 int launch_finalize(const FinJobs &J, cudaStream_t st) {
@@ -1187,68 +1098,6 @@ struct Net {  // pointers of one net (or the first of a z-batched pair) inside a
 };
 Net net_at(float *base, int64_t off, const NetLayout &L) { return Net{base + off + L.w1, base + off + L.b1, base + off + L.w2, base + off + L.b2, base + off + L.w3, base + off + L.b3}; }
 
-// h1 = relu(L1(x)), h2 = relu(L2(h1)) for Z nets that are `z_stride` floats apart
-int forward_hidden(int B, int H1, int H2, int in, const float *obs, const float *act, const Net &n, int64_t z_stride, int Z, float *h1, float *h2,
-                   int tensor, cudaStream_t st, float *split_buf = nullptr, int64_t split_cap = 0) {
-    const int64_t threads = (int64_t)((B + L1_ROWS - 1) / L1_ROWS) * (H1 / 4);
-    dim3 grid((unsigned)((threads + 255) / 256), Z);
-    if (in == OBS)
-        launch_k(td3_layer1_kernel<OBS>, grid, 256, 0, st, B, H1, (const float4 *)obs, nullptr, n.w1, n.b1, z_stride, h1, (int64_t)B * H1);
-    else
-        launch_k(td3_layer1_kernel<OBS + ACT>, grid, 256, 0, st, B, H1, (const float4 *)obs, (const float2 *)act, n.w1, n.b1, z_stride, h1, (int64_t)B * H1);
-    if (int rc = check_launch("td3_layer1_kernel")) return rc;
-    GemmArgs g{};
-    g.A = h1, g.Bm = n.w2, g.aux = n.b2, g.C = h2;
-    g.M = B, g.N = H2, g.K = H1, g.lda = H1, g.ldb = H1, g.ldc = H2, g.ldaux = 0;
-    g.a_z = (int64_t)B * H1, g.b_z = z_stride, g.c_z = (int64_t)B * H2, g.aux_z = z_stride;
-    g.splits = 1, g.k_per_split = H1, g.c_split = 0;
-    g.split_buf = split_buf, g.split_cap = split_cap;
-    return launch_gemm<G_FWD>(g, Z, tensor, st, "td3_gemm_kernel<fwd>");
-}
-
-// given dz2 (and h1, x): dz1 (optional), then every weight gradient of the hidden and input layers into the flat grads
-template <bool YBIAS>
-int launch_skinny_ny(int ny, SkinnyArgs s, int Z, float *part, cudaStream_t st, const char *what, FinJobs *defer);
-
-int backward_hidden(int B, int H1, int H2, const Src &src, const Net &n, const Net &gn, int64_t z_stride, int Z,
-                    const float *h1, const float *dz2, float *dz1, const Workspace &w, bool want_weight_grads, cudaStream_t st,
-                    FinJobs *pending = nullptr) {
-    const int in = src.n0 + src.n1;
-    GemmArgs g{};
-    g.A = dz2, g.Bm = n.w2, g.aux = h1, g.C = dz1;
-    g.M = B, g.N = H1, g.K = H2, g.lda = H2, g.ldb = H1, g.ldc = H1, g.ldaux = H1;
-    g.a_z = (int64_t)B * H2, g.b_z = z_stride, g.c_z = (int64_t)B * H1, g.aux_z = (int64_t)B * H1;
-    g.splits = 1, g.k_per_split = H2, g.c_split = 0;
-    g.split_buf = w.slabs, g.split_cap = w.slab_cap;
-    if (int rc = launch_gemm<G_DGRAD>(g, Z, w.tensor, st, "td3_gemm_kernel<dgrad>")) return rc;
-    if (!want_weight_grads) return 0;
-    // dW2 = dz2^T @ h1, split over the batch into slabs, then summed in order
-    const int64_t w2n = pad4((int64_t)H1 * H2);
-    GemmArgs q{};
-    q.A = dz2, q.Bm = h1, q.aux = nullptr, q.C = w.slabs;
-    q.M = H2, q.N = H1, q.K = B, q.lda = H2, q.ldb = H1, q.ldc = H1, q.ldaux = 0;
-    q.a_z = (int64_t)B * H2, q.b_z = (int64_t)B * H1, q.c_z = w2n, q.aux_z = 0;
-    const int splits = choose_splits(B, H1, H2, Z, w.tensor);
-    q.splits = splits, q.k_per_split = (B + splits - 1) / splits, q.c_split = 2 * w2n;
-    if (int rc = launch_gemm<G_WGRAD>(q, Z, w.tensor, st, "td3_gemm_kernel<wgrad>")) return rc;
-    FinJobs local{};
-    FinJobs &J = pending ? *pending : local;  // the caller's layer-3 job (region 2) rides along
-    J.slab_n4 = (int64_t)H1 * H2 / 4, J.slab_splits = splits, J.slabs = (const float4 *)w.slabs, J.slab_stride4 = 2 * w2n / 4, J.slab_z4 = w2n / 4;
-    J.slab_out = (float4 *)gn.w2, J.slab_out_z4 = z_stride / 4, J.slab_Z = Z;
-    // db2 = colsum(dz2)
-    SkinnyArgs s{};
-    s.X = dz2, s.x_z = (int64_t)B * H2, s.ldx = H2, s.H = H2, s.B = B;
-    s.out_w = nullptr, s.out_b = gn.b2, s.out_z = z_stride;
-    if (int rc = launch_skinny<0, false>(s, Z, w.skinny, st, "td3_skinny_wgrad_kernel<b2>", &J)) return rc;
-    // dW1 = dz1^T @ [x0 | x1] (TD3: [obs | act]), db1 = colsum(dz1)
-    SkinnyArgs t{};
-    t.X = dz1, t.x_z = (int64_t)B * H1, t.ldx = H1, t.H = H1, t.B = B;
-    t.Y0 = src.x0, t.n0 = src.n0, t.ld0 = src.ld0, t.Y1 = src.x1, t.n1 = src.n1, t.ld1 = src.ld1, t.y_z = 0;
-    t.out_w = gn.w1, t.out_b = gn.b1, t.out_z = z_stride;
-    if (int rc = launch_skinny_ny<false>(in, t, Z, w.skinny + w.skinny_region, st, "td3_skinny_wgrad_kernel<w1>", &J)) return rc;
-    return launch_finalize(J, st);
-}
-
 inline Src td3_src(const float *obs, const float *act, int in) {  // [obs (4) | act (in - 4)]
     Src s{};
     s.x0 = obs, s.n0 = OBS, s.ld0 = OBS, s.x0_rows = 0, s.x1 = in > OBS ? act : nullptr, s.n1 = in - OBS, s.ld1 = ACT;
@@ -1256,6 +1105,43 @@ inline Src td3_src(const float *obs, const float *act, int in) {  // [obs (4) | 
 }
 
 #include "cstr_mlp_host.cuh"
+
+struct Workspace {  // carved out of the caller's workspace buffer (floats)
+    float *h1[2], *h2[2];    // forward activations, [z] slabs contiguous: h1[0] + B*H1 == h1[1]
+    float *dz1, *dz2;        // 2 slabs each
+    float *t_h1, *t_h2;      // target-critic activations (2 slabs)
+    float *a_h1, *a_h2;      // actor / actor-target activations
+    float *next_act, *a_pi, *target, *dq, *dpre, *loss_partial, *scalars;
+    float *logp, *next_logp, *std_eps, *raw_log_std, *dpre4, *lp_partial;  // SAC
+    MlpScratch sc;
+    int n_row_blocks;
+    int64_t floats;
+};
+
+Workspace carve(float *base, int B, int H1, int H2) {
+    Workspace w;
+    Bump b(base);
+    const int64_t bh1 = (int64_t)B * H1, bh2 = (int64_t)B * H2;
+    w.h1[0] = b.take(2 * bh1), w.h1[1] = w.h1[0] ? w.h1[0] + bh1 : nullptr;
+    w.h2[0] = b.take(2 * bh2), w.h2[1] = w.h2[0] ? w.h2[0] + bh2 : nullptr;
+    w.dz1 = b.take(2 * bh1), w.dz2 = b.take(2 * bh2);
+    w.t_h1 = b.take(2 * bh1), w.t_h2 = b.take(2 * bh2);
+    w.a_h1 = b.take(bh1), w.a_h2 = b.take(bh2);
+    w.next_act = b.take(2 * (int64_t)B), w.a_pi = b.take(2 * (int64_t)B), w.target = b.take(B), w.dq = b.take(2 * (int64_t)B), w.dpre = b.take(2 * (int64_t)B);
+    w.n_row_blocks = (B + 7) / 8;
+    w.loss_partial = b.take(2 * (int64_t)w.n_row_blocks);
+    w.sc.slab_cap = (int64_t)MAX_SPLITS * 2 * pad4((int64_t)H1 * H2);  // the dW2 slabs of two H2 x H1 critics
+    w.sc.slabs = b.take(w.sc.slab_cap);
+    const int64_t hp = ((int64_t)(H1 > H2 ? H1 : H2) + 31) / 32 * 32;
+    w.sc.skinny_region = (int64_t)((B + SKINNY_ROWS - 1) / SKINNY_ROWS) * 2 * (OBS + ACT + 1) * hp;
+    w.sc.skinny = b.take(3 * w.sc.skinny_region);
+    w.sc.tensor = 0;
+    w.scalars = b.take(8);
+    w.logp = b.take(B), w.next_logp = b.take(B), w.std_eps = b.take(2 * (int64_t)B), w.raw_log_std = b.take(2 * (int64_t)B), w.dpre4 = b.take(4 * (int64_t)B);
+    w.lp_partial = b.take(w.n_row_blocks);
+    w.floats = b.o;
+    return w;
+}
 
 }  // namespace
 
@@ -1269,12 +1155,8 @@ int64_t cstr_td3_param_count(int32_t h1, int32_t h2) {
 int cstr_td3_layout(int32_t h1, int32_t h2, int64_t *offsets) {
     if (!offsets || h1 < 4 || h2 < 4 || (h1 & 3) || (h2 & 3)) return fail_arg(CSTR_EINVAL, "td3_layout: bad sizes or null output");
     const Td3Layout T = td3_layout(h1, h2);
-    const int64_t base[3] = {T.actor_off, T.critic_off[0], T.critic_off[1]};
-    for (int n = 0; n < 3; ++n) {
-        const NetLayout &L = n == 0 ? T.actor : T.critic;
-        const int64_t o[6] = {L.w1, L.b1, L.w2, L.b2, L.w3, L.b3};
-        for (int k = 0; k < 6; ++k) offsets[n * 6 + k] = base[n] + o[k];
-    }
+    put_offsets(offsets, 0, T.actor_off, T.actor);
+    for (int n = 1; n < 3; ++n) put_offsets(offsets, n, T.critic_off[n - 1], T.critic);
     offsets[18] = T.total;
     return 0;
 }
@@ -1288,17 +1170,11 @@ int cstr_td3_update(const cstr_td3_config *cfg, const cstr_td3_state *stt, const
                     const float *dones, const float *rewards, const float *noise, int64_t n_updates, int64_t critic_step, int64_t actor_step,
                     int32_t phases, void *stream) {
     if (int rc = check_cfg(cfg)) return rc;
-    if (!stt || !stt->params || !stt->targets || !stt->grads || !stt->adam_m || !stt->adam_v || !stt->workspace)
-        return fail_arg(CSTR_EINVAL, "td3_update: null state pointer");
-    if (!obs || !actions || !next_obs || !dones || !rewards) return fail_arg(CSTR_EINVAL, "td3_update: null batch pointer");
-    if (!aligned(obs, 16) || !aligned(next_obs, 16) || !aligned(actions, 8) || (noise && !aligned(noise, 8)) || !aligned(stt->params, 16) ||
-        !aligned(stt->targets, 16) || !aligned(stt->grads, 16) || !aligned(stt->adam_m, 16) || !aligned(stt->adam_v, 16) || !aligned(stt->workspace, 16))
-        return fail_arg(CSTR_EALIGN, "td3_update: 16 B (obs/params/workspace) / 8 B (actions, noise) alignment");
+    if (int rc = check_update("td3", stt, cstr_td3_workspace_bytes(cfg), obs, actions, next_obs, dones, rewards, n_updates, critic_step, actor_step)) return rc;
+    if (noise && !aligned(noise, 8)) return fail_arg(CSTR_EALIGN, "td3_update: noise needs 8 B alignment");
     const int B = cfg->batch, H1 = cfg->h1, H2 = cfg->h2;
     Workspace w = carve(stt->workspace, B, H1, H2);
-    w.tensor = cfg->gemm_mode;
-    if (stt->workspace_bytes < w.floats * (int64_t)sizeof(float)) return fail_arg(CSTR_EINVAL, "td3_update: workspace too small (cstr_td3_workspace_bytes)");
-    if (n_updates < 1 || critic_step < 1 || actor_step < 0) return fail_arg(CSTR_EINVAL, "td3_update: counters are 1-based (value after this update)");
+    w.sc.tensor = cfg->gemm_mode;
     const Td3Layout T = td3_layout(H1, H2);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t cz = T.critic.size;
@@ -1309,54 +1185,37 @@ int cstr_td3_update(const cstr_td3_config *cfg, const cstr_td3_state *stt, const
     const bool policy_step = (n_updates % cfg->policy_delay) == 0;
     const int ZC = cfg->n_critics == 1 ? 1 : 2;  // DDPG = TD3 with one critic (core/ddpg/ddpg.py:100-109); its block 1 stays unused
     const float *dev_sc = stt->counters ? w.scalars : nullptr;  // graph mode (see td3_tick_kernel)
-    if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD)) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, policy_step ? 1 : 0, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
-        if (int rc = check_launch("td3_tick_kernel")) return rc;
-    }
+    if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD))
+        if (int rc = launch_tick(stt, w.scalars, policy_step, cfg->lr, cfg->beta1, cfg->beta2, -1.0, -1.0, -1.0, st)) return rc;
 
     if (phases & CSTR_TD3_CRITIC_GRAD) {
         // ---- target (td3.py:166-175) ----
-        if (int rc = forward_hidden(B, H1, H2, OBS, next_obs, nullptr, actor_t, 0, 1, w.a_h1, w.a_h2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+        if (int rc = forward_hidden(B, H1, H2, OBS, next_obs, nullptr, actor_t, 0, 1, w.a_h1, w.a_h2, w.sc, st)) return rc;
         launch_k(td3_actor_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor_t.w3, actor_t.b3, 1, (const float2 *)noise, cfg->target_policy_noise,
                                                  cfg->target_noise_clip, cfg->seed, (uint32_t)n_updates, dev_sc, (float2 *)w.next_act);
         if (int rc = check_launch("td3_actor_head_kernel")) return rc;
-        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, next_obs, w.next_act, critic_t, cz, ZC, w.t_h1, w.t_h2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, next_obs, w.next_act, critic_t, cz, ZC, w.t_h1, w.t_h2, w.sc, st)) return rc;
         launch_k(td3_target_head_kernel, rb, 256, 0, st, B, H2, w.t_h2, (int64_t)B * H2, critic_t.w3, critic_t.b3, cz, rewards, dones, cfg->gamma, ZC, w.target);
         if (int rc = check_launch("td3_target_head_kernel")) return rc;
         // ---- current Q, loss, backward (td3.py:178-186) ----
-        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, ZC, w.h1[0], w.h2[0], w.tensor, st, w.slabs, w.slab_cap)) return rc;
-        launch_k(td3_critic_head_kernel<false>, dim3(rb, ZC), 256, 0, st, B, H2, w.h2[0], (int64_t)B * H2, critic.w3, critic.b3, cz, w.target, 2.f / (float)B, w.dq,
-                                                                  w.dz2, w.loss_partial);
-        if (int rc = check_launch("td3_critic_head_kernel")) return rc;
-        SkinnyArgs s{};  // dW3 = dq^T @ h2, db3 = sum dq
-        s.X = w.h2[0], s.x_z = (int64_t)B * H2, s.ldx = H2, s.H = H2, s.B = B;
-        s.Y0 = w.dq, s.n0 = 1, s.ld0 = 1, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = B;
-        s.out_w = g_critic.w3, s.out_b = g_critic.b3, s.out_z = cz, s.transposed = 1;
-        FinJobs J{};
-        if (int rc = launch_skinny<1, true>(s, ZC, w.skinny + 2 * w.skinny_region, st, "td3_skinny_wgrad_kernel<w3>", &J)) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, ZC, w.h1[0], w.dz2, w.dz1, w, true, st, &J)) return rc;
+        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, ZC, w.h1[0], w.h2[0], w.sc, st)) return rc;
+        if (int rc = critic_loss_backward(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, ZC, w.h1[0], w.h2[0], w.target, 2.f / (float)B, w.dq,
+                                          w.dz2, w.dz1, w.loss_partial, w.sc, st))
+            return rc;
     }
     if (phases & CSTR_TD3_CRITIC_APPLY) {
-        ApplyArgs a{};
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
+        ApplyArgs a = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, critic_step, dev_sc, 0);
         a.adam_lo = T.critic_off[0], a.adam_hi = T.critic_off[0] + ZC * cz, a.polyak_lo = a.polyak_hi = 0;
-        const double bc1 = 1.0 - pow((double)cfg->beta1, (double)critic_step), bc2 = 1.0 - pow((double)cfg->beta2, (double)critic_step);
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = (float)((double)cfg->lr / bc1), a.bc2_sqrt = (float)sqrt(bc2);
-        a.tau = cfg->tau;
-        a.dev_scalars = dev_sc;
         a.loss_partial = w.loss_partial, a.n_loss_partial = ZC * rb, a.loss_scale = 1.f / (float)B, a.loss_acc = stt->losses;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<critic>")) return rc;
     }
     if (policy_step && (phases & CSTR_TD3_ACTOR_GRAD)) {
         // ---- actor loss = -Q1(s, pi(s)).mean() and its backward (td3.py:189-196) ----
-        if (int rc = forward_hidden(B, H1, H2, OBS, obs, nullptr, actor, 0, 1, w.a_h1, w.a_h2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+        if (int rc = forward_hidden(B, H1, H2, OBS, obs, nullptr, actor, 0, 1, w.a_h1, w.a_h2, w.sc, st)) return rc;
         launch_k(td3_actor_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor.w3, actor.b3, 0, nullptr, 0.f, 0.f, 0, 0, nullptr, (float2 *)w.a_pi);
         if (int rc = check_launch("td3_actor_head_kernel<pi>")) return rc;
-        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a_pi, critic, cz, 1, w.h1[0], w.h2[0], w.tensor, st, w.slabs, w.slab_cap)) return rc;
-        launch_k(td3_critic_head_kernel<true>, dim3(rb, 1), 256, 0, st, B, H2, w.h2[0], (int64_t)B * H2, critic.w3, critic.b3, cz, nullptr, 0.f, w.dq, w.dz2,
-                                                                 w.loss_partial);
-        if (int rc = check_launch("td3_critic_head_kernel<policy>")) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, w.a_pi, OBS + ACT), critic, g_critic, cz, 1, w.h1[0], w.dz2, w.dz1, w, false, st)) return rc;
+        if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a_pi, critic, cz, 1, w.h1[0], w.h2[0], w.sc, st)) return rc;
+        if (int rc = policy_critic_backward(B, H1, H2, critic, cz, w.h1[0], w.h2[0], w.dq, w.dz2, w.dz1, w.loss_partial, w.sc, st)) return rc;
         // through the critic's input layer and the tanh into the actor; dz2 of the actor reuses slab 1 of the dz2 buffer
         float *dz2a = w.dz2 + (int64_t)B * H2, *dz1a = w.dz1 + (int64_t)B * H1;
         launch_k(td3_actor_bwd_head_kernel, rb, 256, 0, st, B, H1, H2, w.dz1, critic.w1, (const float2 *)w.a_pi, actor.w3, w.a_h2, (float2 *)w.dpre, dz2a);
@@ -1366,18 +1225,13 @@ int cstr_td3_update(const cstr_td3_config *cfg, const cstr_td3_state *stt, const
         s.Y0 = w.dpre, s.n0 = ACT, s.ld0 = ACT, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = 0;
         s.out_w = g_actor.w3, s.out_b = g_actor.b3, s.out_z = 0, s.transposed = 1;
         FinJobs J{};
-        if (int rc = launch_skinny<ACT, true>(s, 1, w.skinny + 2 * w.skinny_region, st, "td3_skinny_wgrad_kernel<actor w3>", &J)) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, nullptr, OBS), actor, g_actor, 0, 1, w.a_h1, dz2a, dz1a, w, true, st, &J)) return rc;
+        if (int rc = launch_skinny<ACT, true>(s, 1, w.sc.skinny + 2 * w.sc.skinny_region, st, "td3_skinny_wgrad_kernel<actor w3>", J)) return rc;
+        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, nullptr, OBS), nullptr, actor, g_actor, 0, 1, w.a_h1, dz2a, dz1a, w.sc, J, st)) return rc;
     }
     if (policy_step && (phases & CSTR_TD3_ACTOR_APPLY)) {
         if (actor_step < 1) return fail_arg(CSTR_EINVAL, "td3_update: actor_step must be >= 1 on a policy step");
-        ApplyArgs a{};
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
+        ApplyArgs a = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, actor_step, dev_sc, 2);
         a.adam_lo = T.actor_off, a.adam_hi = T.actor_off + T.actor.size, a.polyak_lo = 0, a.polyak_hi = T.total;
-        const double bc1 = 1.0 - pow((double)cfg->beta1, (double)actor_step), bc2 = 1.0 - pow((double)cfg->beta2, (double)actor_step);
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = (float)((double)cfg->lr / bc1), a.bc2_sqrt = (float)sqrt(bc2);
-        a.tau = cfg->tau;
-        a.dev_scalars = dev_sc ? dev_sc + 2 : nullptr;
         a.loss_partial = w.loss_partial, a.n_loss_partial = rb, a.loss_scale = -1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 2 : nullptr;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<actor+polyak>")) return rc;
     }
@@ -1405,12 +1259,8 @@ int64_t cstr_sac_param_count(int32_t h1, int32_t h2) {
 int cstr_sac_layout(int32_t h1, int32_t h2, int64_t *offsets) {
     if (!offsets || h1 < 4 || h2 < 4 || (h1 & 3) || (h2 & 3)) return fail_arg(CSTR_EINVAL, "sac_layout: bad sizes or null output");
     const Td3Layout T = td3_layout(h1, h2, 2 * ACT);
-    const int64_t base[3] = {T.actor_off, T.critic_off[0], T.critic_off[1]};
-    for (int n = 0; n < 3; ++n) {
-        const NetLayout &L = n == 0 ? T.actor : T.critic;
-        const int64_t o[6] = {L.w1, L.b1, L.w2, L.b2, L.w3, L.b3};
-        for (int k = 0; k < 6; ++k) offsets[n * 6 + k] = base[n] + o[k];
-    }
+    put_offsets(offsets, 0, T.actor_off, T.actor);
+    for (int n = 1; n < 3; ++n) put_offsets(offsets, n, T.critic_off[n - 1], T.critic);
     offsets[18] = T.total;      // log_ent_coef
     offsets[19] = T.total + 4;  // block size
     return 0;
@@ -1426,18 +1276,11 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
                     int32_t phases, void *stream) {
     if (int rc = check_sac_cfg(cfg)) return rc;
     if (!(phases & CSTR_TD3_ALL) || (phases & ~CSTR_TD3_ALL)) return fail_arg(CSTR_EINVAL, "sac_update: phases must be a non-empty subset of CSTR_TD3_ALL");
-    if (!stt || !stt->params || !stt->targets || !stt->grads || !stt->adam_m || !stt->adam_v || !stt->workspace)
-        return fail_arg(CSTR_EINVAL, "sac_update: null state pointer");
-    if (!obs || !actions || !next_obs || !dones || !rewards) return fail_arg(CSTR_EINVAL, "sac_update: null batch pointer");
-    if (!aligned(obs, 16) || !aligned(next_obs, 16) || !aligned(actions, 8) || (eps_pi && !aligned(eps_pi, 8)) || (eps_next && !aligned(eps_next, 8)) ||
-        !aligned(stt->params, 16) || !aligned(stt->targets, 16) || !aligned(stt->grads, 16) || !aligned(stt->adam_m, 16) || !aligned(stt->adam_v, 16) ||
-        !aligned(stt->workspace, 16))
-        return fail_arg(CSTR_EALIGN, "sac_update: 16 B (obs/params/workspace) / 8 B (actions, noise) alignment");
+    if (int rc = check_update("sac", stt, cstr_sac_workspace_bytes(cfg), obs, actions, next_obs, dones, rewards, n_updates, adam_step, 0)) return rc;
+    if ((eps_pi && !aligned(eps_pi, 8)) || (eps_next && !aligned(eps_next, 8))) return fail_arg(CSTR_EALIGN, "sac_update: eps_pi / eps_next need 8 B alignment");
     const int B = cfg->batch, H1 = cfg->h1, H2 = cfg->h2;
     Workspace w = carve(stt->workspace, B, H1, H2);
-    w.tensor = cfg->gemm_mode;
-    if (stt->workspace_bytes < w.floats * (int64_t)sizeof(float)) return fail_arg(CSTR_EINVAL, "sac_update: workspace too small (cstr_sac_workspace_bytes)");
-    if (n_updates < 1 || adam_step < 1) return fail_arg(CSTR_EINVAL, "sac_update: counters are 1-based (value after this update)");
+    w.sc.tensor = cfg->gemm_mode;
     const Td3Layout T = td3_layout(H1, H2, 2 * ACT);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t cz = T.critic.size, ent = T.total;
@@ -1445,97 +1288,77 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
     const Net critic_t = net_at(stt->targets, T.critic_off[0], T.critic);
     const Net g_actor = net_at(stt->grads, T.actor_off, T.actor), g_critic = net_at(stt->grads, T.critic_off[0], T.critic);
     const int rb = w.n_row_blocks;
-    const double bc1 = 1.0 - pow((double)cfg->beta1, (double)adam_step), bc2 = 1.0 - pow((double)cfg->beta2, (double)adam_step);
-    const float step_size = (float)((double)cfg->lr / bc1), bc2_sqrt = (float)sqrt(bc2);
 
     const float *dev_sc = stt->counters ? w.scalars : nullptr;  // graph mode: per-update scalars live on the device (td3_tick_kernel)
+    const ApplyArgs adam = adam_args(stt, cfg->lr, cfg->beta1, cfg->beta2, cfg->eps, cfg->tau, adam_step, dev_sc, 0);  // one step for all three optimisers
     // log_ent_coef: gradient and Adam step in one launch when nothing sits between them; gradient only when the caller all-reduces
     // between the phases, or when a peer communicator averages it inside the critic apply (its slot joins that Adam range)
     const bool fused_ent = !stt->peer && (phases & (CSTR_TD3_CRITIC_GRAD | CSTR_TD3_CRITIC_APPLY)) == (CSTR_TD3_CRITIC_GRAD | CSTR_TD3_CRITIC_APPLY);
     auto ent_coef = [&](int mode) {
         launch_k(sac_ent_coef_kernel, 1, 256, 0, st, B, rb, w.lp_partial, cfg->target_entropy, stt->params + ent, stt->grads + ent, stt->adam_m + ent,
-                                              stt->adam_v + ent, cfg->beta1, cfg->beta2, cfg->eps, step_size, bc2_sqrt, dev_sc ? 1 : 0, w.scalars,
+                                              stt->adam_v + ent, cfg->beta1, cfg->beta2, cfg->eps, adam.step_size, adam.bc2_sqrt, dev_sc ? 1 : 0, w.scalars,
                                               stt->losses, mode);
         return check_launch("sac_ent_coef_kernel");
     };
-    if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD)) {
-        launch_k(td3_tick_kernel, 1, 32, 0, st, stt->counters, w.scalars, 1, (double)cfg->lr, (double)cfg->beta1, (double)cfg->beta2, -1.0, -1.0, -1.0);
-        if (int rc = check_launch("td3_tick_kernel")) return rc;
-    }
+    if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD))
+        if (int rc = launch_tick(stt, w.scalars, true, cfg->lr, cfg->beta1, cfg->beta2, -1.0, -1.0, -1.0, st)) return rc;
     if (phases & CSTR_TD3_CRITIC_GRAD) {
     // ---- actions_pi, log_prob of the current actor (sac.py:222-223) and the entropy-coefficient step (:226-243) ----
-    if (int rc = forward_hidden(B, H1, H2, OBS, obs, nullptr, actor, 0, 1, w.a_h1, w.a_h2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS, obs, nullptr, actor, 0, 1, w.a_h1, w.a_h2, w.sc, st)) return rc;
     launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor.w3, actor.b3, (const float2 *)eps_pi, cfg->seed, (uint32_t)n_updates, dev_sc, 0u, (float2 *)w.a_pi,
                                              w.logp, (float2 *)w.std_eps, (float2 *)w.raw_log_std, w.lp_partial);
     if (int rc = check_launch("sac_actor_head_kernel")) return rc;
     // one launch when nothing sits between gradient and step; split around the caller's all-reduce of grads[critics .. log_ent_coef] otherwise
     if (int rc = ent_coef(fused_ent ? 3 : 1)) return rc;
     // ---- target (sac.py:245-254): next action from the CURRENT actor (scratch: the dz slabs are free here) ----
-    if (int rc = forward_hidden(B, H1, H2, OBS, next_obs, nullptr, actor, 0, 1, w.dz1, w.dz2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS, next_obs, nullptr, actor, 0, 1, w.dz1, w.dz2, w.sc, st)) return rc;
     launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.dz2, actor.w3, actor.b3, (const float2 *)eps_next, cfg->seed, (uint32_t)n_updates, dev_sc, 1u,
                                              (float2 *)w.next_act, w.next_logp, nullptr, nullptr, nullptr);
     if (int rc = check_launch("sac_actor_head_kernel<next>")) return rc;
-    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, next_obs, w.next_act, critic_t, cz, 2, w.t_h1, w.t_h2, w.tensor, st, w.slabs, w.slab_cap)) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, next_obs, w.next_act, critic_t, cz, 2, w.t_h1, w.t_h2, w.sc, st)) return rc;
     launch_k(sac_target_head_kernel, rb, 256, 0, st, B, H2, w.t_h2, (int64_t)B * H2, critic_t.w3, critic_t.b3, cz, rewards, dones, w.next_logp, w.scalars,
                                               cfg->gamma, w.target);
     if (int rc = check_launch("sac_target_head_kernel")) return rc;
     // ---- critics (sac.py:256-268): loss = 0.5 * sum_i mse ----
-    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, 2, w.h1[0], w.h2[0], w.tensor, st, w.slabs, w.slab_cap)) return rc;
-    launch_k(td3_critic_head_kernel<false>, dim3(rb, 2), 256, 0, st, B, H2, w.h2[0], (int64_t)B * H2, critic.w3, critic.b3, cz, w.target, 1.f / (float)B, w.dq,
-                                                              w.dz2, w.loss_partial);
-    if (int rc = check_launch("td3_critic_head_kernel<sac>")) return rc;
-    {
-        SkinnyArgs s{};
-        s.X = w.h2[0], s.x_z = (int64_t)B * H2, s.ldx = H2, s.H = H2, s.B = B;
-        s.Y0 = w.dq, s.n0 = 1, s.ld0 = 1, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = B;
-        s.out_w = g_critic.w3, s.out_b = g_critic.b3, s.out_z = cz, s.transposed = 1;
-        FinJobs J{};
-        if (int rc = launch_skinny<1, true>(s, 2, w.skinny + 2 * w.skinny_region, st, "td3_skinny_wgrad_kernel<w3>", &J)) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, 2, w.h1[0], w.dz2, w.dz1, w, true, st, &J)) return rc;
-    }
+    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, actions, critic, cz, 2, w.h1[0], w.h2[0], w.sc, st)) return rc;
+    if (int rc = critic_loss_backward(B, H1, H2, td3_src(obs, actions, OBS + ACT), critic, g_critic, cz, 2, w.h1[0], w.h2[0], w.target, 1.f / (float)B, w.dq, w.dz2,
+                                      w.dz1, w.loss_partial, w.sc, st))
+        return rc;
     }  // CRITIC_GRAD
     if (phases & CSTR_TD3_CRITIC_APPLY) {
         if (!fused_ent && !stt->peer)
             if (int rc = ent_coef(2)) return rc;
-        ApplyArgs a{};
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
+        ApplyArgs a = adam;
         a.adam_lo = T.critic_off[0], a.adam_hi = T.total, a.polyak_lo = a.polyak_hi = 0;
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = step_size, a.bc2_sqrt = bc2_sqrt, a.tau = cfg->tau;
-        a.dev_scalars = dev_sc;
         a.loss_partial = w.loss_partial, a.n_loss_partial = 2 * rb, a.loss_scale = 0.5f / (float)B, a.loss_acc = stt->losses;
         if (stt->peer) a.adam_hi = T.total + 4;  // the log_ent_coef slot rides in the same averaged Adam range (same formulas, same step size)
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<sac critic>")) return rc;
     }
     if (phases & CSTR_TD3_ACTOR_GRAD) {
     // ---- actor (sac.py:270-281): (ent_coef * log_prob - min_i Q_i(s, a_pi)).mean() with the updated critics ----
-    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a_pi, critic, cz, 2, w.h1[0], w.h2[0], w.tensor, st, w.slabs, w.slab_cap)) return rc;
+    if (int rc = forward_hidden(B, H1, H2, OBS + ACT, obs, w.a_pi, critic, cz, 2, w.h1[0], w.h2[0], w.sc, st)) return rc;
     launch_k(sac_qmin_head_kernel, rb, 256, 0, st, B, H2, w.h2[0], (int64_t)B * H2, critic.w3, critic.b3, cz, w.logp, w.scalars, w.dz2, w.loss_partial);
     if (int rc = check_launch("sac_qmin_head_kernel")) return rc;
-    if (int rc = backward_hidden(B, H1, H2, td3_src(obs, w.a_pi, OBS + ACT), critic, g_critic, cz, 2, w.h1[0], w.dz2, w.dz1, w, false, st)) return rc;
+    if (int rc = backward_dz1(B, H1, H2, critic, cz, 2, w.h1[0], w.dz2, w.dz1, w.sc, st)) return rc;
     // the actor's dz2 / dz1 live in the target-activation slabs (free since the target was formed)
     launch_k(sac_actor_bwd_head_kernel, rb, 256, 0, st, B, H1, H2, w.dz1, (int64_t)B * H1, critic.w1, cz, (const float2 *)w.a_pi, (const float2 *)w.std_eps,
                                                  (const float2 *)w.raw_log_std, w.scalars, actor.w3, w.a_h2, (float4 *)w.dpre4, w.t_h2);
     if (int rc = check_launch("sac_actor_bwd_head_kernel")) return rc;
-    {
-        SkinnyArgs s{};  // d[mu; log_std] head = dpre4^T @ h2a, bias = sum dpre4
-        s.X = w.a_h2, s.x_z = 0, s.ldx = H2, s.H = H2, s.B = B;
-        s.Y0 = w.dpre4, s.n0 = 2 * ACT, s.ld0 = 2 * ACT, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = 0;
-        s.out_w = g_actor.w3, s.out_b = g_actor.b3, s.out_z = 0, s.transposed = 1;
-        FinJobs J{};
-        if (int rc = launch_skinny<2 * ACT, true>(s, 1, w.skinny + 2 * w.skinny_region, st, "td3_skinny_wgrad_kernel<sac head>", &J)) return rc;
-        if (int rc = backward_hidden(B, H1, H2, td3_src(obs, nullptr, OBS), actor, g_actor, 0, 1, w.a_h1, w.t_h2, w.t_h1, w, true, st, &J)) return rc;
-    }
+    SkinnyArgs s{};  // d[mu; log_std] head = dpre4^T @ h2a, bias = sum dpre4
+    s.X = w.a_h2, s.x_z = 0, s.ldx = H2, s.H = H2, s.B = B;
+    s.Y0 = w.dpre4, s.n0 = 2 * ACT, s.ld0 = 2 * ACT, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = 0;
+    s.out_w = g_actor.w3, s.out_b = g_actor.b3, s.out_z = 0, s.transposed = 1;
+    FinJobs J{};
+    if (int rc = launch_skinny<2 * ACT, true>(s, 1, w.sc.skinny + 2 * w.sc.skinny_region, st, "td3_skinny_wgrad_kernel<sac head>", J)) return rc;
+    if (int rc = backward_hidden(B, H1, H2, td3_src(obs, nullptr, OBS), nullptr, actor, g_actor, 0, 1, w.a_h1, w.t_h2, w.t_h1, w.sc, J, st)) return rc;
     }  // ACTOR_GRAD
     if (phases & CSTR_TD3_ACTOR_APPLY) {
-        ApplyArgs a{};
-        a.p = stt->params, a.t = stt->targets, a.g = stt->grads, a.m = stt->adam_m, a.v = stt->adam_v;
+        ApplyArgs a = adam;
         a.adam_lo = T.actor_off, a.adam_hi = T.actor_off + T.actor.size;
         // `gradient_step % target_update_interval == 0` (:284) with gradient_step the index inside the current train() call
         const int64_t loop_index = cfg->local_step > 0 ? (int64_t)cfg->local_step - 1 : n_updates - 1;
         const bool sync_targets = (loop_index % cfg->target_update_interval) == 0;
         a.polyak_lo = sync_targets ? T.critic_off[0] : 0, a.polyak_hi = sync_targets ? T.total : 0;
-        a.beta1 = cfg->beta1, a.beta2 = cfg->beta2, a.eps = cfg->eps, a.step_size = step_size, a.bc2_sqrt = bc2_sqrt, a.tau = cfg->tau;
-        a.dev_scalars = dev_sc;
         a.loss_partial = w.loss_partial, a.n_loss_partial = rb, a.loss_scale = 1.f / (float)B, a.loss_acc = stt->losses ? stt->losses + 2 : nullptr;
         if (int rc = launch_apply(a, stt->peer, stt->grads, st, "td3_apply_kernel<sac actor+polyak>")) return rc;
     }
