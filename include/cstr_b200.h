@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define CSTR_B200_ABI_VERSION 16
+#define CSTR_B200_ABI_VERSION 17
 
 #define CSTR_EINVAL (-1)   /* bad argument (null pointer, negative size, unknown mode) */
 #define CSTR_EALIGN (-2)   /* pointer not aligned for the vectorised access the layout implies */
@@ -411,6 +411,34 @@ int cstr_rollout_fused(const cstr_env_params *p, int64_t n, int64_t K, int math_
                        int32_t *step_count, int32_t *episode, double *static_base, int64_t rows,
                        int64_t pos0, float *records, double *reward_sum, const cstr_episode_stats *stats /* nullable */,
                        void *stream);
+
+/* VecNormalize variant.  Replaces, per env step, the same reference code as cstr_rollout_fused plus VecNormalize.step_wait's
+ * statistics (core/common/vec_env/vec_normalize.py:174-223) and _store_transition's original-observation rule
+ * (core/common/off_policy_algorithm.py:468-494):
+ *   - the actor reads normalize_obs(obs) with the statistics in effect at that step (raw obs when norm_obs == 0);
+ *   - training != 0: obs_rms is updated with the post-reset observations of ALL n reactors (norm_obs != 0), returns = returns * gamma
+ *     + reward and ret_rms updated with them (whatever norm_reward is); returns of done rows are then zeroed (also when training == 0);
+ *   - the records hold the raw obs, action, reward, done and timeout; next_obs of a done row is
+ *     unnormalize_obs(normalize_obs(terminal obs)) with the statistics AFTER that step's update (differs from the terminal
+ *     observation where clip_obs binds).
+ * Each step needs statistics reduced over every reactor at the previous one, so the call enqueues one kernel launch per step (plus
+ * one small launch that finishes the last step's done rows); the merge of the per-CTA sums is done in a fixed order, so the
+ * statistics are the same bits from run to run.  No host synchronisation.  Arguments as for cstr_rollout_fused; the
+ * multi-agent rollout has no VecNormalize variant.                                                                           */
+typedef struct cstr_rollout_norm {
+    double *stats;     /* 16 doubles on the device, the layout of cstr_norm_update (in/out)                                         */
+    double *returns;   /* (n,) double VecNormalize.returns (in/out)                                                                 */
+    void *workspace;   /* cstr_rollout_norm_workspace_bytes(n, actor_mode) bytes, 16-byte aligned, zeroed once before the first call */
+    double gamma, epsilon, clip_obs; /* VecNormalize.gamma / epsilon / clip_obs */
+    int32_t training, norm_obs;      /* VecNormalize.training / norm_obs        */
+} cstr_rollout_norm;
+int64_t cstr_rollout_norm_workspace_bytes(int64_t n, int actor_mode);
+int cstr_rollout_fused_norm(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, int actor_mode,
+                            const cstr_actor_f32 *actor, const void *packed_bf16, float sigma,
+                            const float *noise, int warmup, uint32_t t_base, float *state,
+                            int32_t *step_count, int32_t *episode, double *static_base, int64_t rows,
+                            int64_t pos0, float *records, double *reward_sum, const cstr_episode_stats *stats /* nullable */,
+                            const cstr_rollout_norm *norm, void *stream);
 
 /* Multi-agent variant (BASELINE config #5: the two reactors as two agents).  Replaces OffMultiAgentPolicyAlgorithm._sample_action +
  * MultiAgentBasePolicy.predict + env.step + _store_transition + ReplayBuffer.add

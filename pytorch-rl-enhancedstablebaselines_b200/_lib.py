@@ -9,7 +9,7 @@ from typing import Optional
 
 from . import _build
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 MATH_STRICT, MATH_FAST = 0, 1
 INIT_RANDOM, INIT_STATIC = 0, 1
 REC_FLOATS = 16
@@ -55,6 +55,13 @@ class NormParams(Structure):
 
     _fields_ = [("stats", c_void_p), ("epsilon", c_double), ("clip_obs", c_double), ("clip_reward", c_double),
                 ("norm_obs", c_int32), ("norm_reward", c_int32)]
+
+
+class RolloutNorm(Structure):
+    """struct cstr_rollout_norm"""
+
+    _fields_ = [("stats", c_void_p), ("returns", c_void_p), ("workspace", c_void_p), ("gamma", c_double), ("epsilon", c_double),
+                ("clip_obs", c_double), ("training", c_int32), ("norm_obs", c_int32)]
 
 
 class Td3Config(Structure):
@@ -151,6 +158,9 @@ _SIGNATURES = {
     "cstr_peer_error": (c_int, [POINTER(PeerComm), POINTER(c_uint32), P]),
     "cstr_rollout_fused": (c_int, [POINTER(EnvParams), c_int64, c_int64, c_int, c_int, POINTER(ActorF32), P, c_float, P, c_int,
                                    c_uint32, P, P, P, P, c_int64, c_int64, P, P, POINTER(EpisodeStatsStruct), P]),
+    "cstr_rollout_norm_workspace_bytes": (c_int64, [c_int64, c_int]),
+    "cstr_rollout_fused_norm": (c_int, [POINTER(EnvParams), c_int64, c_int64, c_int, c_int, POINTER(ActorF32), P, c_float, P, c_int,
+                                        c_uint32, P, P, P, P, c_int64, c_int64, P, P, POINTER(EpisodeStatsStruct), POINTER(RolloutNorm), P]),
     "cstr_rollout_fused_multi": (c_int, [POINTER(EnvParams), c_int64, c_int64, c_int, P, c_int, c_uint32, P, P, P, P, c_int64, c_int64, P, P,
                                          POINTER(EpisodeStatsStruct), P]),
     "cstr_actor_pack_bf16": (c_int64, [POINTER(ActorF32), P, P]),

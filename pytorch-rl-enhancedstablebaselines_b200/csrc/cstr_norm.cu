@@ -53,17 +53,6 @@ norm_reduce_kernel(int64_t n, const float4 *__restrict__ obs, const float *__res
     }
 }
 
-// RunningMeanStd.update_from_moments (running_mean_std.py:43-56) for the 4 observation dims and the return
-__device__ __forceinline__ void update_from_moments(double &mean, double &var, double &count, double bmean, double bvar, double bcount) {
-    const double delta = bmean - mean;
-    const double tot = count + bcount;
-    const double new_mean = mean + delta * bcount / tot;
-    const double m2 = var * count + bvar * bcount + delta * delta * count * bcount / (count + bcount);
-    mean = new_mean;
-    var = m2 / (count + bcount);
-    count = bcount + count;
-}
-
 __global__ void norm_finalize_kernel(int64_t n, int update_obs, int update_ret, double *__restrict__ stats, double *__restrict__ scratch) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
     const double bn = (double)n;

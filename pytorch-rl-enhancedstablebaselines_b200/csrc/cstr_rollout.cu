@@ -29,13 +29,15 @@ constexpr int ROLL_THREADS = ROLL_PARTS * 32;
 // warp-uniform 16-byte load of a W2 row piece and every h1 read is one wavefront.  Register-blocking FOUR reactors per thread
 // makes one W2 load feed 16 FMAs per lane instead of 4: 28 wavefronts per 192 FMA instructions instead of 64.
 
-template <int MODE, int KIND>
+// NORM (cstr_rollout_fused_norm, K == 1): the actor reads the normalised observation, done rows keep their raw terminal observation until
+// the statistics that include this step exist, and the CTA's moment sums go to norm_merge.
+template <int MODE, int KIND, bool NORM>
 __global__ void __launch_bounds__(ROLL_THREADS, 1)
 rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor_a, cstr_actor_f32 actor_b, int n_agents, float sigma,
                    const float2 *__restrict__ noise, int warmup,
                    uint32_t t_base, float4 *__restrict__ state, int32_t *__restrict__ step_count, int32_t *__restrict__ episode,
                    double *static_base, int64_t rows, int64_t pos0, float4 *__restrict__ records, double *reward_sum, cstr_episode_stats stats,
-                   int has_stats) {
+                   int has_stats, NormLaunch nl) {
     extern __shared__ float h1[];  // [H1][ROLL_M] (reused for the partial heads [PARTS][4][ROLL_M] once layer 2 is done), then the state column
     constexpr int NOUT = KIND == CSTR_ACTOR_GAUSSIAN ? 4 : 2;
     const int lane = threadIdx.x & 31, part = threadIdx.x >> 5;
@@ -56,6 +58,12 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
     double acc_r = 0.0;
     double ep_ret = (has_stats && live) ? stats.ep_return[i] : 0.0;
     uint4 cache = make_uint4(0, 0, 0, 0);
+    double nacc[NORM_SUMS];
+    if constexpr (NORM) {
+#pragma unroll
+        for (int j = 0; j < NORM_SUMS; ++j) nacc[j] = 0.0;
+        if (live) norm_fix_pending(nl, i, n, records);
+    }
 
     for (int64_t k = 0; k < K; ++k) {
         const uint32_t g = t_base + (uint32_t)k;
@@ -74,7 +82,11 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
           float mu_agent[2] = {0.f, 0.f};
           for (int agent = 0; agent < n_agents; ++agent) {
             const cstr_actor_f32 &actor = agent ? actor_b : actor_a;
-            if (owner) s_state[m] = s;
+            if constexpr (NORM) {
+                if (owner) s_state[m] = nl.norm_obs ? norm_obs4(s, nl) : s;
+            } else {
+                if (owner) s_state[m] = s;
+            }
             __syncthreads();
             float4 sv[ROLL_R];
 #pragma unroll
@@ -192,7 +204,14 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
                                                         : step_fast_f32(s, env_a, sc, (float)p.target_c2, p.max_steps);
         if (live) {
             const int64_t row = (pos0 + k) % rows;
-            store_record(records + ((size_t)row * n + i) * 4, obs, s, buf_a, r.reward, r.truncated);
+            float4 next_obs = s;
+            if constexpr (NORM) {
+                if (r.truncated && nl.norm_obs) {
+                    if (nl.training) nl.pending[i] = 1;  // the round trip needs S_{k+1}: the next launch (or the fix-up kernel) writes it
+                    else next_obs = norm_round_trip4(s, nl);  // frozen statistics: S_{k+1} == S_k
+                }
+            }
+            store_record(records + ((size_t)row * n + i) * 4, obs, next_obs, buf_a, r.reward, r.truncated);
             acc_r += (double)r.reward;
             episode_account(stats, has_stats != 0, ep_ret, r.reward, r.truncated, sc);
         }
@@ -200,6 +219,12 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
             if (live) s = reset_f32_env(p, i, ep, static_base);
             sc = 0;
         }
+        if constexpr (NORM) {
+            if (live) norm_account(nl, i, s, r.reward, r.truncated, nacc);
+        }
+    }
+    if constexpr (NORM) {
+        if (nl.training) norm_merge<ROLL_THREADS>(nl, n, nacc, reinterpret_cast<double *>(h1));
     }
     if (!owner) return;
     if (live) {
@@ -215,6 +240,13 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
     }
 }
 
+// the done rows of the last step of a call: their final next_obs, with the statistics that launch left
+__global__ void __launch_bounds__(256) rollout_norm_fix_kernel(int64_t n, NormLaunch nl, float4 *__restrict__ records) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    norm_fix_pending(nl, i, n, records);
+}
+
 }  // namespace cstr
 
 using namespace cstr;
@@ -223,19 +255,19 @@ using namespace cstr;
 int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, const cstr_actor_f32 *actor,
                            const void *packed_bf16, float sigma, const float *noise, int warmup, uint32_t t_base, float *state,
                            int32_t *step_count, int32_t *episode, double *static_base, int64_t rows, int64_t pos0, float *records,
-                           double *reward_sum, const cstr_episode_stats *stats, void *stream);
+                           double *reward_sum, const cstr_episode_stats *stats, const NormLaunch *nl, void *stream);
 
 static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, int actor_mode, const cstr_actor_f32 *actor,
                               const cstr_actor_f32 *actor_b, const void *packed_bf16, float sigma, const float *noise, int warmup, uint32_t t_base,
                               float *state, int32_t *step_count, int32_t *episode, double *static_base, int64_t rows, int64_t pos0, float *records,
-                              double *reward_sum, const cstr_episode_stats *stats, void *stream);
+                              double *reward_sum, const cstr_episode_stats *stats, const NormLaunch *nl, void *stream);
 
 extern "C" int cstr_rollout_fused(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, int actor_mode,
                                   const cstr_actor_f32 *actor, const void *packed_bf16, float sigma, const float *noise, int warmup,
                                   uint32_t t_base, float *state, int32_t *step_count, int32_t *episode, double *static_base,
                                   int64_t rows, int64_t pos0, float *records, double *reward_sum, const cstr_episode_stats *stats, void *stream) {
     return rollout_fused_impl(p, n, K, math_mode, actor_mode, actor, nullptr, packed_bf16, sigma, noise, warmup, t_base, state, step_count, episode,
-                              static_base, rows, pos0, records, reward_sum, stats, stream);
+                              static_base, rows, pos0, records, reward_sum, stats, nullptr, stream);
 }
 
 extern "C" int cstr_rollout_fused_multi(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, const cstr_actor_f32 *agent_actors, int warmup,
@@ -249,13 +281,13 @@ extern "C" int cstr_rollout_fused_multi(const cstr_env_params *p, int64_t n, int
     }
     static const cstr_actor_f32 none = {};
     return rollout_fused_impl(p, n, K, math_mode, 0, agent_actors ? agent_actors : &none, agent_actors ? agent_actors + 1 : &none, nullptr, 0.0f, nullptr,
-                              warmup, t_base, state, step_count, episode, static_base, rows, pos0, records, reward_sum, stats, stream);
+                              warmup, t_base, state, step_count, episode, static_base, rows, pos0, records, reward_sum, stats, nullptr, stream);
 }
 
 static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, int actor_mode, const cstr_actor_f32 *actor,
                               const cstr_actor_f32 *actor_b, const void *packed_bf16, float sigma, const float *noise, int warmup, uint32_t t_base,
                               float *state, int32_t *step_count, int32_t *episode, double *static_base, int64_t rows, int64_t pos0, float *records,
-                              double *reward_sum, const cstr_episode_stats *stats, void *stream) {
+                              double *reward_sum, const cstr_episode_stats *stats, const NormLaunch *nl, void *stream) {
     if (!p || n < 0 || K < 0 || !state || !step_count || !episode || !records || rows <= 0 || pos0 < 0)
         return fail_arg(CSTR_EINVAL, "rollout: null pointer or bad size");
     if (p->init_mode == CSTR_INIT_STATIC && !static_base) return fail_arg(CSTR_EINVAL, "static init_mode needs static_base");
@@ -276,34 +308,90 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
     }
     if (actor_mode == 1 && !warmup)
         return cstr_rollout_tc_launch(p, n, K, math_mode, actor, packed_bf16, sigma, noise, warmup, t_base, state, step_count, episode,
-                                      static_base, rows, pos0, records, reward_sum, stats, stream);
+                                      static_base, rows, pos0, records, reward_sum, stats, nl, stream);
     if (actor_mode != 0 && actor_mode != 1) return fail_arg(CSTR_EINVAL, "rollout: unknown actor_mode");
     cstr_actor_f32 a = {}, b2nd = {};
     if (actor) a = *actor;
     if (actor_b) b2nd = *actor_b;
     const int n_agents = actor_b ? 2 : 1;
     const size_t h1_floats = (size_t)a.H1 * ROLL_M > (size_t)ROLL_PARTS * 4 * ROLL_M ? (size_t)a.H1 * ROLL_M : (size_t)ROLL_PARTS * 4 * ROLL_M;
-    const size_t smem = warmup ? 0 : h1_floats * sizeof(float) + ROLL_M * sizeof(float4);
+    size_t smem = warmup ? 0 : h1_floats * sizeof(float) + ROLL_M * sizeof(float4);
+    if (nl && smem < (ROLL_PARTS * NORM_SUMS + 1) * sizeof(double)) smem = (ROLL_PARTS * NORM_SUMS + 1) * sizeof(double);  // norm_merge's sums
     if (smem > 227 * 1024) return fail_arg(CSTR_EINVAL, "rollout: H1 too large for the fp32 path (max 448)");
     const int grid = (int)((n + ROLL_M - 1) / ROLL_M);
     cudaStream_t st = (cudaStream_t)stream;
     int rc = 0;
 #define CSTR_LAUNCH_ROLL(MODE, KIND)                                                                                                       \
     do {                                                                                                                                   \
-        rc = check_cuda(cudaFuncSetAttribute(rollout_f32_kernel<MODE, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "smem attr"); \
+        rc = check_cuda(cudaFuncSetAttribute(rollout_f32_kernel<MODE, KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "smem attr"); \
         if (!rc)                                                                                                                           \
-            rollout_f32_kernel<MODE, KIND><<<grid, ROLL_THREADS, smem, st>>>(*p, n, K, a, b2nd, n_agents, sigma, (const float2 *)noise, warmup, t_base, (float4 *)state, \
-                                                                       step_count, episode, static_base, rows, pos0, (float4 *)records, reward_sum, st_copy, has_stats); \
+            rollout_f32_kernel<MODE, KIND, false><<<grid, ROLL_THREADS, smem, st>>>(*p, n, K, a, b2nd, n_agents, sigma, (const float2 *)noise, warmup, t_base, (float4 *)state, \
+                                                                       step_count, episode, static_base, rows, pos0, (float4 *)records, reward_sum, st_copy, has_stats, NormLaunch{}); \
     } while (0)
     cstr_episode_stats st_copy = {};
     const int has_stats = stats != nullptr;
     if (stats) {
         st_copy = *stats;
     }
+#define CSTR_LAUNCH_ROLL_NORM(MODE, KIND)                                                                                                  \
+    do {                                                                                                                                   \
+        rc = check_cuda(cudaFuncSetAttribute(rollout_f32_kernel<MODE, KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "smem attr"); \
+        if (!rc)                                                                                                                           \
+            rollout_f32_kernel<MODE, KIND, true><<<grid, ROLL_THREADS, smem, st>>>(*p, n, K, a, b2nd, n_agents, sigma, (const float2 *)noise, warmup,     \
+                                                                            t_base, (float4 *)state, step_count, episode, static_base, rows, pos0,  \
+                                                                            (float4 *)records, reward_sum, st_copy, has_stats, *nl);               \
+    } while (0)
     const bool gauss = a.kind == CSTR_ACTOR_GAUSSIAN;
-    if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
+    if (nl) {
+        if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
+        else { if (gauss) CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_FAST, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_FAST, CSTR_ACTOR_TANH); }
+    } else if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
     else { if (gauss) CSTR_LAUNCH_ROLL(CSTR_MATH_FAST, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL(CSTR_MATH_FAST, CSTR_ACTOR_TANH); }
 #undef CSTR_LAUNCH_ROLL
+#undef CSTR_LAUNCH_ROLL_NORM
     if (rc) return rc;
     return check_launch("rollout_f32_kernel");
+}
+
+// workspace of cstr_rollout_fused_norm: [ticket (16 B)][partials: grid x NORM_SUMS doubles][pending: n bytes]; both kernels use 128-reactor CTAs
+static int64_t norm_grid(int64_t n) { return (n + ROLL_M - 1) / ROLL_M; }
+
+extern "C" int64_t cstr_rollout_norm_workspace_bytes(int64_t n, int actor_mode) {
+    if (n < 0 || (actor_mode != 0 && actor_mode != 1)) return fail_arg(CSTR_EINVAL, "rollout_norm_workspace_bytes: bad size or actor_mode");
+    return 16 + norm_grid(n) * NORM_SUMS * (int64_t)sizeof(double) + ((n + 15) & ~(int64_t)15);
+}
+
+extern "C" int cstr_rollout_fused_norm(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, int actor_mode,
+                                       const cstr_actor_f32 *actor, const void *packed_bf16, float sigma, const float *noise, int warmup,
+                                       uint32_t t_base, float *state, int32_t *step_count, int32_t *episode, double *static_base,
+                                       int64_t rows, int64_t pos0, float *records, double *reward_sum, const cstr_episode_stats *stats,
+                                       const cstr_rollout_norm *norm, void *stream) {
+    if (!norm || !norm->stats || !norm->returns || !norm->workspace) return fail_arg(CSTR_EINVAL, "rollout_norm: stats, returns or workspace missing");
+    if (!aligned(norm->stats, 8) || !aligned(norm->returns, 8) || !aligned(norm->workspace, 16))
+        return fail_arg(CSTR_EALIGN, "rollout_norm: stats/returns 8-byte, workspace 16-byte alignment");
+    if (rows <= 0 || pos0 < 0 || K < 0) return fail_arg(CSTR_EINVAL, "rollout_norm: bad size");
+    uint8_t *ws = (uint8_t *)norm->workspace;
+    NormLaunch nl;
+    nl.stats = norm->stats;
+    nl.returns = norm->returns;
+    nl.ticket = (uint32_t *)ws;
+    nl.partials = (double *)(ws + 16);
+    nl.pending = ws + 16 + norm_grid(n) * NORM_SUMS * sizeof(double);
+    nl.gamma = norm->gamma;
+    nl.eps = norm->epsilon;
+    nl.clip = norm->clip_obs;
+    nl.training = norm->training != 0;
+    nl.norm_obs = norm->norm_obs != 0;
+    // one launch per env step: step k+1 acts on statistics reduced over every reactor at step k
+    for (int64_t k = 0; k < K; ++k) {
+        nl.prev_row = (pos0 + k + rows - 1) % rows;
+        const float *nz = noise ? noise + (size_t)k * n * 2 : nullptr;
+        if (int rc = rollout_fused_impl(p, n, 1, math_mode, actor_mode, actor, nullptr, packed_bf16, sigma, nz, warmup, t_base + (uint32_t)k, state,
+                                        step_count, episode, static_base, rows, pos0 + k, records, reward_sum, stats, &nl, stream))
+            return rc;
+    }
+    if (n == 0 || K == 0 || !nl.training || !nl.norm_obs) return 0;
+    nl.prev_row = (pos0 + K - 1) % rows;
+    rollout_norm_fix_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, nl, (float4 *)records);
+    return check_launch("rollout_norm_fix_kernel");
 }

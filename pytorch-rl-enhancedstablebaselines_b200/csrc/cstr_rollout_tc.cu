@@ -177,12 +177,14 @@ __host__ __device__ inline uint32_t umma_idesc_bf16(int M, int N) {
 // barrier slots inside the first 256 bytes of shared memory
 enum { BAR_W_FULL = 0, BAR_W_EMPTY = 3, BAR_A_FULL = 6, BAR_A_EMPTY = 8, BAR_D_FULL = 10, BAR_A1_FULL = 11, BAR_D1_FULL = 12, BAR_D1_EMPTY = 14, BAR_ORDER = 16, BAR_COUNT = 18 };
 
-template <int MODE, int KIND>
+// NORM (cstr_rollout_fused_norm, K == 1): layer 1 reads the normalised observation, done rows keep their raw terminal observation until
+// the statistics that include this step exist, and the CTA's moment sums go to norm_merge.
+template <int MODE, int KIND, bool NORM>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor, const uint8_t *__restrict__ packed_w2, TcGeometry g,
                   float sigma, const float2 *__restrict__ noise, uint32_t t_base, float4 *__restrict__ state,
                   int32_t *__restrict__ step_count, int32_t *__restrict__ episode, double *static_base, int64_t rows, int64_t pos0,
-                  float4 *__restrict__ records, double *reward_sum, cstr_episode_stats stats, int has_stats) {
+                  float4 *__restrict__ records, double *reward_sum, cstr_episode_stats stats, int has_stats, NormLaunch nl) {
     extern __shared__ __align__(128) uint8_t smem[];
     const uint32_t smem_base = smem_u32(smem);
     const uint32_t bars = smem_base;  // BAR_COUNT x 8 bytes
@@ -239,6 +241,11 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
     const uint32_t tmem_base = *tmem_slot;
 
     const int kgroups = g.KC / 8;  // 16-byte K groups per chunk
+    double nacc[NORM_SUMS];
+    if constexpr (NORM) {
+#pragma unroll
+        for (int j = 0; j < NORM_SUMS; ++j) nacc[j] = 0.0;
+    }
 
     if (warp < TC_ENV_WARPS) {
         // =========================== env warps ===========================================================
@@ -260,6 +267,9 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
         }
         uint32_t gchunk = 0;
         const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
+        if constexpr (NORM) {
+            if (live && half == 0) norm_fix_pending(nl, i, n, records);
+        }
 
 #ifdef CSTR_TC_TIMING
         long long T0 = 0, T1 = 0, T2 = 0, T3 = 0, T4 = 0;
@@ -272,7 +282,11 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
             // ---- (a) layer 1 on the tensor core: publish this step's split-bf16 observation row (A1) ... -------------
             const uint32_t gstep = t_base + (uint32_t)k;
             {
-                const float sf[4] = {s.x, s.y, s.z, s.w};
+                float4 sa = s;
+                if constexpr (NORM) {
+                    if (nl.norm_obs) sa = norm_obs4(s, nl);
+                }
+                const float sf[4] = {sa.x, sa.y, sa.z, sa.w};
                 __nv_bfloat16 hi[4], lo[4];
 #pragma unroll
                 for (int q = 0; q < 4; ++q) { hi[q] = __float2bfloat16_rn(sf[q]); lo[q] = __float2bfloat16_rn(sf[q] - __bfloat162float(hi[q])); }
@@ -379,7 +393,14 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
                                                             : step_fast_f32(s, env_a, sc, (float)p.target_c2, p.max_steps);
             if (live && half == 0) {
                 const int64_t row = (pos0 + k) % rows;
-                store_record(records + ((size_t)row * n + i) * 4, obs, s, buf_a, r.reward, r.truncated);
+                float4 next_obs = s;
+                if constexpr (NORM) {
+                    if (r.truncated && nl.norm_obs) {
+                        if (nl.training) nl.pending[i] = 1;  // the round trip needs S_{k+1}: the next launch (or the fix-up kernel) writes it
+                        else next_obs = norm_round_trip4(s, nl);  // frozen statistics: S_{k+1} == S_k
+                    }
+                }
+                store_record(records + ((size_t)row * n + i) * 4, obs, next_obs, buf_a, r.reward, r.truncated);
                 acc_r += (double)r.reward;
                 episode_account(stats, has_stats != 0, ep_ret, r.reward, r.truncated, sc);
             }
@@ -394,6 +415,9 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
                 s = reset_f32_call(p.seed, env, (uint32_t)ep, p.init_mode, static_base ? sb : nullptr);
                 ep += 1;
                 sc = 0;
+            }
+            if constexpr (NORM) {
+                if (live && half == 0) norm_account(nl, i, s, r.reward, r.truncated, nacc);
             }
         }
         if (live && half == 0) {
@@ -512,6 +536,9 @@ rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor,
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)g.tmem_cols) : "memory");
     }
+    if constexpr (NORM) {  // the odd-step half of the layer-3 partials is never written when K == 1: it holds the sums
+        if (nl.training) norm_merge<TC_THREADS>(nl, n, nacc, reinterpret_cast<double *>(spart + TC_PER * TC_M));
+    }
 }
 
 // W2 (H2,H1) fp32 -> bf16 UMMA image: [kc][kg][n (NP, zero padded)][8 x bf16], one contiguous chunk per kc
@@ -535,7 +562,7 @@ using namespace cstr;
 int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int math_mode, const cstr_actor_f32 *actor,
                            const void *packed_bf16, float sigma, const float *noise, int warmup, uint32_t t_base, float *state,
                            int32_t *step_count, int32_t *episode, double *static_base, int64_t rows, int64_t pos0, float *records,
-                           double *reward_sum, const cstr_episode_stats *stats, void *stream) {
+                           double *reward_sum, const cstr_episode_stats *stats, const NormLaunch *nl, void *stream) {
     (void)warmup;
     TcGeometry g;
     if (!make_geometry(actor->H1, actor->H2, g)) return fail_arg(CSTR_EINVAL, "rollout(tc): H1 must be a multiple of 16 (<=1024), H2 rounded up to 16 plus two layer-1 K-chunks must fit 512 TMEM columns (H2 <= 480), and the operands must fit in shared memory");
@@ -547,19 +574,33 @@ int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int m
     int rc = 0;
 #define CSTR_LAUNCH_TC(MODE, KIND)                                                                                                          \
     do {                                                                                                                                    \
-        rc = check_cuda(cudaFuncSetAttribute(rollout_tc_kernel<MODE, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_bytes), "smem attr"); \
+        rc = check_cuda(cudaFuncSetAttribute(rollout_tc_kernel<MODE, KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_bytes), "smem attr"); \
         if (!rc)                                                                                                                            \
-            rollout_tc_kernel<MODE, KIND><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, *actor, (const uint8_t *)packed_bf16, g, sigma, (const float2 *)noise, \
+            rollout_tc_kernel<MODE, KIND, false><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, *actor, (const uint8_t *)packed_bf16, g, sigma, (const float2 *)noise, \
                                                                                   t_base, (float4 *)state, step_count, episode, static_base, rows, pos0,   \
-                                                                                  (float4 *)records, reward_sum, st_copy, has_stats);     \
+                                                                                  (float4 *)records, reward_sum, st_copy, has_stats, NormLaunch{}); \
     } while (0)
     cstr_episode_stats st_copy = {};
     const int has_stats = stats != nullptr;
     if (stats) st_copy = *stats;
+#define CSTR_LAUNCH_TC_NORM(MODE, KIND)                                                                                                     \
+    do {                                                                                                                                    \
+        rc = check_cuda(cudaFuncSetAttribute(rollout_tc_kernel<MODE, KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_bytes), "smem attr"); \
+        if (!rc)                                                                                                                            \
+            rollout_tc_kernel<MODE, KIND, true><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, *actor, (const uint8_t *)packed_bf16, g, sigma,         \
+                                                                                       (const float2 *)noise, t_base, (float4 *)state, step_count,   \
+                                                                                       episode, static_base, rows, pos0, (float4 *)records,          \
+                                                                                       reward_sum, st_copy, has_stats, *nl);                         \
+    } while (0)
     const bool gauss = actor->kind == CSTR_ACTOR_GAUSSIAN;
-    if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_TC(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_TC(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
+    if (nl) {
+        if (K != 1) return fail_arg(CSTR_EINVAL, "rollout(tc): the VecNormalize variant runs one step per launch");
+        if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_TC_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_TC_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
+        else { if (gauss) CSTR_LAUNCH_TC_NORM(CSTR_MATH_FAST, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_TC_NORM(CSTR_MATH_FAST, CSTR_ACTOR_TANH); }
+    } else if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_TC(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_TC(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
     else { if (gauss) CSTR_LAUNCH_TC(CSTR_MATH_FAST, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_TC(CSTR_MATH_FAST, CSTR_ACTOR_TANH); }
 #undef CSTR_LAUNCH_TC
+#undef CSTR_LAUNCH_TC_NORM
     if (rc) return rc;
     return check_launch("rollout_tc_kernel");
 }

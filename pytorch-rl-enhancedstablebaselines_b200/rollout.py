@@ -14,6 +14,7 @@ from typing import Optional
 from . import _lib
 from .buffer import GpuReplayBuffer
 from .env import _MATH, GpuCSTRVecEnv
+from .normalize import GpuVecNormalize
 
 # rollout_f32_kernel keeps h1 of its 128 reactors in shared memory: 128 * max(H1, 64) floats + 128 float4 <= 227 KB
 FP32_MAX_H1 = 448
@@ -210,10 +211,13 @@ class FusedRollout:
     :param actor_mode: ``"fp32"`` (CUDA-core parity path) or ``"tc"`` (bf16 tcgen05 hidden layer).
     :param sigma: std of the Gaussian exploration noise (``NormalActionNoise``, noise.py:29-48); ignored for
         ``kind="gaussian"`` actors, whose only randomness is their own eps ~ N(0,1).
+    :param vec_normalize: a :class:`GpuVecNormalize` wrapping ``env``: the actor then reads normalised observations and every step advances
+        the wrapper's statistics and returns on the device (``cstr_rollout_fused_norm``, one kernel launch per step); the buffer keeps the
+        original observations, as the reference's ``_store_transition`` does.
     """
 
     def __init__(self, env: GpuCSTRVecEnv, buffer: GpuReplayBuffer, actor: Optional[ActorWeights] = None, sigma: float = 0.1,
-                 actor_mode: str = "fp32"):
+                 actor_mode: str = "fp32", vec_normalize: Optional[GpuVecNormalize] = None):
         if env.dtype != "fp32":
             raise ValueError("the fused rollout is fp32 (the actor and the replay records are float32)")
         if env.reset_rng != "philox":
@@ -234,6 +238,16 @@ class FusedRollout:
         self.t = 0  # global step counter: the Philox counter of the noise / warm-up action streams
         self._lib = _lib.load()
         self.launches = 0
+        self.vec_normalize = vec_normalize
+        if vec_normalize is not None:
+            if vec_normalize.venv is not env:
+                raise ValueError("vec_normalize must wrap env")
+            if isinstance(actor, AgentActorWeights):
+                raise ValueError("the two-agent rollout has no VecNormalize variant")
+            nbytes = self._lib.cstr_rollout_norm_workspace_bytes(env.num_envs, int(actor_mode == "tc"))
+            if nbytes < 0:
+                _lib.check(int(nbytes), "cstr_rollout_norm_workspace_bytes")
+            self._norm_workspace = env._torch.zeros(nbytes, dtype=env._torch.uint8, device=env.device)  # zeroed once; calls leave it zeroed
         if actor_mode == "tc" and actor is not None and actor.packed_bf16 is None:
             actor.pack_bf16()
 
@@ -269,6 +283,9 @@ class FusedRollout:
         packed = None
         if self.actor_mode == "tc" and not warmup:
             packed = self.actor.packed_bf16 if self.actor.packed_bf16 is not None else self.actor.pack_bf16()
+        if self.vec_normalize is not None:
+            self._collect_norm(K, warmup, noise, reward_sum, stats, packed)
+            return
         with torch.cuda.device(env.device):
             rc = self._lib.cstr_rollout_fused(
                 byref(env._params), env.num_envs, K, _MATH[env.math], int(self.actor_mode == "tc"),
@@ -278,6 +295,22 @@ class FusedRollout:
                 env._stream())
         _lib.check(rc, "cstr_rollout_fused")
         self.launches += 1
+        self.t += K
+        buf.advance(K)
+
+    def _collect_norm(self, K, warmup, noise, reward_sum, stats, packed) -> None:
+        env, buf, vn = self.env, self.buffer, self.vec_normalize
+        norm = _lib.RolloutNorm(stats=vn.stats.data_ptr(), returns=vn.returns_device.data_ptr(), workspace=self._norm_workspace.data_ptr(),
+                                gamma=vn.gamma, epsilon=vn.epsilon, clip_obs=vn.clip_obs, training=int(vn.training), norm_obs=int(vn.norm_obs))
+        with env._torch.cuda.device(env.device):
+            rc = self._lib.cstr_rollout_fused_norm(
+                byref(env._params), env.num_envs, K, _MATH[env.math], int(self.actor_mode == "tc"),
+                byref(self.actor._struct) if self.actor is not None else None, _lib.ptr(packed), self.sigma, _lib.ptr(noise), int(warmup),
+                self.t & 0xFFFFFFFF, _lib.ptr(env.state), _lib.ptr(env.step_count), _lib.ptr(env.episode), env._sb_ptr(),
+                buf.buffer_size, buf.pos, _lib.ptr(buf.records), _lib.ptr(reward_sum), byref(stats._struct) if stats is not None else None,
+                byref(norm), env._stream())
+        _lib.check(rc, "cstr_rollout_fused_norm")
+        self.launches += K + int(K > 0 and vn.training and vn.norm_obs)  # one launch per step, then the done rows' fix-up
         self.t += K
         buf.advance(K)
 
@@ -345,7 +378,18 @@ def _actor_unsupported(actor, actor_mode: str) -> Optional[str]:
 
 def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_noise, actor_mode: str = "fp32") -> Optional[str]:
     """Why ``cstr_rollout_fused`` can NOT stand in for this ``collect_rollouts`` call — or None when it can.  ``actor_mode`` is the
-    kernel that would run the actor (``"fp32"`` or ``"tc"``; the two-agent actors always run on ``"fp32"``)."""
+    kernel that would run the actor (``"fp32"`` or ``"tc"``; the two-agent actors always run on ``"fp32"``).  ``env`` may be a
+    :class:`GpuVecNormalize` around the env when it is the model's own ``_vec_normalize_env``."""
+    vec_normalize = getattr(model, "_vec_normalize_env", None)
+    if isinstance(env, GpuVecNormalize):
+        if vec_normalize is not env:
+            return "the GpuVecNormalize the rollout steps through is not the model's _vec_normalize_env"
+        actor = getattr(model, "actor", None)
+        if actor is not None and hasattr(actor, "mu_list"):
+            return "two agents under VecNormalize (the reference's multi-agent store path is not covered by the fused rollout)"
+        env = env.venv
+    elif vec_normalize is not None:
+        return "VecNormalize wraps the env (the reference's host VecNormalize steps through the NumPy protocol; use GpuVecNormalize)"
     if not isinstance(env, GpuCSTRVecEnv):
         return f"env is a {type(env).__name__}, not a GpuCSTRVecEnv (wrappers step through the NumPy protocol)"
     if env.dtype != "fp32" or env.reset_rng != "philox":
@@ -356,8 +400,6 @@ def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_nois
         return "train_freq counts episodes (one kernel launch collects a fixed number of steps)"
     if getattr(model, "use_sde", False):
         return "use_sde (state-dependent exploration matrices)"
-    if getattr(model, "_vec_normalize_env", None) is not None:
-        return "VecNormalize wraps the env (the actor would need normalised observations)"
     actor = getattr(model, "actor", None)
     if actor is not None and hasattr(actor, "mu_list"):  # multi-agent (MADDPG / IDDPG): any noise object is ignored by the reference itself (Q5)
         splits = ([list(s) for s in getattr(model, "observation_splits", [])], [list(s) for s in getattr(model, "action_splits", [])])
@@ -383,6 +425,10 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
       ``ep_len_mean``), ``_episode_num`` advances by their number, ``_dump_logs`` runs when it crosses a multiple of ``log_interval``;
     * callbacks: ``on_rollout_start`` / ``on_step`` / ``on_rollout_end`` once per launch (``on_step`` sees ``num_timesteps`` advanced by
       the whole launch); a False from ``on_step`` stops training as in the reference.
+
+    Under a :class:`GpuVecNormalize` (``bind_vec_normalize_class``) the launches are ``cstr_rollout_fused_norm``: normalised actor input,
+    the wrapper's statistics and returns advanced every step, original observations stored; when ``learn()`` returns, ``_last_obs``
+    (normalised), ``_last_original_obs`` and the wrapper's ``old_obs`` / ``old_reward`` hold what the reference loop leaves there.
 
     Nothing per-env runs in Python and nothing leaves the device except the finished-episode list.  Models the kernel does not cover
     (see :func:`fused_rollout_unsupported`) keep the reference's own ``collect_rollouts`` with a one-time warning.
@@ -411,7 +457,8 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
         # kernel draws the noise itself
         def _setup_learn(self, *args, **kwargs):
             noise = self.action_noise
-            if noise is not None and isinstance(self.env, GpuCSTRVecEnv) and _noise_sigma(noise) is not None and self.env.num_envs > 1:
+            if (noise is not None and isinstance(self.env, (GpuCSTRVecEnv, GpuVecNormalize)) and _noise_sigma(noise) is not None
+                    and self.env.num_envs > 1):
                 self.action_noise = None
             try:
                 return super()._setup_learn(*args, **kwargs)
@@ -429,11 +476,14 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
         def _fused_rollout_engine(self, env, replay_buffer, sigma: float) -> FusedRollout:
             kind, modules = self._fused_actor_modules()
             roll = self._fused_roll
-            if roll is None or roll.env is not env or roll.buffer is not replay_buffer:
+            vec_normalize = env if isinstance(env, GpuVecNormalize) else None
+            env = env.venv if vec_normalize is not None else env
+            if roll is None or roll.env is not env or roll.buffer is not replay_buffer or roll.vec_normalize is not vec_normalize:
                 actor = (AgentActorWeights(modules[0], device=env.device) if kind == "agents"
                          else ActorWeights.from_sac_actor(*modules, device=env.device) if kind == "gaussian"
                          else ActorWeights.from_module(modules[0], device=env.device))
-                roll = FusedRollout(env, replay_buffer, actor, sigma=sigma, actor_mode="fp32" if kind == "agents" else actor_mode)
+                roll = FusedRollout(env, replay_buffer, actor, sigma=sigma, actor_mode="fp32" if kind == "agents" else actor_mode,
+                                    vec_normalize=vec_normalize)
                 roll.t = int(self.num_timesteps // max(env.num_envs, 1))
                 self._fused_roll, self._fused_stats = roll, EpisodeStats(env.num_envs, device=env.device)
             roll.sigma = sigma
@@ -487,8 +537,16 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
         def learn(self, *args, **kwargs):
             self._fused_t0 = time.time()
             out = super().learn(*args, **kwargs)
-            if self._fused_roll is not None:  # `_last_obs` is the host copy the reference's own paths (predict, save) expect
-                self._last_obs = self._fused_roll.env.state.cpu().numpy()
+            roll = self._fused_roll
+            if roll is not None:  # `_last_obs` is the host copy the reference's own paths (predict, save) expect
+                raw = roll.env.state.cpu().numpy()
+                vn = roll.vec_normalize
+                if vn is None:
+                    self._last_obs = raw
+                else:  # what the reference's last step_wait + collect_rollouts leave (vec_normalize.py:183-186, off_policy_algorithm.py:497-503)
+                    buf = roll.buffer
+                    vn.old_obs, vn.old_reward = raw, buf.records[(buf.pos - 1) % buf.buffer_size, :, 10].cpu().numpy()
+                    self._last_original_obs, self._last_obs = raw, vn.normalize_obs(raw)
             return out
 
         def _excluded_save_params(self):
