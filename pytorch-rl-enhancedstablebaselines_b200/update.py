@@ -12,6 +12,9 @@ operands with fp32 accumulation (reduced precision, throughput mode; no per-step
 ``adopt_policy`` re-points the parameters of the reference's ``TD3Policy`` modules at views of the flat blocks, so
 ``policy.predict``, ``model.save`` and the fused rollout keep seeing the live weights without copies.
 ``bind_td3_class(TD3)`` returns a subclass of the reference algorithm whose ``train()`` runs here.
+
+Every engine (:class:`FusedTD3Update`, :class:`FusedSACUpdate` and the BCQ / multi-agent engines of ``update_ext``) is built on
+:class:`_FusedEngine`, which owns that flat-block plumbing.
 """
 from __future__ import annotations
 
@@ -28,73 +31,74 @@ _GEMM_MODES = {"fp32": 0, "tensor": 1, "bf16": 2}
 _TENSORS = ("W1", "b1", "W2", "b2", "W3", "b3")
 
 
-class FusedTD3Update:
-    def __init__(self, net_arch: Sequence[int] = (400, 300), batch_size: int = 256, device: Any = "cuda", gamma: float = 0.99, tau: float = 0.005,
-                 learning_rate: float = 1e-3, policy_delay: int = 2, target_policy_noise: float = 0.2, target_noise_clip: float = 0.5,
-                 betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", n_critics: int = 2, dp_rank: int = 0):
+class _FusedEngine:
+    """What every fused update engine shares: five flat float32 device blocks (``params, targets, grads, adam_m, adam_v``) in the layout
+    the library reports, the workspace, the hand-over of torch modules and Adam state, CUDA-graph replay and the peer-memory gradient
+    all-reduce.  An engine names its three-layer nets (``NETS``, ``_dims``) and the nets with a target block of their own
+    (``TARGET_NETS``); its constructor calls this one, sets its own fields, then hands the library's layout to ``_allocate``."""
+
+    NETS: Sequence[str] = ()
+    TARGET_NETS: Optional[Sequence[str]] = None  # None: every net of NETS
+    N_LOSS = 4
+
+    def __init__(self, device, gamma: float, tau: float, learning_rate: float, policy_delay: int, betas, eps: float, seed: int, gemm: str,
+                 dp_rank: int):
         torch = _lib.require_cuda()
-        self._torch = torch
-        self._libc = _lib.load()
-        if len(net_arch) != 2:
-            raise ValueError("FusedTD3Update supports the two-hidden-layer MLPs of TD3's MlpPolicy (net_arch=[h1, h2])")
-        self.h1, self.h2 = int(net_arch[0]), int(net_arch[1])
-        if self.h1 % 4 or self.h2 % 4:
-            raise ValueError("hidden sizes must be multiples of 4")
+        self._torch, self._libc = torch, _lib.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
-            raise _lib.CstrLibraryError("FusedTD3Update needs a CUDA device (no CPU fallback)")
+            raise _lib.CstrLibraryError(f"{type(self).__name__} needs a CUDA device (no CPU fallback)")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
-        self.gamma, self.tau, self.learning_rate = float(gamma), float(tau), float(learning_rate)
-        self.policy_delay, self.target_policy_noise, self.target_noise_clip = int(policy_delay), float(target_policy_noise), float(target_noise_clip)
-        self.betas, self.eps, self.seed = (float(betas[0]), float(betas[1])), float(eps), int(seed)
-        # data-parallel training: every rank holds the same `seed`, and the in-kernel noise is keyed by (seed, batch row, update), so
-        # without the rank in the key row b of every shard would draw the same smoothing noise / eps (perfectly correlated global batch)
-        self.dp_rank = int(dp_rank)
         if gemm not in _GEMM_MODES:
             raise ValueError("gemm must be 'fp32' (FFMA tiles, the reference's arithmetic), 'tensor' (tcgen05 bf16x3 split, fp32-grade) or "
                              "'bf16' (tcgen05, plain bf16 operands: reduced precision)")
-        self.gemm = gemm
-        if n_critics not in (1, 2):
-            raise ValueError("n_critics must be 2 (TD3) or 1 (DDPG)")
-        self.n_critics = int(n_critics)
-        offs = (c_int64 * 19)()
-        _lib.check(self._libc.cstr_td3_layout(self.h1, self.h2, offs), "cstr_td3_layout")
-        self.param_count = int(offs[18])
-        self._offsets = {(NET_NAMES[n], _TENSORS[k]): int(offs[n * 6 + k]) for n in range(3) for k in range(6)}
-        self.actor_range = (0, self._offsets[("critic0", "W1")])
-        self.critic_range = (self._offsets[("critic0", "W1")], self.param_count)
-        with torch.cuda.device(self.device):
-            z = lambda: torch.zeros(self.param_count, dtype=torch.float32, device=self.device)  # noqa: E731
-            self.params, self.targets, self.grads, self.adam_m, self.adam_v = z(), z(), z(), z(), z()
-            self.loss_sums = torch.zeros(4, dtype=torch.float32, device=self.device)
-            self._counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # graph mode: n_updates, critic_step, actor_step, sample_draw
-        self._graph = None
-        self._graph_key = None
-        self._graph_out = None
+        self.gamma, self.tau, self.learning_rate = float(gamma), float(tau), float(learning_rate)
+        self.policy_delay = int(policy_delay)  # updates per actor step, and per captured graph cycle
+        self.betas, self.eps, self.seed, self.gemm = (float(betas[0]), float(betas[1])), float(eps), int(seed), gemm
+        # data-parallel training: every rank holds the same `seed`, and the in-kernel noise is keyed by (seed, batch row, update), so
+        # without the rank in the key row b of every shard would draw the same smoothing noise / eps (perfectly correlated global batch)
+        self.dp_rank = int(dp_rank)
+        self._graph = self._graph_key = self._graph_out = None
         self._peer = None  # cstr_peer_comm of enable_peer_allreduce()
         self._workspace = None
         self._batch = 0
+        self._moments: Dict[int, Any] = {}  # id(adopted parameter) -> (adam_m view, adam_v view)
+        self.n_updates = self.critic_step = self.actor_step = self.launches = 0
+
+    def _two_hidden(self, arch: Sequence[int]) -> None:
+        if len(arch) != 2:
+            raise ValueError(f"{type(self).__name__} supports two-hidden-layer MLPs ([h1, h2]), got {list(arch)}")
+        self.h1, self.h2 = int(arch[0]), int(arch[1])
+        if self.h1 % 4 or self.h2 % 4:
+            raise ValueError("hidden sizes must be multiples of 4")
+
+    def _allocate(self, offs, batch_size: int) -> None:
+        """Take the layout the library wrote into ``offs`` (six offsets per net of ``NETS``, the parameter count last) and allocate the
+        five blocks, the losses, the graph-mode counters and the workspace."""
+        torch = self._torch
+        self.param_count = int(offs[len(offs) - 1])
+        self._offsets = {(net, t): int(offs[n * 6 + k]) for n, net in enumerate(self.NETS) for k, t in enumerate(_TENSORS)}
+        with torch.cuda.device(self.device):
+            z = lambda: torch.zeros(self.param_count, dtype=torch.float32, device=self.device)  # noqa: E731
+            self.params, self.targets, self.grads, self.adam_m, self.adam_v = z(), z(), z(), z(), z()
+            self.loss_sums = torch.zeros(self.N_LOSS, dtype=torch.float32, device=self.device)
+            self._counters = torch.zeros(4, dtype=torch.int64, device=self.device)  # graph mode: n_updates, critic_step, actor_step, sample_draw
         self._set_batch(int(batch_size))
-        self.n_updates = 0
-        self.critic_step = 0
-        self.actor_step = 0
-        self.launches = 0
 
     # ---- layout ---------------------------------------------------------------------------------------------------
     def _shape(self, net: str, tensor: str):
-        i, o = (4, 2) if net == "actor" else (6, 1)
-        return {"W1": (self.h1, i), "b1": (self.h1,), "W2": (self.h2, self.h1), "b2": (self.h2,), "W3": (o, self.h2), "b3": (o,)}[tensor]
+        i, h1, h2, o = self._dims(net)
+        return {"W1": (h1, i), "b1": (h1,), "W2": (h2, h1), "b2": (h2,), "W3": (o, h2), "b3": (o,)}[tensor]
 
     def views(self, block: str = "params") -> Dict[str, List[Any]]:
         """``{net: [W1, b1, W2, b2, W3, b3]}`` as views of one flat block (``params|targets|grads|adam_m|adam_v``)."""
         flat = getattr(self, block)
         out = {}
-        for net in NET_NAMES:
+        for net in self.NETS:
             out[net] = []
             for t in _TENSORS:
-                shape = self._shape(net, t)
-                off = self._offsets[(net, t)]
+                shape, off = self._shape(net, t), self._offsets[(net, t)]
                 out[net].append(flat[off:off + int(np.prod(shape))].view(shape))
         return out
 
@@ -109,90 +113,72 @@ class FusedTD3Update:
             self._workspace = self._torch.empty(need // 4, dtype=self._torch.float32, device=self.device)
         self._batch = batch
 
-    def _workspace_bytes(self, batch: int) -> int:
-        return int(self._libc.cstr_td3_workspace_bytes(byref(self._config(batch))))
-
     def _keyed_seed(self) -> int:
         return (self.seed + 0x9E3779B97F4A7C15 * self.dp_rank) & (2**64 - 1)
 
-    def _config(self, batch: int) -> "_lib.Td3Config":
-        return _lib.Td3Config(h1=self.h1, h2=self.h2, batch=batch, policy_delay=self.policy_delay, gamma=self.gamma, tau=self.tau, lr=self.learning_rate,
-                              beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, target_policy_noise=self.target_policy_noise,
-                              target_noise_clip=self.target_noise_clip, seed=self._keyed_seed(), gemm_mode=_GEMM_MODES[self.gemm],
-                              n_critics=getattr(self, "n_critics", 2))
-
     # ---- weights in / out -------------------------------------------------------------------------------------------
+    def _trained_nets(self) -> Sequence[str]:
+        return self.NETS
+
+    def _target_nets(self) -> Sequence[str]:
+        return self.NETS if self.TARGET_NETS is None else self.TARGET_NETS
+
     def load_nets(self, nets: Dict[str, Sequence[Any]]) -> None:
-        """``nets`` maps ``actor, critic0, critic1`` (and optionally ``*_target``) to six arrays/tensors in nn.Linear layout."""
+        """``nets`` maps every net the engine trains to six arrays/tensors in nn.Linear layout (a head of several modules stacked), and
+        optionally ``<net>_target`` for the nets with a target block (default: a copy of the net)."""
         torch = self._torch
-        for block, suffix in (("params", ""), ("targets", "_target")):
-            v = self.views(block)
-            for net in NET_NAMES[:1 + self.n_critics]:
-                src = nets.get(net + suffix, nets[net] if suffix else None)
-                for dst, s in zip(v[net], src):
-                    dst.copy_(torch.as_tensor(np.asarray(s) if not isinstance(s, torch.Tensor) else s).to(self.device, torch.float32).reshape(dst.shape))
+        v, t = self.views("params"), self.views("targets")
+        for net in self._trained_nets():
+            pairs = list(zip(v[net], nets[net]))
+            if net in self._target_nets():
+                pairs += zip(t[net], nets.get(net + "_target", nets[net]))
+            for dst, s in pairs:
+                dst.copy_(torch.as_tensor(np.asarray(s) if not isinstance(s, torch.Tensor) else s).to(self.device, torch.float32).reshape(dst.shape))
 
     def nets(self) -> Dict[str, List[np.ndarray]]:
-        out = {}
-        for block, suffix in (("params", ""), ("targets", "_target")):
-            for net, ts in self.views(block).items():
-                out[net + suffix] = [t.cpu().numpy() for t in ts]
+        out = {net: [x.cpu().numpy() for x in ts] for net, ts in self.views("params").items()}
+        targets = self._target_nets()
+        out.update({net + "_target": [x.cpu().numpy() for x in ts] for net, ts in self.views("targets").items() if net in targets})
         return out
 
-    def adopt_modules(self, actor, critics: Sequence[Any], actor_target, critic_targets: Sequence[Any]) -> None:
-        """Copy the weights of ``nn.Sequential(Linear, ReLU, Linear, ReLU, Linear[, Tanh])`` modules in and re-point their
-        parameters at the flat blocks (zero-copy sharing from then on)."""
-        if len(critics) != self.n_critics or len(critic_targets) != self.n_critics:
-            raise ValueError(f"expected {self.n_critics} critic network(s)")
-        pairs = [("params", "actor", actor), ("targets", "actor", actor_target)]
-        for z in range(self.n_critics):
-            pairs += [("params", f"critic{z}", critics[z]), ("targets", f"critic{z}", critic_targets[z])]
-        for block, net, module in pairs:
-            ps = list(module.parameters())
-            if len(ps) != 6:
-                raise ValueError("expected a 3-layer MLP (6 parameter tensors)")
-            for view, p in zip(self.views(block)[net], ps):
-                if tuple(p.shape) != tuple(view.shape):
-                    raise ValueError(f"shape mismatch for {net}: module {tuple(p.shape)} vs layout {tuple(view.shape)}")
-                view.copy_(p.data.to(self.device, self._torch.float32))
-                p.data = view
+    def _adopt(self, online, targets) -> None:
+        """Copy each module parameter of the ``(view, parameter)`` pairs into its view and re-point ``p.data`` at it (zero-copy sharing
+        from then on).  ``online`` views lie in ``params``: their parameters' Adam moments are the same slices of ``adam_m`` / ``adam_v``."""
+        online = list(online)
+        for view, p in online + list(targets):
+            if tuple(p.shape) != tuple(view.shape):
+                raise ValueError(f"shape mismatch: module {tuple(p.shape)} vs layout {tuple(view.shape)}")
+            view.copy_(p.data.to(self.device, self._torch.float32))
+            p.data = view
+        self._moments = {}
+        for view, p in online:
+            off, n = (view.data_ptr() - self.params.data_ptr()) // 4, view.numel()
+            self._moments[id(p)] = (self.adam_m[off:off + n].view(view.shape), self.adam_v[off:off + n].view(view.shape))
 
-    def adopt_policy(self, policy) -> None:
-        """The reference's ``TD3Policy`` (core/td3/policies.py:172-210): ``actor.mu``, ``critic.q_networks`` and the targets."""
-        if len(policy.critic.q_networks) != self.n_critics:
-            raise ValueError(f"this engine was built for n_critics={self.n_critics}, the policy has {len(policy.critic.q_networks)}")
-        self.adopt_modules(policy.actor.mu, list(policy.critic.q_networks), policy.actor_target.mu, list(policy.critic_target.q_networks))
-        self._opt_params = {"actor": list(policy.actor.mu.parameters()), "critic": [p for q in policy.critic.q_networks for p in q.parameters()]}
+    def _import_adam(self, opt) -> int:
+        """Copy ``exp_avg`` / ``exp_avg_sq`` of every adopted parameter of the ``torch.optim.Adam`` ``opt`` into the moments and take its
+        ``betas`` / ``eps``; returns the largest step count found (0 for an optimiser that has not stepped)."""
+        group = opt.param_groups[0]
+        self.betas, self.eps = (float(group["betas"][0]), float(group["betas"][1])), float(group["eps"])
+        step = 0
+        for p in group["params"]:
+            st = opt.state.get(p)
+            if st and id(p) in self._moments:
+                m, v = self._moments[id(p)]
+                m.copy_(st["exp_avg"])
+                v.copy_(st["exp_avg_sq"])
+                step = max(step, int(float(st["step"])))
+        return step
 
-    def import_optimizer_state(self, actor_optimizer, critic_optimizer) -> None:
-        """Take over Adam moments / step counts of ``torch.optim.Adam`` optimisers created over the adopted modules."""
-        for tag, opt, nets in (("actor", actor_optimizer, ("actor",)), ("critic", critic_optimizer, ("critic0", "critic1")[:self.n_critics])):
-            group = opt.param_groups[0]
-            self.betas, self.eps = (float(group["betas"][0]), float(group["betas"][1])), float(group["eps"])
-            m = [t for n in nets for t in self.views("adam_m")[n]]
-            v = [t for n in nets for t in self.views("adam_v")[n]]
-            step = 0
-            for p, mv, vv in zip(group["params"], m, v):
-                st = opt.state.get(p)
-                if st:
-                    mv.copy_(st["exp_avg"])
-                    vv.copy_(st["exp_avg_sq"])
-                    step = int(float(st["step"]))
-            if tag == "actor":
-                self.actor_step = step
-            else:
-                self.critic_step = step
-
-    def export_optimizer_state(self, actor_optimizer, critic_optimizer) -> None:
-        """Write moments / step counts back so ``model.save`` and a later torch ``optimizer.step()`` continue from here."""
-        torch = self._torch
-        for opt, nets, step in ((actor_optimizer, ("actor",), self.actor_step), (critic_optimizer, ("critic0", "critic1")[:self.n_critics], self.critic_step)):
-            if step == 0:
-                continue
-            m = [t for n in nets for t in self.views("adam_m")[n]]
-            v = [t for n in nets for t in self.views("adam_v")[n]]
-            for p, mv, vv in zip(opt.param_groups[0]["params"], m, v):
-                opt.state[p] = {"step": torch.tensor(float(step)), "exp_avg": mv, "exp_avg_sq": vv}
+    def _export_adam(self, opt, step: int) -> None:
+        """Make the engine's moment views the Adam state of every adopted parameter of ``opt``, at ``step`` (skipped when it is 0), so that
+        ``model.save`` and a later torch ``optimizer.step()`` continue from here."""
+        if step == 0:
+            return
+        for p in opt.param_groups[0]["params"]:
+            if id(p) in self._moments:
+                m, v = self._moments[id(p)]
+                opt.state[p] = {"step": self._torch.tensor(float(step)), "exp_avg": m, "exp_avg_sq": v}
 
     # ---- the gradient step ----------------------------------------------------------------------------------------------
     def _stream(self) -> int:
@@ -207,11 +193,31 @@ class FusedTD3Update:
             raise ValueError(f"batch tensor has {t.numel()} elements, expected {self._batch}x{cols}")
         return t
 
+    def _batch_f32(self, batch):
+        """(obs, actions, next_obs, dones, rewards) of a ``ReplayBufferSamples`` or 5-tuple as contiguous float32 device tensors; sets
+        the batch size."""
+        obs, act, nobs, dones, rew = batch
+        self._set_batch(int(obs.shape[0]))
+        return self._f32(obs, 4), self._f32(act, 2), self._f32(nobs, 4), self._f32(dones, 1), self._f32(rew, 1)
+
     def _state(self, counters: bool) -> "_lib.Td3State":
         return _lib.Td3State(params=self.params.data_ptr(), targets=self.targets.data_ptr(), grads=self.grads.data_ptr(), adam_m=self.adam_m.data_ptr(),
                              adam_v=self.adam_v.data_ptr(), workspace=self._workspace.data_ptr(), workspace_bytes=self._workspace.numel() * 4,
                              losses=self.loss_sums.data_ptr(), counters=self._counters.data_ptr() if counters else None,
                              peer=ctypes.addressof(self._peer) if self._peer is not None else None)
+
+    def _phases(self, run: Callable[[int], None], allreduce, actor_due: bool) -> None:
+        """``run(TD3_ALL)``; or, with a host-side ``allreduce`` hook, GRAD -> all-reduce of the critic gradients -> APPLY | ACTOR_GRAD ->
+        all-reduce of the actor gradients (when the actor steps) -> ACTOR_APPLY."""
+        if allreduce is None:
+            run(_lib.TD3_ALL)
+            return
+        run(_lib.TD3_CRITIC_GRAD)
+        allreduce(self.grads[self._reduced_critic[0]:self._reduced_critic[1]])
+        run(_lib.TD3_CRITIC_APPLY | _lib.TD3_ACTOR_GRAD)
+        if actor_due:
+            allreduce(self.grads[self.actor_range[0]:self.actor_range[1]])
+        run(_lib.TD3_ACTOR_APPLY)
 
     # ---- data-parallel training: the gradient all-reduce inside the Adam kernel (include/cstr_b200.h, cstr_peer_comm) ---------------
     def enable_peer_allreduce(self, group=None) -> bool:
@@ -294,7 +300,7 @@ class FusedTD3Update:
         draw = self._counters[3:4]
 
         def cycle():
-            for k in range(1, self._cycle_len() + 1):  # by-value counters only choose the launch structure: update k of the cycle
+            for k in range(1, self.policy_delay + 1):  # by-value counters only choose the launch structure: update k of the cycle
                 buffer.sample_into(out, draw, env=env)
                 self._graph_launch(batch_size, st, out, k, allreduce)
 
@@ -317,9 +323,106 @@ class FusedTD3Update:
         return (id(buffer), batch_size, buffer.size(), buffer.n_envs, id(env), self.policy_delay, self.learning_rate, self.params.data_ptr(),
                 self._workspace.data_ptr() if self._workspace is not None else 0, self.grads.data_ptr(), id(allreduce) if allreduce is not None else 0)
 
-    def _cycle_len(self) -> int:
-        return self.policy_delay
+    def _train_graph(self, graph: bool, gradient_steps: int, buffer, batch_size: int, env, allreduce=None) -> int:
+        """With ``graph`` and a capturable set-up (Philox-index buffer with a full ring, device-side normalisation, no host hook unless
+        ``_hook_capturable``), replays whole cycles while the update count is cycle-aligned.  Returns the number of gradient steps done."""
+        # a captured cycle bakes the sampling range in: only worth capturing once the ring is full (its range is constant from then on)
+        if not (graph and _hook_capturable(allreduce) and getattr(buffer, "index_mode", None) == "philox" and buffer.full and _graph_env_ok(env)):
+            return 0
+        if self.n_updates % self.policy_delay or gradient_steps < self.policy_delay:
+            return 0
+        key = self._make_graph_key(buffer, batch_size, env, allreduce)
+        if self._graph is None or key != self._graph_key:
+            self._capture(buffer, batch_size, env, allreduce)
+        cycles = gradient_steps // self.policy_delay
+        self._counters.copy_(self._torch.tensor([self.n_updates, self.critic_step, self.actor_step, buffer._draw], dtype=self._torch.int64),
+                             non_blocking=True)
+        with self._torch.cuda.device(self.device):
+            for _ in range(cycles):
+                self._graph.replay()
+        done = cycles * self.policy_delay
+        self.n_updates += done
+        self.critic_step += done
+        self.actor_step += done // self.policy_delay
+        buffer._draw += done
+        self.launches += cycles * (23 * (self.policy_delay - 1) + 44 + self.policy_delay)
+        return done
 
+    def pop_losses(self):
+        """Means since the last call of the losses the kernels sum, ``None`` for one not computed since (the actor's between policy steps):
+        TD3 (critic, actor), SAC (critic, actor, ent_coef_loss, ent_coef), BCQ (vae, critic, actor) — what the reference's train() logs."""
+        s = self.loss_sums.cpu().numpy().astype(np.float64)
+        self.loss_sums.zero_()
+        return tuple(s[2 * i] / s[2 * i + 1] if s[2 * i + 1] else None for i in range(self.N_LOSS // 2))
+
+
+class FusedTD3Update(_FusedEngine):
+    NETS = NET_NAMES
+
+    def __init__(self, net_arch: Sequence[int] = (400, 300), batch_size: int = 256, device: Any = "cuda", gamma: float = 0.99, tau: float = 0.005,
+                 learning_rate: float = 1e-3, policy_delay: int = 2, target_policy_noise: float = 0.2, target_noise_clip: float = 0.5,
+                 betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", n_critics: int = 2, dp_rank: int = 0):
+        super().__init__(device, gamma, tau, learning_rate, policy_delay, betas, eps, seed, gemm, dp_rank)
+        self._two_hidden(net_arch)
+        self.target_policy_noise, self.target_noise_clip = float(target_policy_noise), float(target_noise_clip)
+        if n_critics not in (1, 2):
+            raise ValueError("n_critics must be 2 (TD3) or 1 (DDPG)")
+        self.n_critics = int(n_critics)
+        offs = (c_int64 * 19)()
+        _lib.check(self._libc.cstr_td3_layout(self.h1, self.h2, offs), "cstr_td3_layout")
+        self._allocate(offs, batch_size)
+        self.actor_range = (0, self._offsets[("critic0", "W1")])
+        self.critic_range = (self._offsets[("critic0", "W1")], self.param_count)
+        self._reduced_critic = self.critic_range
+
+    def _dims(self, net: str):
+        return (4, self.h1, self.h2, 2) if net == "actor" else (6, self.h1, self.h2, 1)
+
+    def _trained_nets(self) -> Sequence[str]:
+        return NET_NAMES[:1 + self.n_critics]  # DDPG's layout keeps critic1's slots, unused
+
+    def _workspace_bytes(self, batch: int) -> int:
+        return int(self._libc.cstr_td3_workspace_bytes(byref(self._config(batch))))
+
+    def _config(self, batch: int) -> "_lib.Td3Config":
+        return _lib.Td3Config(h1=self.h1, h2=self.h2, batch=batch, policy_delay=self.policy_delay, gamma=self.gamma, tau=self.tau, lr=self.learning_rate,
+                              beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, target_policy_noise=self.target_policy_noise,
+                              target_noise_clip=self.target_noise_clip, seed=self._keyed_seed(), gemm_mode=_GEMM_MODES[self.gemm],
+                              n_critics=self.n_critics)
+
+    # ---- weights in / out -------------------------------------------------------------------------------------------
+    def adopt_modules(self, actor, critics: Sequence[Any], actor_target, critic_targets: Sequence[Any]) -> None:
+        """Copy the weights of ``nn.Sequential(Linear, ReLU, Linear, ReLU, Linear[, Tanh])`` modules in and re-point their
+        parameters at the flat blocks (zero-copy sharing from then on)."""
+        if len(critics) != self.n_critics or len(critic_targets) != self.n_critics:
+            raise ValueError(f"expected {self.n_critics} critic network(s)")
+        v, t = self.views("params"), self.views("targets")
+        online, targets = [], []
+        for net, module, target in [("actor", actor, actor_target)] + [(f"critic{z}", critics[z], critic_targets[z]) for z in range(self.n_critics)]:
+            ps, pts = list(module.parameters()), list(target.parameters())
+            if len(ps) != 6 or len(pts) != 6:
+                raise ValueError("expected a 3-layer MLP (6 parameter tensors)")
+            online += zip(v[net], ps)
+            targets += zip(t[net], pts)
+        self._adopt(online, targets)
+
+    def adopt_policy(self, policy) -> None:
+        """The reference's ``TD3Policy`` (core/td3/policies.py:172-210): ``actor.mu``, ``critic.q_networks`` and the targets."""
+        if len(policy.critic.q_networks) != self.n_critics:
+            raise ValueError(f"this engine was built for n_critics={self.n_critics}, the policy has {len(policy.critic.q_networks)}")
+        self.adopt_modules(policy.actor.mu, list(policy.critic.q_networks), policy.actor_target.mu, list(policy.critic_target.q_networks))
+
+    def import_optimizer_state(self, actor_optimizer, critic_optimizer) -> None:
+        """Take over Adam moments / step counts of ``torch.optim.Adam`` optimisers created over the adopted modules."""
+        self.actor_step = self._import_adam(actor_optimizer)
+        self.critic_step = self._import_adam(critic_optimizer)
+
+    def export_optimizer_state(self, actor_optimizer, critic_optimizer) -> None:
+        """Write moments / step counts back so ``model.save`` and a later torch ``optimizer.step()`` continue from here."""
+        self._export_adam(actor_optimizer, self.actor_step)
+        self._export_adam(critic_optimizer, self.critic_step)
+
+    # ---- the gradient step ----------------------------------------------------------------------------------------------
     def _graph_launch(self, batch_size: int, st, out, k: int, allreduce=None) -> None:
         cfg = self._config(batch_size)
 
@@ -328,45 +431,13 @@ class FusedTD3Update:
                                             _lib.ptr(out[4]), None, k, 1, 1, phases, self._stream())
             _lib.check(rc, "cstr_td3_update (graph capture)")
 
-        if allreduce is None:
-            run(_lib.TD3_ALL)
-        else:  # the collective is captured between the phases: GRAD -> all-reduce -> APPLY is ONE graph
-            run(_lib.TD3_CRITIC_GRAD)
-            allreduce(self.grads[self.critic_range[0]:self.critic_range[1]])
-            run(_lib.TD3_CRITIC_APPLY | _lib.TD3_ACTOR_GRAD)
-            if k % self.policy_delay == 0:
-                allreduce(self.grads[self.actor_range[0]:self.actor_range[1]])
-            run(_lib.TD3_ACTOR_APPLY)
-
-    def _train_graph(self, gradient_steps: int, buffer, batch_size: int, env, allreduce=None) -> int:
-        """Replays whole cycles while the update count is cycle-aligned; returns the number of gradient steps done."""
-        if self.n_updates % self._cycle_len() or gradient_steps < self._cycle_len():
-            return 0
-        key = self._make_graph_key(buffer, batch_size, env, allreduce)
-        if self._graph is None or key != self._graph_key:
-            self._capture(buffer, batch_size, env, allreduce)
-        cycles = gradient_steps // self._cycle_len()
-        self._counters.copy_(self._torch.tensor([self.n_updates, self.critic_step, self.actor_step, buffer._draw], dtype=self._torch.int64),
-                             non_blocking=True)
-        with self._torch.cuda.device(self.device):
-            for _ in range(cycles):
-                self._graph.replay()
-        done = cycles * self._cycle_len()
-        self.n_updates += done
-        self.critic_step += done
-        self.actor_step += done // self.policy_delay
-        buffer._draw += done
-        self.launches += cycles * (23 * (self.policy_delay - 1) + 44 + self.policy_delay)
-        return done
+        self._phases(run, allreduce, k % self.policy_delay == 0)  # a hook is captured between the phases: GRAD -> all-reduce -> APPLY is ONE graph
 
     def update(self, batch, noise=None, allreduce: Optional[Callable[[Any], None]] = None) -> None:
         """One iteration of the loop body (td3.py:162-206) on ``batch`` (``ReplayBufferSamples`` or a 5-tuple in that order).
         ``noise``: explicit N(0, target_policy_noise) draws (B,2) for parity tests; default = Philox in the kernel.
         ``allreduce``: called on the flat gradient range between backward and Adam (data-parallel training)."""
-        obs, act, nobs, dones, rew = batch
-        self._set_batch(int(obs.shape[0]))
-        obs, act, nobs = self._f32(obs, 4), self._f32(act, 2), self._f32(nobs, 4)
-        dones, rew = self._f32(dones, 1), self._f32(rew, 1)
+        obs, act, nobs, dones, rew = self._batch_f32(batch)
         nz = None if noise is None else self._f32(noise, 2)
         self.n_updates += 1
         self.critic_step += 1
@@ -382,15 +453,7 @@ class FusedTD3Update:
             _lib.check(rc, "cstr_td3_update")
 
         with self._torch.cuda.device(self.device):
-            if allreduce is None or self._peer is not None:  # a peer communicator averages inside the APPLY kernels
-                run(_lib.TD3_ALL)
-            else:
-                run(_lib.TD3_CRITIC_GRAD)
-                allreduce(self.grads[self.critic_range[0]:self.critic_range[1]])
-                run(_lib.TD3_CRITIC_APPLY | _lib.TD3_ACTOR_GRAD)
-                if policy_step:
-                    allreduce(self.grads[self.actor_range[0]:self.actor_range[1]])
-                run(_lib.TD3_ACTOR_APPLY)
+            self._phases(run, allreduce if self._peer is None else None, policy_step)  # a peer communicator averages inside the APPLY kernels
         self.launches += 23 if not policy_step else 44  # without the split-K finish kernels of small batches
 
     def train(self, gradient_steps: int, buffer, batch_size: Optional[int] = None, env=None, allreduce=None, graph: bool = False) -> None:
@@ -401,22 +464,11 @@ class FusedTD3Update:
         graph on every rank.  An ``allreduce=`` hook (``dist.all_reduce`` over NCCL) runs launch by launch between the phases unless
         ``CSTR_NCCL_GRAPH=1`` (see ``_hook_capturable``)."""
         bs = int(batch_size or self._batch)
-        done = 0
         if self._peer is not None:
             allreduce = None
-        # a captured cycle bakes the sampling range in: only worth capturing once the ring is full (its range is constant from then on)
-        if graph and _hook_capturable(allreduce) and getattr(buffer, "index_mode", None) == "philox" and buffer.full and _graph_env_ok(env):
-            done = self._train_graph(gradient_steps, buffer, bs, env, allreduce)
+        done = self._train_graph(graph, gradient_steps, buffer, bs, env, allreduce)
         for _ in range(gradient_steps - done):
             self.update(buffer.sample(bs, env=env), allreduce=allreduce)
-
-    def pop_losses(self):
-        """(mean critic loss, mean actor loss or None) since the last call — what TD3.train logs (td3.py:207-210)."""
-        s = self.loss_sums.cpu().numpy().astype(np.float64)
-        self.loss_sums.zero_()
-        critic = s[0] / s[1] if s[1] else None
-        actor = s[2] / s[3] if s[3] else None
-        return critic, actor
 
 
 class _DeviceMemory:
@@ -458,10 +510,11 @@ def fused_update_unsupported(model, max_critics: int = 2) -> Optional[str]:
     4-value observation, a 2-value action, two ReLU hidden layers shared by actor and critics (multiples of 4), 1-2 critics and plain
     Adam.  Anything else keeps the reference's own torch ``train()``."""
     import torch.nn as nn
-    import torch.optim as optim
+
     pol = model.policy
-    if tuple(model.observation_space.shape or ()) != (4,) or tuple(model.action_space.shape or ()) != (2,):
-        return f"spaces {model.observation_space.shape} -> {model.action_space.shape} are not the CSTR's (4,) -> (2,)"
+    why = _spaces_reason(model)
+    if why:
+        return why
     if getattr(pol, "activation_fn", nn.ReLU) is not nn.ReLU:
         return f"activation_fn {pol.activation_fn.__name__} (kernels are ReLU)"
     arch = pol.net_arch
@@ -477,10 +530,29 @@ def fused_update_unsupported(model, max_critics: int = 2) -> Optional[str]:
         return f"n_critics={n_critics}"
     if type(pol.actor.features_extractor).__name__ != "FlattenExtractor":
         return f"features extractor {type(pol.actor.features_extractor).__name__}"
-    for opt in (pol.actor.optimizer, pol.critic.optimizer):
+    opt = _not_plain_adam((pol.actor.optimizer, pol.critic.optimizer))
+    if opt is not None:
+        g = opt.param_groups[0]
+        return f"optimizer {type(opt).__name__} {({k: v for k, v in g.items() if k in ('weight_decay', 'amsgrad', 'maximize')})} (kernels are plain Adam)"
+    return None
+
+
+def _spaces_reason(model) -> Optional[str]:
+    """Why the model's spaces are not the CSTR's flat (4,) observation and (2,) action that every fused kernel is built for, or None."""
+    if tuple(model.observation_space.shape or ()) != (4,) or tuple(model.action_space.shape or ()) != (2,):
+        return f"spaces {model.observation_space.shape} -> {model.action_space.shape} are not the CSTR's (4,) -> (2,)"
+    return None
+
+
+def _not_plain_adam(optimizers):
+    """The first of ``optimizers`` the fused Adam kernels cannot stand in for (not ``torch.optim.Adam``, or with weight decay, amsgrad or
+    maximize), or None."""
+    import torch.optim as optim
+
+    for opt in optimizers:
         g = opt.param_groups[0]
         if type(opt) is not optim.Adam or g.get("weight_decay", 0) or g.get("amsgrad", False) or g.get("maximize", False):
-            return f"optimizer {type(opt).__name__} {({k: v for k, v in g.items() if k in ('weight_decay', 'amsgrad', 'maximize')})} (kernels are plain Adam)"
+            return opt
     return None
 
 
@@ -544,36 +616,33 @@ def bind_td3_class(td3_base: type) -> type:
     return FusedTD3
 
 
-class FusedSACUpdate(FusedTD3Update):
+class FusedSACUpdate(_FusedEngine):
     """SAC gradient steps on the device: one iteration of the loop body of ``SAC.train`` (``core/sac/sac.py:213-288``) per ``update()``
     through ``cstr_sac_update`` — squashed-Gaussian actor sample and log-prob, automatic entropy coefficient, soft twin-min target,
     critics, actor (backward through both critics and the tanh-Gaussian), polyak.  Same flat-block design as :class:`FusedTD3Update`;
     the actor head is ONE (4, h2) matrix [mu; log_std], ``log_ent_coef`` lives in a slot after the three nets."""
 
+    NETS = NET_NAMES
+    TARGET_NETS = NET_NAMES[1:]  # SAC has no target actor
+    N_LOSS = 8
+
     def __init__(self, net_arch: Sequence[int] = (256, 256), batch_size: int = 256, device: Any = "cuda", gamma: float = 0.99, tau: float = 0.005,
                  learning_rate: float = 3e-4, target_entropy: float = -2.0, ent_coef_init: float = 1.0, target_update_interval: int = 1,
                  betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", dp_rank: int = 0):
+        super().__init__(device, gamma, tau, learning_rate, 1, betas, eps, seed, gemm, dp_rank)
+        self._two_hidden(net_arch)
         self.target_entropy, self.target_update_interval = float(target_entropy), int(target_update_interval)
-        super().__init__(net_arch, batch_size, device, gamma, tau, learning_rate, 1, 0.0, 0.0, betas, eps, seed, gemm, dp_rank=dp_rank)
-        torch = self._torch
         offs = (c_int64 * 20)()
         _lib.check(self._libc.cstr_sac_layout(self.h1, self.h2, offs), "cstr_sac_layout")
-        self.param_count = int(offs[19])
-        self._offsets = {(NET_NAMES[n], _TENSORS[k]): int(offs[n * 6 + k]) for n in range(3) for k in range(6)}
         self._ent_offset = int(offs[18])
+        self._allocate(offs, batch_size)
         self.actor_range = (0, self._offsets[("critic0", "W1")])
         self.critic_range = (self._offsets[("critic0", "W1")], self._ent_offset)
-        with torch.cuda.device(self.device):
-            z = lambda: torch.zeros(self.param_count, dtype=torch.float32, device=self.device)  # noqa: E731
-            self.params, self.targets, self.grads, self.adam_m, self.adam_v = z(), z(), z(), z(), z()
-            self.loss_sums = torch.zeros(8, dtype=torch.float32, device=self.device)
+        self._reduced_critic = (self.critic_range[0], self._ent_offset + 4)  # both critics and the log_ent_coef slot, contiguous
         self.params[self._ent_offset] = float(np.log(ent_coef_init))
-        self._batch = 0
-        self._set_batch(int(batch_size))
 
-    def _shape(self, net: str, tensor: str):
-        i, o = (4, 4) if net == "actor" else (6, 1)
-        return {"W1": (self.h1, i), "b1": (self.h1,), "W2": (self.h2, self.h1), "b2": (self.h2,), "W3": (o, self.h2), "b3": (o,)}[tensor]
+    def _dims(self, net: str):
+        return (4, self.h1, self.h2, 4) if net == "actor" else (6, self.h1, self.h2, 1)
 
     @property
     def log_ent_coef(self):
@@ -587,58 +656,23 @@ class FusedSACUpdate(FusedTD3Update):
     def _workspace_bytes(self, batch: int) -> int:
         return int(self._libc.cstr_sac_workspace_bytes(byref(self._sac_config(batch))))
 
-    def load_nets(self, nets: Dict[str, Sequence[Any]]) -> None:
-        """``actor`` (head = [mu; log_std] stacked), ``critic0``, ``critic1`` and optionally ``critic*_target``."""
-        torch = self._torch
-        for block, suffix, names in (("params", "", NET_NAMES), ("targets", "_target", NET_NAMES[1:])):
-            v = self.views(block)
-            for net in names:
-                src = nets.get(net + suffix, nets[net])
-                for dst, s in zip(v[net], src):
-                    dst.copy_(torch.as_tensor(np.asarray(s) if not isinstance(s, torch.Tensor) else s).to(self.device, torch.float32).reshape(dst.shape))
-
-    def nets(self) -> Dict[str, List[np.ndarray]]:
-        out = {net: [t.cpu().numpy() for t in ts] for net, ts in self.views("params").items()}
-        out.update({net + "_target": [t.cpu().numpy() for t in ts] for net, ts in self.views("targets").items() if net != "actor"})
-        return out
-
     def adopt_policy(self, policy) -> None:
         """The reference's ``SACPolicy`` (core/sac/policies.py): ``actor.latent_pi`` + ``actor.mu`` + ``actor.log_std``, twin critics."""
         a, v, t = policy.actor, self.views("params"), self.views("targets")
-        lat = list(a.latent_pi.parameters())
-        pairs = list(zip(v["actor"][:4], lat)) + [(v["actor"][4][0:2], a.mu.weight), (v["actor"][4][2:4], a.log_std.weight),
-                                                 (v["actor"][5][0:2], a.mu.bias), (v["actor"][5][2:4], a.log_std.bias)]
+        head_w, head_b = v["actor"][4], v["actor"][5]
+        online = list(zip(v["actor"][:4], a.latent_pi.parameters())) + [(head_w[0:2], a.mu.weight), (head_w[2:4], a.log_std.weight),
+                                                                        (head_b[0:2], a.mu.bias), (head_b[2:4], a.log_std.bias)]
+        targets = []
         for z, q in enumerate(policy.critic.q_networks):
-            pairs += list(zip(v[f"critic{z}"], q.parameters()))
+            online += zip(v[f"critic{z}"], q.parameters())
         for z, q in enumerate(policy.critic_target.q_networks):
-            pairs += list(zip(t[f"critic{z}"], q.parameters()))
-        for view, p in pairs:
-            if tuple(p.shape) != tuple(view.shape):
-                raise ValueError(f"shape mismatch: module {tuple(p.shape)} vs layout {tuple(view.shape)}")
-            view.copy_(p.data.to(self.device, self._torch.float32))
-            p.data = view
-        # Adam moment views per module parameter (same slicing as the weights), for import/export_optimizer_state
-        am, av = self.views("adam_m"), self.views("adam_v")
-        head = lambda blk: [blk["actor"][4][0:2], blk["actor"][4][2:4], blk["actor"][5][0:2], blk["actor"][5][2:4]]  # noqa: E731
-        actor_params = lat + [a.mu.weight, a.log_std.weight, a.mu.bias, a.log_std.bias]
-        critic_params = [p for q in policy.critic.q_networks for p in q.parameters()]
-        self._moments = {id(p): mv for p, mv in zip(actor_params, zip(am["actor"][:4] + head(am), av["actor"][:4] + head(av)))}
-        self._moments.update({id(p): mv for p, mv in zip(critic_params, zip(am["critic0"] + am["critic1"], av["critic0"] + av["critic1"]))})
+            targets += zip(t[f"critic{z}"], q.parameters())
+        self._adopt(online, targets)
 
-    def import_optimizer_state(self, actor_optimizer, critic_optimizer, ent_coef_optimizer=None) -> None:  # type: ignore[override]
+    def import_optimizer_state(self, actor_optimizer, critic_optimizer, ent_coef_optimizer=None) -> None:
         """Take over Adam moments / the step count of the reference's three optimisers (sac.py:187, policies.py:264-284) after ``adopt_policy``.
         One step count serves all three: the reference steps each exactly once per gradient step."""
-        step = 0
-        for opt in (actor_optimizer, critic_optimizer):
-            group = opt.param_groups[0]
-            self.betas, self.eps = (float(group["betas"][0]), float(group["betas"][1])), float(group["eps"])
-            for p in group["params"]:
-                st = opt.state.get(p)
-                if st and id(p) in self._moments:
-                    m, v = self._moments[id(p)]
-                    m.copy_(st["exp_avg"])
-                    v.copy_(st["exp_avg_sq"])
-                    step = max(step, int(float(st["step"])))
+        step = max(self._import_adam(actor_optimizer), self._import_adam(critic_optimizer))
         if ent_coef_optimizer is not None:
             for p in ent_coef_optimizer.param_groups[0]["params"]:
                 st = ent_coef_optimizer.state.get(p)
@@ -648,33 +682,25 @@ class FusedSACUpdate(FusedTD3Update):
                     step = max(step, int(float(st["step"])))
         self.critic_step = self.actor_step = step
 
-    def export_optimizer_state(self, actor_optimizer, critic_optimizer, ent_coef_optimizer=None) -> None:  # type: ignore[override]
+    def export_optimizer_state(self, actor_optimizer, critic_optimizer, ent_coef_optimizer=None) -> None:
         """Write moments / step count back so ``model.save`` and a later torch ``optimizer.step()`` continue from here."""
-        torch = self._torch
-        if self.critic_step == 0:
-            return
-        step = lambda: torch.tensor(float(self.critic_step))  # noqa: E731
-        for opt in (actor_optimizer, critic_optimizer):
-            for p in opt.param_groups[0]["params"]:
-                if id(p) in self._moments:
-                    m, v = self._moments[id(p)]
-                    opt.state[p] = {"step": step(), "exp_avg": m, "exp_avg_sq": v}
-        if ent_coef_optimizer is not None:
+        step = self.critic_step
+        self._export_adam(actor_optimizer, step)
+        self._export_adam(critic_optimizer, step)
+        if ent_coef_optimizer is not None and step:
             e = self._ent_offset
             for p in ent_coef_optimizer.param_groups[0]["params"]:
-                ent_coef_optimizer.state[p] = {"step": step(), "exp_avg": self.adam_m[e:e + 1].reshape(p.shape), "exp_avg_sq": self.adam_v[e:e + 1].reshape(p.shape)}
+                ent_coef_optimizer.state[p] = {"step": self._torch.tensor(float(step)), "exp_avg": self.adam_m[e:e + 1].reshape(p.shape),
+                                               "exp_avg_sq": self.adam_v[e:e + 1].reshape(p.shape)}
 
-    def update(self, batch, eps_pi=None, eps_next=None, allreduce: Optional[Callable[[Any], None]] = None,  # type: ignore[override]
+    def update(self, batch, eps_pi=None, eps_next=None, allreduce: Optional[Callable[[Any], None]] = None,
                gradient_step: Optional[int] = None) -> None:
         """One iteration of sac.py:213-288.  ``eps_pi`` / ``eps_next``: explicit standard-normal draws (B,2) of the two rsample() calls
         (parity tests); default = Philox inside the kernel.  ``allreduce``: called on grads[critics .. log_ent_coef] and on grads[actor]
         between backward and Adam (data-parallel training: every rank ends with the gradient of the global batch).
         ``gradient_step``: the index of this step inside the current ``train()`` call — what the reference's target sync tests
         (``gradient_step % target_update_interval``, sac.py:284); None = the engine's own running count of updates."""
-        obs, act, nobs, dones, rew = batch
-        self._set_batch(int(obs.shape[0]))
-        obs, act, nobs = self._f32(obs, 4), self._f32(act, 2), self._f32(nobs, 4)
-        dones, rew = self._f32(dones, 1), self._f32(rew, 1)
+        obs, act, nobs, dones, rew = self._batch_f32(batch)
         e1 = None if eps_pi is None else self._f32(eps_pi, 2)
         e2 = None if eps_next is None else self._f32(eps_next, 2)
         self.n_updates += 1
@@ -689,14 +715,7 @@ class FusedSACUpdate(FusedTD3Update):
             _lib.check(rc, "cstr_sac_update")
 
         with self._torch.cuda.device(self.device):
-            if allreduce is None or self._peer is not None:
-                run(_lib.TD3_ALL)
-            else:
-                run(_lib.TD3_CRITIC_GRAD)
-                allreduce(self.grads[self.critic_range[0]:self._ent_offset + 4])  # both critics and the log_ent_coef slot, contiguous
-                run(_lib.TD3_CRITIC_APPLY | _lib.TD3_ACTOR_GRAD)
-                allreduce(self.grads[self.actor_range[0]:self.actor_range[1]])
-                run(_lib.TD3_ACTOR_APPLY)
+            self._phases(run, allreduce if self._peer is None else None, True)
         self.launches += 50
 
     def _graph_launch(self, batch_size: int, st, out, k: int, allreduce=None) -> None:
@@ -707,32 +726,16 @@ class FusedSACUpdate(FusedTD3Update):
                                             _lib.ptr(out[4]), None, None, 1, 1, phases, self._stream())
             _lib.check(rc, "cstr_sac_update (graph capture)")
 
-        if allreduce is None:
-            run(_lib.TD3_ALL)
-        else:
-            run(_lib.TD3_CRITIC_GRAD)
-            allreduce(self.grads[self.critic_range[0]:self._ent_offset + 4])
-            run(_lib.TD3_CRITIC_APPLY | _lib.TD3_ACTOR_GRAD)
-            allreduce(self.grads[self.actor_range[0]:self.actor_range[1]])
-            run(_lib.TD3_ACTOR_APPLY)
+        self._phases(run, allreduce, True)
 
-    def train(self, gradient_steps: int, buffer, batch_size: Optional[int] = None, env=None, allreduce=None, graph: bool = False) -> None:  # type: ignore[override]
+    def train(self, gradient_steps: int, buffer, batch_size: Optional[int] = None, env=None, allreduce=None, graph: bool = False) -> None:
         """``graph=True`` (single GPU, Philox-index buffer, full ring, target_update_interval 1): every update replays one captured CUDA graph."""
         bs = int(batch_size or self._batch)
-        done = 0
         if self._peer is not None:
             allreduce = None
-        if (graph and _hook_capturable(allreduce) and getattr(buffer, "index_mode", None) == "philox" and buffer.full and self.target_update_interval == 1
-                and _graph_env_ok(env)):
-            done = self._train_graph(gradient_steps, buffer, bs, env, allreduce)
+        done = self._train_graph(graph and self.target_update_interval == 1, gradient_steps, buffer, bs, env, allreduce)
         for g in range(done, gradient_steps):  # g = the reference's loop index: the target sync tests `g % target_update_interval` (sac.py:284)
             self.update(buffer.sample(bs, env=env), allreduce=allreduce, gradient_step=g)
-
-    def pop_losses(self):
-        """(critic loss, actor loss, ent_coef_loss, ent_coef) means since the last call — the keys SAC.train logs (sac.py:290-296)."""
-        s = self.loss_sums.cpu().numpy().astype(np.float64)
-        self.loss_sums.zero_()
-        return tuple(s[2 * i] / s[2 * i + 1] if s[2 * i + 1] else None for i in range(4))
 
 
 def bind_sac_class(sac_base: type) -> type:

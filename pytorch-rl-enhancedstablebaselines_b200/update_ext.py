@@ -7,9 +7,10 @@ the reference's ``(B, 10)`` reshape as written), the twin critics, and the delay
 ``FusedMultiAgentUpdate`` runs one iteration of ``MADDPG.train`` / ``IDDPG.train`` (``core/maddpg/maddpg.py:127-185``,
 ``core/iddpg/iddpg.py:127-185``) through ``cstr_ma_update`` for the two-reactor agents of BASELINE config #5.
 
-Both keep five flat float32 device blocks (``params, targets, grads, adam_m, adam_v``) like :class:`FusedTD3Update`, whose plumbing
-(workspace, CUDA-graph replay, the peer-memory gradient all-reduce) they inherit; ``bind_bcq_class`` / ``bind_multiagent_class`` return
-subclasses of the reference algorithms whose ``train()`` runs here and whose policy modules share memory with the flat blocks.
+Both keep five flat float32 device blocks (``params, targets, grads, adam_m, adam_v``) like :class:`FusedTD3Update`; the plumbing
+(workspace, module and Adam hand-over, CUDA-graph replay, the peer-memory gradient all-reduce) is ``update._FusedEngine``'s.
+``bind_bcq_class`` / ``bind_multiagent_class`` return subclasses of the reference algorithms whose ``train()`` runs here and whose policy
+modules share memory with the flat blocks.
 """
 from __future__ import annotations
 
@@ -19,74 +20,20 @@ from typing import Any, Dict, List, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from .update import _GEMM_MODES, _TENSORS, FusedTD3Update, _dist_rank, _fallback_once, _graph_env_ok
+from .update import _GEMM_MODES, _FusedEngine, _dist_rank, _fallback_once, _not_plain_adam, _spaces_reason
 
 
-class _FlatEngine(FusedTD3Update):
-    """Shared set-up of the engines below: the flat blocks, counters and the attributes FusedTD3Update's plumbing reads."""
+class _FlatEngine(_FusedEngine):
+    """BCQ and multi-agent engines: no host-side all-reduce hook, so ``train`` runs ``update`` without one."""
 
-    NETS: Sequence[str] = ()
-    N_LOSS = 4
-
-    def _base_init(self, device, batch_size, gamma, tau, learning_rate, betas, eps, seed, gemm, dp_rank, cycle) -> None:
-        torch = _lib.require_cuda()
-        self._torch, self._libc = torch, _lib.load()
-        self.device = torch.device(device)
-        if self.device.type != "cuda":
-            raise _lib.CstrLibraryError(f"{type(self).__name__} needs a CUDA device (no CPU fallback)")
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        if gemm not in _GEMM_MODES:
-            raise ValueError("gemm must be 'fp32', 'tensor' or 'bf16'")
-        self.gamma, self.tau, self.learning_rate = float(gamma), float(tau), float(learning_rate)
-        self.betas, self.eps, self.seed, self.gemm, self.dp_rank = (float(betas[0]), float(betas[1])), float(eps), int(seed), gemm, int(dp_rank)
-        self.policy_delay = int(cycle)  # the length of a captured graph cycle
-        self._graph = self._graph_key = self._graph_out = self._peer = self._workspace = None
-        self._batch = 0
-        self.n_updates = self.critic_step = self.actor_step = self.launches = 0
-        self._initial_batch = int(batch_size)
-
-    def _alloc_blocks(self) -> None:
-        torch = self._torch
-        with torch.cuda.device(self.device):
-            z = lambda: torch.zeros(self.param_count, dtype=torch.float32, device=self.device)  # noqa: E731
-            self.params, self.targets, self.grads, self.adam_m, self.adam_v = z(), z(), z(), z(), z()
-            self.loss_sums = torch.zeros(self.N_LOSS, dtype=torch.float32, device=self.device)
-            self._counters = torch.zeros(4, dtype=torch.int64, device=self.device)
-        self._set_batch(self._initial_batch)
-
-    def views(self, block: str = "params") -> Dict[str, List[Any]]:
-        flat = getattr(self, block)
-        out = {}
-        for net in self.NETS:
-            out[net] = []
-            for t in _TENSORS:
-                shape, off = self._shape(net, t), self._offsets[(net, t)]
-                out[net].append(flat[off:off + int(np.prod(shape))].view(shape))
-        return out
-
-    def _copy_in(self, dst, src) -> None:
-        torch = self._torch
-        dst.copy_(torch.as_tensor(np.asarray(src) if not isinstance(src, torch.Tensor) else src).to(self.device, torch.float32).reshape(dst.shape))
-
-    def _cycle_len(self) -> int:
-        return self.policy_delay
-
-    def pop_losses(self):
-        s = self.loss_sums.cpu().numpy().astype(np.float64)
-        self.loss_sums.zero_()
-        return tuple(s[2 * i] / s[2 * i + 1] if s[2 * i + 1] else None for i in range(self.N_LOSS // 2))
-
-    def train(self, gradient_steps: int, buffer, batch_size: Optional[int] = None, env=None, allreduce=None, graph: bool = False) -> None:  # type: ignore[override]
+    def train(self, gradient_steps: int, buffer, batch_size: Optional[int] = None, env=None, allreduce=None, graph: bool = False) -> None:
         """sample + update, ``gradient_steps`` times; ``graph=True`` (Philox-index buffer, full ring) replays whole cycles of ``actor_delay`` /
         ``policy_delay`` updates from one captured CUDA graph.  Data-parallel training: ``enable_peer_allreduce()`` (the averaging is part of the
         Adam kernels); a host-side ``allreduce=`` hook is not offered for these engines."""
         if allreduce is not None:
             raise ValueError("data-parallel BCQ / multi-agent updates average their gradients through enable_peer_allreduce()")
         bs = int(batch_size or self._batch)
-        done = 0
-        if graph and getattr(buffer, "index_mode", None) == "philox" and buffer.full and _graph_env_ok(env):
-            done = self._train_graph(gradient_steps, buffer, bs, env, None)
+        done = self._train_graph(graph, gradient_steps, buffer, bs, env, None)
         for _ in range(gradient_steps - done):
             self.update(buffer.sample(bs, env=env))
 
@@ -98,29 +45,24 @@ class FusedBCQUpdate(_FlatEngine):
     def __init__(self, latent_dim: int = 32, vae_hidden: int = 64, pert_hidden: int = 64, critic_arch: Sequence[int] = (400, 300), batch_size: int = 256,
                  device: Any = "cuda", gamma: float = 0.99, tau: float = 0.005, learning_rate: float = 1e-3, max_perturbation: float = 0.05,
                  actor_delay: int = 2, n_candidates: int = 10, betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", dp_rank: int = 0):
-        self._base_init(device, batch_size, gamma, tau, learning_rate, betas, eps, seed, gemm, dp_rank, actor_delay)
-        if len(critic_arch) != 2:
-            raise ValueError("critic_arch must be [h1, h2]")
+        super().__init__(device, gamma, tau, learning_rate, actor_delay, betas, eps, seed, gemm, dp_rank)
+        self._two_hidden(critic_arch)
         self.latent, self.vae_hidden, self.pert_hidden = int(latent_dim), int(vae_hidden), int(pert_hidden)
-        self.h1, self.h2 = int(critic_arch[0]), int(critic_arch[1])
         self.max_perturbation, self.actor_delay, self.n_candidates = float(max_perturbation), int(actor_delay), int(n_candidates)
         offs = (c_int64 * 31)()
         rc = self._libc.cstr_bcq_layout(byref(self._config(1)), offs)
         if rc:
             msg = self._libc.cstr_last_error()
             raise ValueError(msg.decode() if msg else "bad BCQ configuration")
-        self.param_count = int(offs[30])
-        self._offsets = {(self.NETS[n], _TENSORS[k]): int(offs[n * 6 + k]) for n in range(5) for k in range(6)}
+        self._allocate(offs, batch_size)
         self.vae_range = (0, self._offsets[("pert", "W1")])
         self.pert_range = (self._offsets[("pert", "W1")], self._offsets[("critic0", "W1")])
         self.critic_range = (self._offsets[("critic0", "W1")], self.param_count)
-        self._alloc_blocks()
 
-    def _shape(self, net: str, tensor: str):
+    def _dims(self, net: str):
         L, Hv, Hp = self.latent, self.vae_hidden, self.pert_hidden
-        i, h1, h2, o = {"vae_enc": (6, Hv, Hv, 2 * L), "vae_dec": (4 + L, Hv, Hv, 2), "pert": (6, Hp, Hp, 2), "critic0": (6, self.h1, self.h2, 1),
-                        "critic1": (6, self.h1, self.h2, 1)}[net]
-        return {"W1": (h1, i), "b1": (h1,), "W2": (h2, h1), "b2": (h2,), "W3": (o, h2), "b3": (o,)}[tensor]
+        return {"vae_enc": (6, Hv, Hv, 2 * L), "vae_dec": (4 + L, Hv, Hv, 2), "pert": (6, Hp, Hp, 2), "critic0": (6, self.h1, self.h2, 1),
+                "critic1": (6, self.h1, self.h2, 1)}[net]
 
     def _config(self, batch: int) -> "_lib.BcqConfig":
         return _lib.BcqConfig(latent=self.latent, vae_hidden=self.vae_hidden, pert_hidden=self.pert_hidden, h1=self.h1, h2=self.h2, batch=batch,
@@ -131,38 +73,23 @@ class FusedBCQUpdate(_FlatEngine):
     def _workspace_bytes(self, batch: int) -> int:
         return int(self._libc.cstr_bcq_workspace_bytes(byref(self._config(batch))))
 
-    def load_nets(self, nets: Dict[str, Sequence[Any]]) -> None:
-        """``vae_enc`` (head = [mean; log_std] stacked), ``vae_dec``, ``pert``, ``critic0``, ``critic1`` and optionally ``pert_target`` /
-        ``critic*_target`` (default: copies), six arrays each in nn.Linear layout."""
-        v, t = self.views("params"), self.views("targets")
-        for net in self.NETS:
-            for dst, s in zip(v[net], nets[net]):
-                self._copy_in(dst, s)
-            for dst, s in zip(t[net], nets.get(net + "_target", nets[net])):
-                self._copy_in(dst, s)
-
     def nets(self) -> Dict[str, List[np.ndarray]]:
-        out = {net: [x.cpu().numpy() for x in ts] for net, ts in self.views("params").items()}
-        for net, ts in self.views("targets").items():  # the target VAE is a copy of the VAE (bcq.py:158-159)
-            out[net + "_target"] = out[net] if net.startswith("vae") else [x.cpu().numpy() for x in ts]
+        out = super().nets()
+        out.update({net + "_target": out[net] for net in ("vae_enc", "vae_dec")})  # the target VAE is a copy of the VAE (bcq.py:158-159)
         return out
 
-    def update(self, batch, eps_vae=None, z_next=None, z_actor=None) -> None:  # type: ignore[override]
+    def update(self, batch, eps_vae=None, z_next=None, z_actor=None) -> None:
         """One iteration of bcq.py:137-205.  ``eps_vae`` (B, L), ``z_next`` (n_candidates*B, L), ``z_actor`` (B, L): explicit standard-normal
         draws (unclamped) for parity tests; default = Philox inside the kernels."""
-        obs, act, nobs, dones, rew = batch
-        B = int(obs.shape[0])
-        self._set_batch(B)
-        obs, act, nobs = self._f32(obs, 4), self._f32(act, 2), self._f32(nobs, 4)
-        dones, rew = self._f32(dones, 1), self._f32(rew, 1)
+        obs, act, nobs, dones, rew = self._batch_f32(batch)
         L = self.latent
-        draws = [None if d is None else self._draw(d, rows * L) for d, rows in ((eps_vae, B), (z_next, B * self.n_candidates), (z_actor, B))]
+        draws = [None if d is None else self._f32(d, cols) for d, cols in ((eps_vae, L), (z_next, self.n_candidates * L), (z_actor, L))]
         self.n_updates += 1
         self.critic_step += 1
         actor_now = self.n_updates % self.actor_delay == 0
         if actor_now:
             self.actor_step += 1
-        cfg, st = self._config(B), self._state(counters=False)
+        cfg, st = self._config(self._batch), self._state(counters=False)
         with self._torch.cuda.device(self.device):
             rc = self._libc.cstr_bcq_update(byref(cfg), byref(st), _lib.ptr(obs), _lib.ptr(act), _lib.ptr(nobs), _lib.ptr(dones), _lib.ptr(rew),
                                             _lib.ptr(draws[0]), _lib.ptr(draws[1]), _lib.ptr(draws[2]), self.n_updates, self.critic_step,
@@ -170,100 +97,52 @@ class FusedBCQUpdate(_FlatEngine):
         _lib.check(rc, "cstr_bcq_update")
         self.launches += 92 if actor_now else 66
 
-    def _draw(self, t, numel):
-        torch = self._torch
-        if not isinstance(t, torch.Tensor):
-            t = torch.as_tensor(np.ascontiguousarray(t), device=self.device)
-        t = t.to(device=self.device, dtype=torch.float32).contiguous()
-        if t.numel() != numel:
-            raise ValueError(f"latent draw has {t.numel()} elements, expected {numel}")
-        return t
-
     def _graph_launch(self, batch_size: int, st, out, k: int, allreduce=None) -> None:
         cfg = self._config(batch_size)
         rc = self._libc.cstr_bcq_update(byref(cfg), byref(st), _lib.ptr(out[0]), _lib.ptr(out[1]), _lib.ptr(out[2]), _lib.ptr(out[3]), _lib.ptr(out[4]),
                                         None, None, None, k, 1, 1, self._stream())
         _lib.check(rc, "cstr_bcq_update (graph capture)")
 
-    def _train_graph(self, gradient_steps, buffer, batch_size, env, allreduce=None) -> int:
-        before = self.actor_step
-        done = super()._train_graph(gradient_steps, buffer, batch_size, env, None)
-        self.actor_step = before + done // self.actor_delay
-        return done
-
     # ---- the reference's BCQPolicy (core/bcq/policies.py:263-452) ---------------------------------------------------------------
     def adopt_policy(self, policy) -> None:
         """Copy the weights of the reference's ``BCQPolicy`` in and re-point its parameters at the flat blocks.  The target VAE's parameters
         are pointed at the VAE's own storage: the reference overwrites it with the VAE after every step (bcq.py:158-159, 198)."""
-        vae, vae_t = policy.actor.vae, policy.actor_target.vae
-        v, t = self.views("params"), self.views("targets")
-        L = self.latent
-        enc = list(vae.encoder.parameters())
+        v, t, L = self.views("params"), self.views("targets"), self.latent
+        enc = v["vae_enc"]
 
-        def vae_pairs(views, module_vae):
-            e = list(module_vae.encoder.parameters())
-            return (list(zip(views["vae_enc"][:4], e)) + [(views["vae_enc"][4][0:L], module_vae.mean.weight), (views["vae_enc"][4][L:2 * L], module_vae.log_std.weight),
-                                                           (views["vae_enc"][5][0:L], module_vae.mean.bias), (views["vae_enc"][5][L:2 * L], module_vae.log_std.bias)]
-                    + list(zip(views["vae_dec"], module_vae.decoder.parameters())))
+        def vae_pairs(vae):
+            return (list(zip(enc[:4], vae.encoder.parameters())) + [(enc[4][0:L], vae.mean.weight), (enc[4][L:2 * L], vae.log_std.weight),
+                                                                   (enc[5][0:L], vae.mean.bias), (enc[5][L:2 * L], vae.log_std.bias)]
+                    + list(zip(v["vae_dec"], vae.decoder.parameters())))
 
-        pairs = vae_pairs(v, vae) + list(zip(v["pert"], policy.actor.perturbation.model.parameters()))
-        pairs += list(zip(t["pert"], policy.actor_target.perturbation.model.parameters()))
+        online = vae_pairs(policy.actor.vae) + list(zip(v["pert"], policy.actor.perturbation.model.parameters()))
+        targets = list(zip(t["pert"], policy.actor_target.perturbation.model.parameters()))
         for z, q in enumerate(policy.critic.q_networks):
-            pairs += list(zip(v[f"critic{z}"], q.parameters()))
+            online += zip(v[f"critic{z}"], q.parameters())
         for z, q in enumerate(policy.critic_target.q_networks):
-            pairs += list(zip(t[f"critic{z}"], q.parameters()))
-        for view, p in pairs:
-            if tuple(p.shape) != tuple(view.shape):
-                raise ValueError(f"shape mismatch: module {tuple(p.shape)} vs layout {tuple(view.shape)}")
-            view.copy_(p.data.to(self.device, self._torch.float32))
+            targets += zip(t[f"critic{z}"], q.parameters())
+        self._adopt(online, targets)
+        for view, p in vae_pairs(policy.actor_target.vae):  # shared storage with the VAE
             p.data = view
-        for view, p in vae_pairs(v, vae_t):  # shared storage with the VAE
-            p.data = view
-        am, av = self.views("adam_m"), self.views("adam_v")
-        self._moments = {}
-        for (m, p), (vv, _) in zip(vae_pairs(am, vae) + list(zip(am["pert"], policy.actor.perturbation.model.parameters())),
-                                   vae_pairs(av, vae) + list(zip(av["pert"], policy.actor.perturbation.model.parameters()))):
-            self._moments[id(p)] = (m, vv)
-        for z, q in enumerate(policy.critic.q_networks):
-            for p, m, vv in zip(q.parameters(), am[f"critic{z}"], av[f"critic{z}"]):
-                self._moments[id(p)] = (m, vv)
-        del enc
 
-    def import_optimizer_state(self, vae_optimizer, perturbation_optimizer, critic_optimizer) -> None:  # type: ignore[override]
-        steps = []
-        for opt in (vae_optimizer, perturbation_optimizer, critic_optimizer):
-            group = opt.param_groups[0]
-            self.betas, self.eps = (float(group["betas"][0]), float(group["betas"][1])), float(group["eps"])
-            step = 0
-            for p in group["params"]:
-                st = opt.state.get(p)
-                if st and id(p) in self._moments:
-                    m, v = self._moments[id(p)]
-                    m.copy_(st["exp_avg"])
-                    v.copy_(st["exp_avg_sq"])
-                    step = max(step, int(float(st["step"])))
-            steps.append(step)
-        self.critic_step, self.actor_step = max(steps[0], steps[2]), steps[1]
+    def import_optimizer_state(self, vae_optimizer, perturbation_optimizer, critic_optimizer) -> None:
+        vae, pert, critic = (self._import_adam(opt) for opt in (vae_optimizer, perturbation_optimizer, critic_optimizer))
+        self.critic_step, self.actor_step = max(vae, critic), pert
 
-    def export_optimizer_state(self, vae_optimizer, perturbation_optimizer, critic_optimizer) -> None:  # type: ignore[override]
-        torch = self._torch
-        for opt, step in ((vae_optimizer, self.critic_step), (perturbation_optimizer, self.actor_step), (critic_optimizer, self.critic_step)):
-            if step == 0:
-                continue
-            for p in opt.param_groups[0]["params"]:
-                if id(p) in self._moments:
-                    m, v = self._moments[id(p)]
-                    opt.state[p] = {"step": torch.tensor(float(step)), "exp_avg": m, "exp_avg_sq": v}
+    def export_optimizer_state(self, vae_optimizer, perturbation_optimizer, critic_optimizer) -> None:
+        self._export_adam(vae_optimizer, self.critic_step)
+        self._export_adam(perturbation_optimizer, self.actor_step)
+        self._export_adam(critic_optimizer, self.critic_step)
 
 
 def bcq_update_unsupported(model) -> Optional[str]:
     """Why ``cstr_bcq_update`` can NOT stand in for ``model.train()`` — or None when it can."""
     import torch.nn as nn
-    import torch.optim as optim
 
     pol = model.policy
-    if tuple(model.observation_space.shape or ()) != (4,) or tuple(model.action_space.shape or ()) != (2,):
-        return f"spaces {model.observation_space.shape} -> {model.action_space.shape} are not the CSTR's (4,) -> (2,)"
+    why = _spaces_reason(model)
+    if why:
+        return why
     if getattr(pol, "activation_fn", nn.ReLU) is not nn.ReLU:
         return "activation_fn is not ReLU"
     arch = pol.actor_arch
@@ -274,10 +153,9 @@ def bcq_update_unsupported(model) -> Optional[str]:
         return f"critic_net_arch {c} / n_critics {len(pol.critic.q_networks)}: two hidden layers (multiples of 4) and two critics"
     if type(pol.actor.features_extractor).__name__ != "FlattenExtractor":
         return f"features extractor {type(pol.actor.features_extractor).__name__}"
-    for opt in (pol.actor.vae_optimizer, pol.actor.perturbation_optimizer, pol.critic.optimizer):
-        g = opt.param_groups[0]
-        if type(opt) is not optim.Adam or g.get("weight_decay", 0) or g.get("amsgrad", False) or g.get("maximize", False):
-            return f"optimizer {type(opt).__name__} is not plain Adam"
+    opt = _not_plain_adam((pol.actor.vae_optimizer, pol.actor.perturbation_optimizer, pol.critic.optimizer))
+    if opt is not None:
+        return f"optimizer {type(opt).__name__} is not plain Adam"
     return None
 
 
@@ -344,26 +222,21 @@ class FusedMultiAgentUpdate(_FlatEngine):
                  tau: float = 0.005, actor_lrs: Sequence[float] = (1e-3, 1e-3), critic_lrs: Sequence[float] = (1e-3, 1e-3), policy_delay: int = 2,
                  target_policy_noise: float = 0.2, target_noise_clip: float = 0.5, n_critics: int = 2, betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0,
                  gemm: str = "fp32", dp_rank: int = 0):
-        self._base_init(device, batch_size, gamma, tau, actor_lrs[0], betas, eps, seed, gemm, dp_rank, policy_delay)
-        if len(net_arch) != 2:
-            raise ValueError("net_arch must be [h1, h2]")
-        self.h1, self.h2, self.centralised, self.n_critics = int(net_arch[0]), int(net_arch[1]), bool(centralised), int(n_critics)
+        super().__init__(device, gamma, tau, actor_lrs[0], policy_delay, betas, eps, seed, gemm, dp_rank)
+        self._two_hidden(net_arch)
+        self.centralised, self.n_critics = bool(centralised), int(n_critics)
         self.actor_lrs, self.critic_lrs = [float(x) for x in actor_lrs], [float(x) for x in critic_lrs]
         self.target_policy_noise, self.target_noise_clip = float(target_policy_noise), float(target_noise_clip)
         self.NETS = tuple([f"actor{i}" for i in range(2)] + [f"critic{i}_{k}" for i in range(2) for k in range(self.n_critics)])
-        n_nets = len(self.NETS)
-        offs = (c_int64 * (n_nets * 6 + 1))()
+        offs = (c_int64 * (len(self.NETS) * 6 + 1))()
         rc = self._libc.cstr_ma_layout(byref(self._config(1)), offs)
         if rc:
             msg = self._libc.cstr_last_error()
             raise ValueError(msg.decode() if msg else "bad multi-agent configuration")
-        self.param_count = int(offs[n_nets * 6])
-        self._offsets = {(self.NETS[n], _TENSORS[k]): int(offs[n * 6 + k]) for n in range(n_nets) for k in range(6)}
-        self._alloc_blocks()
+        self._allocate(offs, batch_size)
 
-    def _shape(self, net: str, tensor: str):
-        i = 2 if net.startswith("actor") else (6 if self.centralised else 3)
-        return {"W1": (self.h1, i), "b1": (self.h1,), "W2": (self.h2, self.h1), "b2": (self.h2,), "W3": (1, self.h2), "b3": (1,)}[tensor]
+    def _dims(self, net: str):
+        return (2 if net.startswith("actor") else (6 if self.centralised else 3), self.h1, self.h2, 1)
 
     def _config(self, batch: int) -> "_lib.MaConfig":
         cfg = _lib.MaConfig(centralised=int(self.centralised), h1=self.h1, h2=self.h2, batch=batch, policy_delay=self.policy_delay, n_critics=self.n_critics,
@@ -376,27 +249,11 @@ class FusedMultiAgentUpdate(_FlatEngine):
     def _workspace_bytes(self, batch: int) -> int:
         return int(self._libc.cstr_ma_workspace_bytes(byref(self._config(batch))))
 
-    def load_nets(self, nets: Dict[str, Sequence[Any]]) -> None:
-        v, t = self.views("params"), self.views("targets")
-        for net in self.NETS:
-            for dst, s in zip(v[net], nets[net]):
-                self._copy_in(dst, s)
-            for dst, s in zip(t[net], nets.get(net + "_target", nets[net])):
-                self._copy_in(dst, s)
-
-    def nets(self) -> Dict[str, List[np.ndarray]]:
-        out = {net: [x.cpu().numpy() for x in ts] for net, ts in self.views("params").items()}
-        out.update({net + "_target": [x.cpu().numpy() for x in ts] for net, ts in self.views("targets").items()})
-        return out
-
-    def update(self, batch, noise=None) -> None:  # type: ignore[override]
+    def update(self, batch, noise=None) -> None:
         """One iteration of maddpg.py / iddpg.py :127-185.  ``noise``: explicit N(0, target_policy_noise) draws, (2, B) agent-major (or a
         sequence of two (B, 1) arrays), for parity tests; default = Philox in the kernel."""
-        obs, act, nobs, dones, rew = batch
-        B = int(obs.shape[0])
-        self._set_batch(B)
-        obs, act, nobs = self._f32(obs, 4), self._f32(act, 2), self._f32(nobs, 4)
-        dones, rew = self._f32(dones, 1), self._f32(rew, 1)
+        obs, act, nobs, dones, rew = self._batch_f32(batch)
+        B = self._batch
         nz = None
         if noise is not None:
             torch = self._torch
@@ -431,51 +288,24 @@ class FusedMultiAgentUpdate(_FlatEngine):
     # ---- the reference's MADDPGPolicy / IDDPGPolicy (core/maddpg/policies.py:281-500) -------------------------------------------------
     def adopt_policy(self, policy) -> None:
         v, t = self.views("params"), self.views("targets")
-        am, av = self.views("adam_m"), self.views("adam_v")
-        pairs, self._moments = [], {}
+        online, targets = [], []
         for i in range(2):
-            pairs += list(zip(v[f"actor{i}"], policy.actor.mu_list[i].parameters())) + list(zip(t[f"actor{i}"], policy.actor_target.mu_list[i].parameters()))
-            for p, m, vv in zip(policy.actor.mu_list[i].parameters(), am[f"actor{i}"], av[f"actor{i}"]):
-                self._moments[id(p)] = (m, vv)
+            online += zip(v[f"actor{i}"], policy.actor.mu_list[i].parameters())
+            targets += zip(t[f"actor{i}"], policy.actor_target.mu_list[i].parameters())
             for k in range(self.n_critics):
-                q, qt = policy.critic.q_networks_list[i][k], policy.critic_target.q_networks_list[i][k]
-                pairs += list(zip(v[f"critic{i}_{k}"], q.parameters())) + list(zip(t[f"critic{i}_{k}"], qt.parameters()))
-                for p, m, vv in zip(q.parameters(), am[f"critic{i}_{k}"], av[f"critic{i}_{k}"]):
-                    self._moments[id(p)] = (m, vv)
-        for view, p in pairs:
-            if tuple(p.shape) != tuple(view.shape):
-                raise ValueError(f"shape mismatch: module {tuple(p.shape)} vs layout {tuple(view.shape)}")
-            view.copy_(p.data.to(self.device, self._torch.float32))
-            p.data = view
+                online += zip(v[f"critic{i}_{k}"], policy.critic.q_networks_list[i][k].parameters())
+                targets += zip(t[f"critic{i}_{k}"], policy.critic_target.q_networks_list[i][k].parameters())
+        self._adopt(online, targets)
 
-    def import_optimizer_state(self, actor_optimizers, critic_optimizers) -> None:  # type: ignore[override]
-        a_step = c_step = 0
-        for opts, is_actor in ((actor_optimizers, True), (critic_optimizers, False)):
-            for opt in opts:
-                group = opt.param_groups[0]
-                self.betas, self.eps = (float(group["betas"][0]), float(group["betas"][1])), float(group["eps"])
-                for p in group["params"]:
-                    st = opt.state.get(p)
-                    if st and id(p) in self._moments:
-                        m, v = self._moments[id(p)]
-                        m.copy_(st["exp_avg"])
-                        v.copy_(st["exp_avg_sq"])
-                        if is_actor:
-                            a_step = max(a_step, int(float(st["step"])))
-                        else:
-                            c_step = max(c_step, int(float(st["step"])))
-        self.actor_step, self.critic_step = a_step, c_step
+    def import_optimizer_state(self, actor_optimizers, critic_optimizers) -> None:
+        self.actor_step = max([self._import_adam(opt) for opt in actor_optimizers], default=0)
+        self.critic_step = max([self._import_adam(opt) for opt in critic_optimizers], default=0)
 
-    def export_optimizer_state(self, actor_optimizers, critic_optimizers) -> None:  # type: ignore[override]
-        torch = self._torch
-        for opts, step in ((actor_optimizers, self.actor_step), (critic_optimizers, self.critic_step)):
-            if step == 0:
-                continue
-            for opt in opts:
-                for p in opt.param_groups[0]["params"]:
-                    if id(p) in self._moments:
-                        m, v = self._moments[id(p)]
-                        opt.state[p] = {"step": torch.tensor(float(step)), "exp_avg": m, "exp_avg_sq": v}
+    def export_optimizer_state(self, actor_optimizers, critic_optimizers) -> None:
+        for opt in actor_optimizers:
+            self._export_adam(opt, self.actor_step)
+        for opt in critic_optimizers:
+            self._export_adam(opt, self.critic_step)
 
 
 def _ma_arch(policy):
@@ -505,11 +335,11 @@ def _ma_arch(policy):
 
 def multiagent_update_unsupported(model) -> Optional[str]:
     import torch.nn as nn
-    import torch.optim as optim
 
     pol = model.policy
-    if tuple(model.observation_space.shape or ()) != (4,) or tuple(model.action_space.shape or ()) != (2,):
-        return f"spaces {model.observation_space.shape} -> {model.action_space.shape} are not the CSTR's (4,) -> (2,)"
+    why = _spaces_reason(model)
+    if why:
+        return why
     if model.n_agents != 2 or [list(s) for s in model.observation_splits] != [[0, 1], [2, 3]] or [list(s) for s in model.action_splits] != [[0], [1]]:
         return "agents are not the two reactors (observation_splits [[0,1],[2,3]], action_splits [[0],[1]])"
     if getattr(pol, "activation_fn", nn.ReLU) is not nn.ReLU:
@@ -519,10 +349,9 @@ def multiagent_update_unsupported(model) -> Optional[str]:
         return "actors / critics are not two-hidden-layer ReLU MLPs of one common width pair (multiples of 4) with inputs 2 and 3 or 6"
     if not 1 <= pol.critic.n_critics <= 2:
         return f"n_critics={pol.critic.n_critics}"
-    for opt in list(pol.actor.optimizer_list) + list(pol.critic.optimizer_list):
-        g = opt.param_groups[0]
-        if type(opt) is not optim.Adam or g.get("weight_decay", 0) or g.get("amsgrad", False) or g.get("maximize", False):
-            return f"optimizer {type(opt).__name__} is not plain Adam"
+    opt = _not_plain_adam(list(pol.actor.optimizer_list) + list(pol.critic.optimizer_list))
+    if opt is not None:
+        return f"optimizer {type(opt).__name__} is not plain Adam"
     for i in range(2):
         if sum(1 for _ in pol.actor.features_extractor_list[i].parameters()):
             return "features extractors with parameters"
