@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define CSTR_B200_ABI_VERSION 17
+#define CSTR_B200_ABI_VERSION 18
 
 #define CSTR_EINVAL (-1)   /* bad argument (null pointer, negative size, unknown mode) */
 #define CSTR_EALIGN (-2)   /* pointer not aligned for the vectorised access the layout implies */
@@ -291,7 +291,19 @@ typedef struct cstr_sac_config {
     int32_t local_step;   /* which gradient step of the current SAC.train() call this is, 1-based: the reference's target sync tests the LOOP
                              index (`gradient_step % target_update_interval == 0`, core/sac/sac.py:284), which restarts at 0 on every
                              train() call.  0 = unknown: fall back to the global counter ((n_updates - 1) % interval)              */
+    int32_t sde;          /* 1 = gSDE actor (use_sde=True, full_std, no expln), see below; 0 = the squashed Gaussian above            */
+    float clip_mean;      /* gSDE: Hardtanh bound of the mean (<= 0: no Hardtanh)                                                   */
+    uint64_t sde_seed;    /* gSDE: Philox key of the exploration eps, NOT keyed by the data-parallel rank (every rank draws one E)  */
 } cstr_sac_config;
+/* gSDE mode (sde = 1; core/sac/policies.py, core/common/distributions.py StateDependentNoiseDistribution with learn_features=True):
+ * the actor's (4, h2) head slot holds [mu.weight (2,h2) | log_std (h2,2) row-major] and its 4-float bias slot [mu.bias (2) | 0 0]
+ * (gradient 0 written to the pad); the layout, the Adam and the data-parallel ranges are unchanged.  Each update draws ONE exploration
+ * matrix E = exp(log_std) * eps (reset_noise() with batch size 1 at the top of the loop body), eps (h2,2) from Philox (key sde_seed,
+ * counter (k, n_updates), stream 10; in graph mode the update index comes from the device counters) or, for parity tests, from eps_pi
+ * given as (h2,2) standard normals (eps_next must then be NULL).  mean = Hardtanh(mu(latent)), sigma = sqrt(latent^2 @ std^2 + 1e-6),
+ * a = tanh(mean + latent @ E) for actions_pi and next_actions, log_prob = sum_j Normal(mean_j, sigma_j).log_prob(g_j) - sum_j log(1 -
+ * tanh(g_j)^2 + 1e-6) with g = atanh(clamp(a, -1 + eps32, 1 - eps32)) (zero gradient where the clamp binds).  The actor loss reaches
+ * log_std through sigma and through E.                                                                                            */
 
 int64_t cstr_sac_param_count(int32_t h1, int32_t h2);
 int cstr_sac_layout(int32_t h1, int32_t h2, int64_t *offsets /* 20 */);
@@ -375,23 +387,37 @@ int cstr_ma_update(const cstr_ma_config *cfg, const cstr_td3_state *state, const
  *   actor_mode 0: fp32 CUDA-core actor (parity path)
  *   actor_mode 1: bf16 tcgen05 tensor-core hidden layer, fp32 accumulate (throughput path);
  *                 needs the packed weights from cstr_actor_pack_bf16.
- * noise: TANH actors add sigma * N(0,1) exploration noise (NormalActionNoise) — from Philox (stream "noise") when
+ * noise: TANH and SDE actors add sigma * N(0,1) exploration noise (NormalActionNoise) — from Philox (stream "noise") when
  * noise == NULL, else the (K,n,2) tensor is added as is.  GAUSSIAN actors use the same source as their eps ~ N(0,1)
  * (noise tensor = eps itself; sigma is ignored).
+ * SDE actors (gSDE, use_sde=True) run on actor_mode 0 only and have no VecNormalize variant: both return CSTR_EINVAL.
  * warmup != 0: uniform random actions instead of the actor (learning_starts phase, :386-388).
  * Each step writes ring row (pos0 + k) % rows of the replay records and leaves `state` at the
  * observation to act on next.  rows = ring capacity in rows.                                       */
 #define CSTR_ACTOR_TANH 0     /* TD3/DDPG actor: a = tanh(head)            core/td3/policies.py:75-78          */
 #define CSTR_ACTOR_GAUSSIAN 1 /* SAC actor: a = tanh(mu + exp(clamp(log_std,-20,2)) * eps), eps ~ N(0,1)
                                  core/sac/policies.py:151-168, core/common/distributions.py:207-260           */
+#define CSTR_ACTOR_SDE 2      /* SAC actor with gSDE: latent = relu(W2 relu(W1 x + b1) + b2), mean = hardtanh(W3 latent + b3, clip_mean),
+                                 a = tanh(mean + latent @ explore[i]) with reactor i's (H2,2) exploration matrix
+                                 (StateDependentNoiseDistribution, learn_features=True, full_std=True, use_expln=False)          */
 typedef struct cstr_actor_f32 {
     const float *W1, *b1; /* (H1,4), (H1) */
     const float *W2, *b2; /* (H2,H1), (H2) */
-    const float *W3, *b3; /* TANH: (2,H2), (2).  GAUSSIAN: (4,H2), (4) = rows [mu_0, mu_1, log_std_0, log_std_1] */
+    const float *W3, *b3; /* TANH, SDE: (2,H2), (2).  GAUSSIAN: (4,H2), (4) = rows [mu_0, mu_1, log_std_0, log_std_1] */
     int32_t H1, H2;
-    int32_t kind;         /* CSTR_ACTOR_TANH | CSTR_ACTOR_GAUSSIAN */
-    int32_t reserved;
+    int32_t kind;         /* CSTR_ACTOR_TANH | CSTR_ACTOR_GAUSSIAN | CSTR_ACTOR_SDE */
+    float clip_mean;      /* SDE: the Hardtanh bound of mean (<= 0: no Hardtanh); 0 for the other kinds */
+    const float *explore; /* SDE: (n,H2,2) per-reactor exploration matrices, std folded in (cstr_sde_sample), 8-byte aligned, row i =
+                             local reactor i of this call; NULL for the other kinds */
 } cstr_actor_f32;
+
+/* gSDE exploration matrices for the SDE actor (StateDependentNoiseDistribution.sample_weights, core/common/distributions.py):
+ * explore[i] = exp(log_std) * eps_i for the n reactors of this shard, eps_i (H2,2) standard normals from Philox keyed on
+ * (seed, global reactor id env_offset + i, epoch) on the "sde" stream, so a row does not depend on how the reactors are sharded.
+ * log_std: (H2,2) row-major; explore: (n,H2,2), 16-byte aligned.  The caller draws once per reset_noise() and passes a new epoch
+ * each time; the rollout reads the stored matrices (at H2 = 256 they are 2 KiB per reactor).                                  */
+int cstr_sde_sample(const float *log_std, int32_t h2, int64_t n, int64_t env_offset, uint64_t seed, uint32_t epoch, float *explore,
+                    void *stream);
 
 /* Monitor-style episode accounting for the fused rollout (core/common/monitor.py:85-111, the feed of
  * ep_info_buffer, core/common/base_class.py:462-481), all on the device: ep_return (n,) double is the running return of

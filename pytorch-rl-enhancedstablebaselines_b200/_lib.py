@@ -9,11 +9,11 @@ from typing import Optional
 
 from . import _build
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 MATH_STRICT, MATH_FAST = 0, 1
 INIT_RANDOM, INIT_STATIC = 0, 1
 REC_FLOATS = 16
-ACTOR_TANH, ACTOR_GAUSSIAN = 0, 1
+ACTOR_TANH, ACTOR_GAUSSIAN, ACTOR_SDE = 0, 1, 2
 
 
 class CstrLibraryError(RuntimeError):
@@ -40,7 +40,8 @@ class ActorF32(Structure):
         ("W2", c_void_p), ("b2", c_void_p),
         ("W3", c_void_p), ("b3", c_void_p),
         ("H1", c_int32), ("H2", c_int32),
-        ("kind", c_int32), ("reserved", c_int32),
+        ("kind", c_int32), ("clip_mean", c_float),
+        ("explore", c_void_p),
     ]
 
 
@@ -93,7 +94,7 @@ class SacConfig(Structure):
 
     _fields_ = [("h1", c_int32), ("h2", c_int32), ("batch", c_int32), ("target_update_interval", c_int32), ("gamma", c_float), ("tau", c_float),
                 ("lr", c_float), ("beta1", c_float), ("beta2", c_float), ("eps", c_float), ("target_entropy", c_float), ("reserved0", c_float),
-                ("seed", c_uint64), ("gemm_mode", c_int32), ("local_step", c_int32)]
+                ("seed", c_uint64), ("gemm_mode", c_int32), ("local_step", c_int32), ("sde", c_int32), ("clip_mean", c_float), ("sde_seed", c_uint64)]
 
 
 class BcqConfig(Structure):
@@ -164,6 +165,7 @@ _SIGNATURES = {
     "cstr_rollout_fused_multi": (c_int, [POINTER(EnvParams), c_int64, c_int64, c_int, P, c_int, c_uint32, P, P, P, P, c_int64, c_int64, P, P,
                                          POINTER(EpisodeStatsStruct), P]),
     "cstr_actor_pack_bf16": (c_int64, [POINTER(ActorF32), P, P]),
+    "cstr_sde_sample": (c_int, [P, c_int32, c_int64, c_int64, c_uint64, c_uint32, P, P]),
     "cstr_probe_pipe": (c_int, [c_int, c_int64, c_int, c_int, P, P]),
     "cstr_selftest": (c_int, [c_int, P, P]),
 }

@@ -31,15 +31,20 @@ constexpr int ROLL_THREADS = ROLL_PARTS * 32;
 
 // NORM (cstr_rollout_fused_norm, K == 1): the actor reads the normalised observation, done rows keep their raw terminal observation until
 // the statistics that include this step exist, and the CTA's moment sums go to norm_merge.
+// KIND == CSTR_ACTOR_SDE (gSDE): the layer-2 epilogue also accumulates noise = latent @ explore[i] into partial heads 2 and 3, each lane
+// reading its own reactors' (H2,2) matrices (row i of `explore`); the head is then tanh(hardtanh(mu) + noise) plus the additive noise
+// of the TANH kind.
 template <int MODE, int KIND, bool NORM>
 __global__ void __launch_bounds__(ROLL_THREADS, 1)
-rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor_a, cstr_actor_f32 actor_b, int n_agents, float sigma,
+rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, ActorNet actor_a, ActorNet actor_b, int n_agents, float sigma,
                    const float2 *__restrict__ noise, int warmup,
                    uint32_t t_base, float4 *__restrict__ state, int32_t *__restrict__ step_count, int32_t *__restrict__ episode,
                    double *static_base, int64_t rows, int64_t pos0, float4 *__restrict__ records, double *reward_sum, cstr_episode_stats stats,
-                   int has_stats, NormLaunch nl) {
+                   int has_stats, NormLaunch nl, const float2 *__restrict__ explore) {
     extern __shared__ float h1[];  // [H1][ROLL_M] (reused for the partial heads [PARTS][4][ROLL_M] once layer 2 is done), then the state column
-    constexpr int NOUT = KIND == CSTR_ACTOR_GAUSSIAN ? 4 : 2;
+    constexpr bool SDE = KIND == CSTR_ACTOR_SDE;
+    constexpr int NOUT = KIND == CSTR_ACTOR_GAUSSIAN ? 4 : 2;  // rows of W3
+    constexpr int NPART = SDE ? 4 : NOUT;                      // partial heads per warp: [mu_0, mu_1, noise_0, noise_1] for SDE
     const int lane = threadIdx.x & 31, part = threadIdx.x >> 5;
     const bool owner = part < ROLL_M / 32;  // warps 0..3 own one reactor per lane: state registers, head, env step, record
     const int m = part * 32 + lane;         // the owned reactor (owners only)
@@ -81,7 +86,7 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
         } else {
           float mu_agent[2] = {0.f, 0.f};
           for (int agent = 0; agent < n_agents; ++agent) {
-            const cstr_actor_f32 &actor = agent ? actor_b : actor_a;
+            const ActorNet &actor = agent ? actor_b : actor_a;
             if constexpr (NORM) {
                 if (owner) s_state[m] = nl.norm_obs ? norm_obs4(s, nl) : s;
             } else {
@@ -156,6 +161,16 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
 #pragma unroll
                             for (int r = 0; r < ROLL_R; ++r) o[r][c] = fmaf(w3, fmaxf(acc[q][r] + b2, 0.0f), o[r][c]);
                         }
+                        if constexpr (SDE) {
+#pragma unroll
+                            for (int r = 0; r < ROLL_R; ++r) {  // past-the-end reactors read the last one's matrix; their heads are discarded
+                                const int64_t ir = min((int64_t)blockIdx.x * ROLL_M + lane + 32 * r, n - 1);
+                                const float2 e = __ldg(explore + (size_t)ir * H2 + nb + q);
+                                const float lat = fmaxf(acc[q][r] + b2, 0.0f);
+                                o[r][2] = fmaf(lat, e.x, o[r][2]);
+                                o[r][3] = fmaf(lat, e.y, o[r][3]);
+                            }
+                        }
                     }
                 }
             }
@@ -163,7 +178,7 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
 #pragma unroll
             for (int r = 0; r < ROLL_R; ++r)
 #pragma unroll
-                for (int c = 0; c < NOUT; ++c) s_o[(part * 4 + c) * ROLL_M + lane + 32 * r] = o[r][c];
+                for (int c = 0; c < NPART; ++c) s_o[(part * 4 + c) * ROLL_M + lane + 32 * r] = o[r][c];
             __syncthreads();
             if (owner) {
                 float oo[4] = {0.f, 0.f, 0.f, 0.f};
@@ -174,6 +189,16 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
                     for (int q = 0; q < ROLL_PARTS; ++q) v += s_o[(q * 4 + c) * ROLL_M + m];
                     oo[c] = v;
                 }
+                if constexpr (SDE) {  // get_actions: tanh(mean + latent @ E), mean = Hardtanh(mu) when clip_mean > 0 (sac/policies.py)
+                    float nse[2] = {0.f, 0.f};
+#pragma unroll
+                    for (int c = 0; c < 2; ++c)
+#pragma unroll
+                        for (int q = 0; q < ROLL_PARTS; ++q) nse[c] += s_o[(q * 4 + 2 + c) * ROLL_M + m];
+                    const float cm = actor.clip_mean;
+#pragma unroll
+                    for (int c = 0; c < 2; ++c) oo[c] = __fadd_rn(cm > 0.0f ? fminf(fmaxf(oo[c], -cm), cm) : oo[c], nse[c]);
+                }
                 float2 nz;
                 if (noise) nz = live ? noise[k * n + i] : make_float2(0.f, 0.f);
                 else if (KIND == CSTR_ACTOR_GAUSSIAN) nz = philox_normal2(p.seed, env, g);
@@ -181,7 +206,7 @@ rollout_f32_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor
                 else nz = make_float2(0.f, 0.f);
                 float mu0, mu1;
                 float2 add;
-                actor_head<KIND>(oo, nz, mu0, mu1, add);
+                actor_head<SDE ? CSTR_ACTOR_TANH : KIND>(oo, nz, mu0, mu1, add);
                 if (n_agents == 1) {
                     action_maps(mu0, add.x, env_a.x, buf_a.x);
                     action_maps(mu1, add.y, env_a.y, buf_a.y);
@@ -297,7 +322,13 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
         if (!actor || !actor->W1 || !actor->b1 || !actor->W2 || !actor->b2 || !actor->W3 || !actor->b3)
             return fail_arg(CSTR_EINVAL, "rollout: actor weights missing");
         if (actor->H1 <= 0 || actor->H2 <= 0 || (actor->H1 & 3)) return fail_arg(CSTR_EINVAL, "rollout: H1 must be a positive multiple of 4");
-        if (actor->kind != CSTR_ACTOR_TANH && actor->kind != CSTR_ACTOR_GAUSSIAN) return fail_arg(CSTR_EINVAL, "rollout: unknown actor kind");
+        if (actor->kind != CSTR_ACTOR_TANH && actor->kind != CSTR_ACTOR_GAUSSIAN && actor->kind != CSTR_ACTOR_SDE)
+            return fail_arg(CSTR_EINVAL, "rollout: unknown actor kind");
+        if (actor->kind == CSTR_ACTOR_SDE) {
+            if (actor_mode != 0 || nl) return fail_arg(CSTR_EINVAL, "rollout: the gSDE actor runs on the fp32 kernel (actor_mode 0) without VecNormalize");
+            if (!actor->explore) return fail_arg(CSTR_EINVAL, "rollout: the gSDE actor needs its exploration matrices (cstr_sde_sample)");
+            if (!aligned(actor->explore, 8)) return fail_arg(CSTR_EALIGN, "rollout: explore 8 B alignment");
+        }
         if (!aligned(actor->W1, 16) || !aligned(actor->W2, 16)) return fail_arg(CSTR_EALIGN, "rollout: W1/W2 16 B alignment");
     }
     if (stats && (!stats->ep_return || !stats->finished || !stats->count)) return fail_arg(CSTR_EINVAL, "rollout: episode stats pointers missing");
@@ -310,9 +341,9 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
         return cstr_rollout_tc_launch(p, n, K, math_mode, actor, packed_bf16, sigma, noise, warmup, t_base, state, step_count, episode,
                                       static_base, rows, pos0, records, reward_sum, stats, nl, stream);
     if (actor_mode != 0 && actor_mode != 1) return fail_arg(CSTR_EINVAL, "rollout: unknown actor_mode");
-    cstr_actor_f32 a = {}, b2nd = {};
-    if (actor) a = *actor;
-    if (actor_b) b2nd = *actor_b;
+    ActorNet a = {}, b2nd = {};
+    if (actor) a = actor_net(*actor);
+    if (actor_b) b2nd = actor_net(*actor_b);
     const int n_agents = actor_b ? 2 : 1;
     const size_t h1_floats = (size_t)a.H1 * ROLL_M > (size_t)ROLL_PARTS * 4 * ROLL_M ? (size_t)a.H1 * ROLL_M : (size_t)ROLL_PARTS * 4 * ROLL_M;
     size_t smem = warmup ? 0 : h1_floats * sizeof(float) + ROLL_M * sizeof(float4);
@@ -326,7 +357,8 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
         rc = check_cuda(cudaFuncSetAttribute(rollout_f32_kernel<MODE, KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "smem attr"); \
         if (!rc)                                                                                                                           \
             rollout_f32_kernel<MODE, KIND, false><<<grid, ROLL_THREADS, smem, st>>>(*p, n, K, a, b2nd, n_agents, sigma, (const float2 *)noise, warmup, t_base, (float4 *)state, \
-                                                                       step_count, episode, static_base, rows, pos0, (float4 *)records, reward_sum, st_copy, has_stats, NormLaunch{}); \
+                                                                       step_count, episode, static_base, rows, pos0, (float4 *)records, reward_sum, st_copy, has_stats, NormLaunch{},    \
+                                                                       (const float2 *)(KIND == CSTR_ACTOR_SDE ? actor->explore : nullptr)); \
     } while (0)
     cstr_episode_stats st_copy = {};
     const int has_stats = stats != nullptr;
@@ -339,10 +371,13 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
         if (!rc)                                                                                                                           \
             rollout_f32_kernel<MODE, KIND, true><<<grid, ROLL_THREADS, smem, st>>>(*p, n, K, a, b2nd, n_agents, sigma, (const float2 *)noise, warmup,     \
                                                                             t_base, (float4 *)state, step_count, episode, static_base, rows, pos0,  \
-                                                                            (float4 *)records, reward_sum, st_copy, has_stats, *nl);               \
+                                                                            (float4 *)records, reward_sum, st_copy, has_stats, *nl, nullptr);      \
     } while (0)
     const bool gauss = a.kind == CSTR_ACTOR_GAUSSIAN;
-    if (nl) {
+    if (!warmup && a.kind == CSTR_ACTOR_SDE) {
+        if (math_mode == CSTR_MATH_STRICT) CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_SDE);
+        else CSTR_LAUNCH_ROLL(CSTR_MATH_FAST, CSTR_ACTOR_SDE);
+    } else if (nl) {
         if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
         else { if (gauss) CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_FAST, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL_NORM(CSTR_MATH_FAST, CSTR_ACTOR_TANH); }
     } else if (math_mode == CSTR_MATH_STRICT) { if (gauss) CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_GAUSSIAN); else CSTR_LAUNCH_ROLL(CSTR_MATH_STRICT, CSTR_ACTOR_TANH); }
@@ -351,6 +386,45 @@ static int rollout_fused_impl(const cstr_env_params *p, int64_t n, int64_t K, in
 #undef CSTR_LAUNCH_ROLL_NORM
     if (rc) return rc;
     return check_launch("rollout_f32_kernel");
+}
+
+// gSDE exploration matrices: thread t of reactor i writes explore[i][4t .. 4t+3] = exp(log_std[4t .. 4t+3]) * N(0,1) from one Philox
+// call on counter (global id, epoch, "sde" stream | t): the Box-Muller pair of philox_normal4 in cstr_mlp.cuh
+constexpr uint32_t STREAM_SDE = 11u;
+__global__ void __launch_bounds__(256) sde_sample_kernel(const float *__restrict__ log_std, int h2, int64_t n, int64_t env_offset, uint64_t seed,
+                                                          uint32_t epoch, float *__restrict__ explore) {
+    const int per = (2 * h2 + 3) / 4;  // Philox calls per reactor (the last one is half used when h2 is odd)
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n * per) return;
+    const int64_t i = idx / per;
+    const uint32_t t = (uint32_t)(idx - i * per);
+    const uint64_t env = (uint64_t)(env_offset + i);
+    // the call index takes the low byte of the counter's last word (as for the other streams) and, past 255, its top 16 bits
+    const uint4 r = philox4x32_10(make_uint4((uint32_t)env, (uint32_t)(env >> 32), epoch, (STREAM_SDE << 8) | (t & 0xffu) | ((t >> 8) << 16)),
+                                  (uint32_t)seed, (uint32_t)(seed >> 32));
+    const float u1 = fmaf(u24(r.x), 1.0f, 5.9604644775390625e-08f), u2 = u24(r.y);
+    const float u3 = fmaf(u24(r.z), 1.0f, 5.9604644775390625e-08f), u4 = u24(r.w);
+    const float ra = sqrtf(-2.0f * logf(u1)), rb = sqrtf(-2.0f * logf(u3));
+    float s1, c1, s2, c2;
+    sincospif(2.0f * u2, &s1, &c1);
+    sincospif(2.0f * u4, &s2, &c2);
+    const float z[4] = {ra * c1, ra * s1, rb * c2, rb * s2};
+    const int j0 = 4 * (int)t;
+    float *out = explore + (size_t)i * 2 * h2;
+#pragma unroll
+    for (int c = 0; c < 4; ++c)
+        if (j0 + c < 2 * h2) out[j0 + c] = __fmul_rn(expf(log_std[j0 + c]), z[c]);  // Normal(0, std).rsample() = 0 + eps * std
+}
+
+extern "C" int cstr_sde_sample(const float *log_std, int32_t h2, int64_t n, int64_t env_offset, uint64_t seed, uint32_t epoch, float *explore,
+                               void *stream) {
+    if (!log_std || !explore || h2 <= 0 || n < 0 || env_offset < 0) return fail_arg(CSTR_EINVAL, "sde_sample: null pointer or bad size");
+    if (h2 > (1 << 23)) return fail_arg(CSTR_EINVAL, "sde_sample: h2 too large");
+    if (!aligned(explore, 16)) return fail_arg(CSTR_EALIGN, "sde_sample: explore 16 B alignment");
+    if (n == 0) return 0;
+    const int64_t threads = n * ((2 * (int64_t)h2 + 3) / 4);
+    sde_sample_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(log_std, h2, n, env_offset, seed, epoch, explore);
+    return check_launch("sde_sample_kernel");
 }
 
 // workspace of cstr_rollout_fused_norm: [ticket (16 B)][partials: grid x NORM_SUMS doubles][pending: n bytes]; both kernels use 128-reactor CTAs

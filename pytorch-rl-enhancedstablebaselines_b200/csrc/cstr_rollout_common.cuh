@@ -30,6 +30,15 @@ __device__ __forceinline__ float2 philox_normal2(uint64_t seed, uint64_t env, ui
     return make_float2(rad * cs, rad * sn);
 }
 
+// The kernels' by-value copy of cstr_actor_f32 without its explore pointer: the gSDE instances take that pointer as a parameter of their
+// own, after all the others, so the parameters of the other instances keep their place in the constant bank (and their SASS).
+struct ActorNet {
+    const float *W1, *b1, *W2, *b2, *W3, *b3;
+    int32_t H1, H2, kind;
+    float clip_mean;
+};
+inline ActorNet actor_net(const cstr_actor_f32 &a) { return ActorNet{a.W1, a.b1, a.W2, a.b2, a.W3, a.b3, a.H1, a.H2, a.kind, a.clip_mean}; }
+
 // Actor head -> squashed action in [-1,1] and the additive exploration noise that follows it.
 //   TANH (TD3):      a = tanh(o[0..1]);  noise = sigma*N(0,1) (or the caller's tensor)        td3/policies.py:75-78, noise.py:29-48
 //   GAUSSIAN (SAC):  a = tanh(mu + exp(clamp(log_std,-20,2))*eps), no additive noise          sac/policies.py:151-168

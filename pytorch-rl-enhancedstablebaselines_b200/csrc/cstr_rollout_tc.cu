@@ -181,7 +181,7 @@ enum { BAR_W_FULL = 0, BAR_W_EMPTY = 3, BAR_A_FULL = 6, BAR_A_EMPTY = 8, BAR_D_F
 // the statistics that include this step exist, and the CTA's moment sums go to norm_merge.
 template <int MODE, int KIND, bool NORM>
 __global__ void __launch_bounds__(TC_THREADS, 1)
-rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, cstr_actor_f32 actor, const uint8_t *__restrict__ packed_w2, TcGeometry g,
+rollout_tc_kernel(cstr_env_params p, int64_t n, int64_t K, ActorNet actor, const uint8_t *__restrict__ packed_w2, TcGeometry g,
                   float sigma, const float2 *__restrict__ noise, uint32_t t_base, float4 *__restrict__ state,
                   int32_t *__restrict__ step_count, int32_t *__restrict__ episode, double *static_base, int64_t rows, int64_t pos0,
                   float4 *__restrict__ records, double *reward_sum, cstr_episode_stats stats, int has_stats, NormLaunch nl) {
@@ -576,7 +576,7 @@ int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int m
     do {                                                                                                                                    \
         rc = check_cuda(cudaFuncSetAttribute(rollout_tc_kernel<MODE, KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_bytes), "smem attr"); \
         if (!rc)                                                                                                                            \
-            rollout_tc_kernel<MODE, KIND, false><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, *actor, (const uint8_t *)packed_bf16, g, sigma, (const float2 *)noise, \
+            rollout_tc_kernel<MODE, KIND, false><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, net, (const uint8_t *)packed_bf16, g, sigma, (const float2 *)noise, \
                                                                                   t_base, (float4 *)state, step_count, episode, static_base, rows, pos0,   \
                                                                                   (float4 *)records, reward_sum, st_copy, has_stats, NormLaunch{}); \
     } while (0)
@@ -587,11 +587,12 @@ int cstr_rollout_tc_launch(const cstr_env_params *p, int64_t n, int64_t K, int m
     do {                                                                                                                                    \
         rc = check_cuda(cudaFuncSetAttribute(rollout_tc_kernel<MODE, KIND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem_bytes), "smem attr"); \
         if (!rc)                                                                                                                            \
-            rollout_tc_kernel<MODE, KIND, true><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, *actor, (const uint8_t *)packed_bf16, g, sigma,         \
+            rollout_tc_kernel<MODE, KIND, true><<<grid, TC_THREADS, g.smem_bytes, st>>>(*p, n, K, net, (const uint8_t *)packed_bf16, g, sigma,         \
                                                                                        (const float2 *)noise, t_base, (float4 *)state, step_count,   \
                                                                                        episode, static_base, rows, pos0, (float4 *)records,          \
                                                                                        reward_sum, st_copy, has_stats, *nl);                         \
     } while (0)
+    const ActorNet net = actor_net(*actor);
     const bool gauss = actor->kind == CSTR_ACTOR_GAUSSIAN;
     if (nl) {
         if (K != 1) return fail_arg(CSTR_EINVAL, "rollout(tc): the VecNormalize variant runs one step per launch");

@@ -643,6 +643,191 @@ sac_actor_bwd_head_kernel(int B, int H1, int H2, const float *__restrict__ dz1c,
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// SAC with gSDE (use_sde=True: StateDependentNoiseDistribution, learn_features=True, full_std=True, use_expln=False; core/sac/policies.py,
+// core/common/distributions.py).  The actor head slot holds [mu.weight (2,H2) | log_std (H2,2)], the bias slot [mu.bias (2) | 0 0].
+// One exploration matrix E = exp(log_std) * eps (H2,2) per update (reset_noise() with batch size 1 at the top of sac.py's loop) serves
+// every row of actions_pi, next_actions and the actor loss; it is an rsample, so the loss reaches log_std through E as well.
+// ------------------------------------------------------------------------------------------------------------------
+constexpr uint32_t STREAM_SAC_SDE = 10u;
+constexpr float SDE_VAR_EPS = 1e-6f, SDE_ATANH_EPS = 1.1920928955078125e-07f;  // proba_distribution's variance epsilon; finfo(float32).eps
+
+// sde[0 : 2H2] = E, sde[2H2 : 4H2] = std^2, with std = exp(log_std); eps from eps_in (H2,2) or Philox (key seed = the UN-rank-keyed seed,
+// counter (k, update index), stream 10): every data-parallel rank draws the same E
+__global__ void __launch_bounds__(256)
+sac_sde_draw_kernel(int H2, const float *__restrict__ log_std, const float2 *__restrict__ eps_in, uint64_t seed, uint32_t update_index,
+                    const float *__restrict__ dev_scalars, float *__restrict__ sde) {
+    pdl_enter();
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= H2) return;
+    float2 e;
+    if (eps_in) e = eps_in[k];
+    else {
+        const uint32_t ui = dev_scalars ? __float_as_uint(dev_scalars[4]) : update_index;
+        const uint4 r = philox_env(seed, (uint64_t)k, ui, STREAM_SAC_SDE, 0);
+        const float u1 = fmaf(u24(r.x), 1.0f, 5.9604644775390625e-08f), u2 = u24(r.y);
+        const float rad = sqrtf(-2.0f * logf(u1));
+        float sn, cs;
+        sincospif(2.0f * u2, &sn, &cs);
+        e = make_float2(rad * cs, rad * sn);
+    }
+    const float s0 = expf(log_std[2 * k]), s1 = expf(log_std[2 * k + 1]);
+    sde[2 * k] = s0 * e.x, sde[2 * k + 1] = s1 * e.y;
+    sde[2 * H2 + 2 * k] = s0 * s0, sde[2 * H2 + 2 * k + 1] = s1 * s1;
+}
+
+// log_prob of the gSDE distribution at the squashed action a (distributions.py log_prob: the tanh is INVERTED, g = atanh(clamp(a)))
+__device__ __forceinline__ float sde_gauss_arg(float a) {
+    const float y = fminf(fmaxf(a, -1.f + SDE_ATANH_EPS), 1.f - SDE_ATANH_EPS);
+    return 0.5f * (log1pf(y) - log1pf(-y));
+}
+
+// per row: mu_raw = h2 @ Wmu^T + b, mean = hardtanh(mu_raw), var = h2^2 @ std^2, sigma = sqrt(var + 1e-6), noise = h2 @ E,
+// a = tanh(mean + noise), log_prob = sum_j Normal(mean_j, sigma_j).log_prob(g_j) - sum_j log(1 - tanh(g_j)^2 + 1e-6)
+__global__ void __launch_bounds__(256)
+sac_sde_head_kernel(int B, int H2, const float *__restrict__ h2, const float *__restrict__ W3, const float *__restrict__ b3, const float *__restrict__ sde,
+                    float clip_mean, float2 *__restrict__ act_out, float *__restrict__ logp_out, float2 *__restrict__ mu_raw_out,
+                    float2 *__restrict__ sigma_out, float *__restrict__ lp_partial) {
+    pdl_enter();
+    __shared__ float sl[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, b = blockIdx.x * 8 + warp;
+    float lp = 0.f;
+    if (b < B) {
+        const float *h = h2 + (int64_t)b * H2;
+        const float m0 = row_dot(h, W3, H2, lane) + b3[0], m1 = row_dot(h, W3 + H2, H2, lane) + b3[1];
+        const float2 *E = reinterpret_cast<const float2 *>(sde), *S2 = E + H2;
+        float n0 = 0.f, n1 = 0.f, v0 = 0.f, v1 = 0.f;
+        for (int k = lane; k < H2; k += 32) {
+            const float x = h[k], x2 = x * x;
+            const float2 e = E[k], s2 = S2[k];
+            n0 = fmaf(x, e.x, n0), n1 = fmaf(x, e.y, n1), v0 = fmaf(x2, s2.x, v0), v1 = fmaf(x2, s2.y, v1);
+        }
+        n0 = warp_sum(n0), n1 = warp_sum(n1), v0 = warp_sum(v0), v1 = warp_sum(v1);
+        if (lane == 0) {
+            const float mr[2] = {m0, m1}, nz[2] = {n0, n1}, vr[2] = {v0, v1};
+            float a[2], sg[2];
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                const float mean = clip_mean > 0.f ? fminf(fmaxf(mr[i], -clip_mean), clip_mean) : mr[i];
+                sg[i] = sqrtf(vr[i] + SDE_VAR_EPS);
+                a[i] = tanhf(mean + nz[i]);
+                const float g = sde_gauss_arg(a[i]), d = g - mean, t = tanhf(g);
+                lp += -(d * d) / (2.f * sg[i] * sg[i]) - logf(sg[i]) - SAC_HALF_LOG_2PI - logf(1.f - t * t + SAC_SQUASH_EPS);
+            }
+            act_out[b] = make_float2(a[0], a[1]);
+            logp_out[b] = lp;
+            if (mu_raw_out) mu_raw_out[b] = make_float2(m0, m1);
+            if (sigma_out) sigma_out[b] = make_float2(sg[0], sg[1]);
+        }
+    }
+    if (lp_partial) {
+        if (lane == 0) sl[warp] = lp;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            float t = 0.f;
+            for (int i = 0; i < 8; ++i) t += sl[i];
+            lp_partial[blockIdx.x] = t;
+        }
+    }
+}
+
+// actor-loss backward through the gSDE head, per row (c = ent_coef / B, s = dL/da from the critics):
+//   d = g - mean;  dlp/dg = -d/sigma^2 + 2t(1-t^2)/(1-t^2+1e-6) (t = tanh g), 0 where the atanh clamp binds;  du = s (1-a^2) + c dlp/dg
+//   dmean = du + c d/sigma^2 -> dmu_raw (0 outside the open Hardtanh interval);  dnoise = du;  dvar = c (d^2/sigma^3 - 1/sigma) / (2 sigma)
+//   dlatent = (dmu_raw @ Wmu + dnoise @ E^T + 2 h2 * (dvar @ std2^T)) * (h2 > 0)
+// Y rows: y4[b] = [dmu_raw_0, dmu_raw_1, dnoise_0, dnoise_1], y2[b] = [dvar_0, dvar_1] (for sac_sde_wgrad_kernel)
+__global__ void __launch_bounds__(256)
+sac_sde_bwd_head_kernel(int B, int H1, int H2, const float *__restrict__ dz1c, int64_t dz_z, const float *__restrict__ W1c, int64_t w_z,
+                        const float2 *__restrict__ a_pi, const float2 *__restrict__ mu_raw, const float2 *__restrict__ sigma, const float *__restrict__ scalars,
+                        const float *__restrict__ W3a, const float *__restrict__ sde, float clip_mean, const float *__restrict__ h2a,
+                        float4 *__restrict__ y4, float2 *__restrict__ y2, float *__restrict__ dz2a) {
+    pdl_enter();
+    const int lane = threadIdx.x & 31, b = blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (b >= B) return;
+    float s[2] = {0.f, 0.f};
+    for (int z = 0; z < 2; ++z) {
+        const float *d = dz1c + z * dz_z + (int64_t)b * H1, *W = W1c + z * w_z;
+        for (int j = lane; j < H1; j += 32) {
+            const float v = d[j];
+            s[0] = fmaf(v, __ldg(W + j * (OBS + ACT) + OBS), s[0]);
+            s[1] = fmaf(v, __ldg(W + j * (OBS + ACT) + OBS + 1), s[1]);
+        }
+    }
+    s[0] = warp_sum(s[0]), s[1] = warp_sum(s[1]);
+    const float2 a2 = a_pi[b], m2 = mu_raw[b], sg2 = sigma[b];
+    const float av[2] = {a2.x, a2.y}, mr[2] = {m2.x, m2.y}, sg[2] = {sg2.x, sg2.y};
+    const float c = scalars[5] / (float)B;
+    float dmu[2], dn[2], dv[2];
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {
+        const bool inside = !(clip_mean > 0.f) || (mr[i] > -clip_mean && mr[i] < clip_mean);
+        const float mean = clip_mean > 0.f ? fminf(fmaxf(mr[i], -clip_mean), clip_mean) : mr[i];
+        const float g = sde_gauss_arg(av[i]), d = g - mean, t = tanhf(g), omt = 1.f - t * t, is2 = 1.f / (sg[i] * sg[i]);
+        const bool clamped = av[i] < -1.f + SDE_ATANH_EPS || av[i] > 1.f - SDE_ATANH_EPS;
+        const float dlp_dg = clamped ? 0.f : -d * is2 + 2.f * t * omt / (omt + SAC_SQUASH_EPS);
+        const float du = s[i] * (1.f - av[i] * av[i]) + c * dlp_dg;
+        dmu[i] = inside ? du + c * d * is2 : 0.f;
+        dn[i] = du;
+        dv[i] = c * (d * d * is2 / sg[i] - 1.f / sg[i]) / (2.f * sg[i]);
+    }
+    if (lane == 0) {
+        y4[b] = make_float4(dmu[0], dmu[1], dn[0], dn[1]);
+        y2[b] = make_float2(dv[0], dv[1]);
+    }
+    const float *h = h2a + (int64_t)b * H2;
+    const float2 *E = reinterpret_cast<const float2 *>(sde), *S2 = E + H2;
+    float *o = dz2a + (int64_t)b * H2;
+    for (int k = lane; k < H2; k += 32) {
+        const float x = h[k];
+        const float2 e = E[k], s2 = S2[k];
+        float acc = fmaf(dmu[0], W3a[k], dmu[1] * W3a[H2 + k]);
+        acc = fmaf(dn[0], e.x, acc), acc = fmaf(dn[1], e.y, acc);
+        acc = fmaf(2.f * x, fmaf(dv[0], s2.x, dv[1] * s2.y), acc);
+        o[k] = x > 0.f ? acc : 0.f;
+    }
+}
+
+// head weight gradients over the batch, one CTA per 32 latent units, 8 warps interleaved over rows, fixed-order sums (deterministic):
+//   dWmu[j][k] = sum_b y4[b][j] h[b][k];  dlog_std[k][j] = E[k][j] sum_b y4[b][2+j] h[b][k] + 2 std2[k][j] sum_b y2[b][j] h[b][k]^2
+//   CTA 0 also writes the bias slot [sum_b dmu_raw_0, sum_b dmu_raw_1, 0, 0]
+__global__ void __launch_bounds__(256)
+sac_sde_wgrad_kernel(int B, int H2, const float *__restrict__ h2a, const float4 *__restrict__ y4, const float2 *__restrict__ y2, const float *__restrict__ sde,
+                     float *__restrict__ gw3, float *__restrict__ gb3) {
+    pdl_enter();
+    __shared__ float red[8][7][32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, k = blockIdx.x * 32 + lane;
+    float acc[7] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // dWmu0, dWmu1, dE0, dE1, dv0, dv1, (bias: dmu sums in lanes 0 / 1)
+    float bsum0 = 0.f, bsum1 = 0.f;
+    for (int b = warp; b < B; b += 8) {
+        const float4 y = y4[b];
+        const float2 v = y2[b];
+        if (k < H2) {
+            const float x = h2a[(int64_t)b * H2 + k], x2 = x * x;
+            acc[0] = fmaf(y.x, x, acc[0]), acc[1] = fmaf(y.y, x, acc[1]), acc[2] = fmaf(y.z, x, acc[2]), acc[3] = fmaf(y.w, x, acc[3]);
+            acc[4] = fmaf(v.x, x2, acc[4]), acc[5] = fmaf(v.y, x2, acc[5]);
+        }
+        bsum0 += y.x, bsum1 += y.y;
+    }
+    acc[6] = lane == 0 ? bsum0 : bsum1;
+#pragma unroll
+    for (int i = 0; i < 7; ++i) red[warp][i][lane] = acc[i];
+    __syncthreads();
+    if (warp != 0) return;
+    float t[7];
+#pragma unroll
+    for (int i = 0; i < 7; ++i) {
+        t[i] = 0.f;
+        for (int w = 0; w < 8; ++w) t[i] += red[w][i][lane];
+    }
+    if (k < H2) {
+        const float2 e = reinterpret_cast<const float2 *>(sde)[k], s2 = reinterpret_cast<const float2 *>(sde)[H2 + k];
+        gw3[k] = t[0], gw3[H2 + k] = t[1];
+        gw3[2 * H2 + 2 * k] = fmaf(e.x, t[2], 2.f * s2.x * t[4]);
+        gw3[2 * H2 + 2 * k + 1] = fmaf(e.y, t[3], 2.f * s2.y * t[5]);
+    }
+    if (blockIdx.x == 0 && lane < 4) gb3[lane] = lane < 2 ? t[6] : 0.f;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // skinny weight gradients:  out_w[j][i] (or [i][j]) = sum_b X[b][j] * Y[b][i],  out_b = sum_b X[b][j]  (or sum_b Y[b][i])
 //   layer 1:  X = dz1 (B,H1), Y = [obs | act]        -> dW1 (H1,in), db1 (H1)
 //   layer 2 bias: X = dz2 (B,H2), no Y               -> db2 (H2)
@@ -1113,12 +1298,13 @@ struct Workspace {  // carved out of the caller's workspace buffer (floats)
     float *a_h1, *a_h2;      // actor / actor-target activations
     float *next_act, *a_pi, *target, *dq, *dpre, *loss_partial, *scalars;
     float *logp, *next_logp, *std_eps, *raw_log_std, *dpre4, *lp_partial;  // SAC
+    float *sde;                                                            // SAC gSDE: E (H2,2), std^2 (H2,2)
     MlpScratch sc;
     int n_row_blocks;
     int64_t floats;
 };
 
-Workspace carve(float *base, int B, int H1, int H2) {
+Workspace carve(float *base, int B, int H1, int H2, bool sde = false) {
     Workspace w;
     Bump b(base);
     const int64_t bh1 = (int64_t)B * H1, bh2 = (int64_t)B * H2;
@@ -1139,6 +1325,7 @@ Workspace carve(float *base, int B, int H1, int H2) {
     w.scalars = b.take(8);
     w.logp = b.take(B), w.next_logp = b.take(B), w.std_eps = b.take(2 * (int64_t)B), w.raw_log_std = b.take(2 * (int64_t)B), w.dpre4 = b.take(4 * (int64_t)B);
     w.lp_partial = b.take(w.n_row_blocks);
+    w.sde = sde ? b.take(4 * (int64_t)H2) : nullptr;  // last, so that the other configurations keep their workspace size
     w.floats = b.o;
     return w;
 }
@@ -1248,6 +1435,8 @@ static int check_sac_cfg(const cstr_sac_config *c) {
     if (c->target_update_interval < 1) return fail_arg(CSTR_EINVAL, "sac: target_update_interval must be >= 1");
     if (c->local_step < 0) return fail_arg(CSTR_EINVAL, "sac: local_step must be >= 0 (0 = use the global update counter)");
     if (c->gemm_mode < CSTR_TD3_GEMM_FP32 || c->gemm_mode > CSTR_TD3_GEMM_BF16) return fail_arg(CSTR_EINVAL, "sac: gemm_mode must be 0, 1 or 2");
+    if (c->sde != 0 && c->sde != 1) return fail_arg(CSTR_EINVAL, "sac: sde must be 0 or 1");
+    if (!(c->clip_mean == c->clip_mean)) return fail_arg(CSTR_EINVAL, "sac: clip_mean is NaN");
     return 0;
 }
 
@@ -1268,7 +1457,7 @@ int cstr_sac_layout(int32_t h1, int32_t h2, int64_t *offsets) {
 
 int64_t cstr_sac_workspace_bytes(const cstr_sac_config *cfg) {
     if (check_sac_cfg(cfg)) return -1;
-    return carve(nullptr, cfg->batch, cfg->h1, cfg->h2).floats * (int64_t)sizeof(float);
+    return carve(nullptr, cfg->batch, cfg->h1, cfg->h2, cfg->sde != 0).floats * (int64_t)sizeof(float);
 }
 
 int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const float *obs, const float *actions, const float *next_obs,
@@ -1278,8 +1467,10 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
     if (!(phases & CSTR_TD3_ALL) || (phases & ~CSTR_TD3_ALL)) return fail_arg(CSTR_EINVAL, "sac_update: phases must be a non-empty subset of CSTR_TD3_ALL");
     if (int rc = check_update("sac", stt, cstr_sac_workspace_bytes(cfg), obs, actions, next_obs, dones, rewards, n_updates, adam_step, 0)) return rc;
     if ((eps_pi && !aligned(eps_pi, 8)) || (eps_next && !aligned(eps_next, 8))) return fail_arg(CSTR_EALIGN, "sac_update: eps_pi / eps_next need 8 B alignment");
+    if (cfg->sde && eps_next) return fail_arg(CSTR_EINVAL, "sac_update: in gSDE mode eps_pi carries the (h2,2) exploration eps and eps_next must be NULL");
+    const bool sde = cfg->sde != 0;
     const int B = cfg->batch, H1 = cfg->h1, H2 = cfg->h2;
-    Workspace w = carve(stt->workspace, B, H1, H2);
+    Workspace w = carve(stt->workspace, B, H1, H2, cfg->sde != 0);
     w.sc.tensor = cfg->gemm_mode;
     const Td3Layout T = td3_layout(H1, H2, 2 * ACT);
     cudaStream_t st = (cudaStream_t)stream;
@@ -1303,16 +1494,25 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
     if (stt->counters && (phases & CSTR_TD3_CRITIC_GRAD))
         if (int rc = launch_tick(stt, w.scalars, true, cfg->lr, cfg->beta1, cfg->beta2, -1.0, -1.0, -1.0, st)) return rc;
     if (phases & CSTR_TD3_CRITIC_GRAD) {
+    if (sde) {  // actor.reset_noise() at the top of the loop body (sac.py): one E for the whole update, the same on every rank
+        launch_k(sac_sde_draw_kernel, (unsigned)((H2 + 255) / 256), 256, 0, st, H2, (const float *)(actor.w3 + 2 * H2), (const float2 *)eps_pi, cfg->sde_seed,
+                 (uint32_t)n_updates, dev_sc, w.sde);
+        if (int rc = check_launch("sac_sde_draw_kernel")) return rc;
+    }
     // ---- actions_pi, log_prob of the current actor (sac.py:222-223) and the entropy-coefficient step (:226-243) ----
     if (int rc = forward_hidden(B, H1, H2, OBS, obs, nullptr, actor, 0, 1, w.a_h1, w.a_h2, w.sc, st)) return rc;
-    launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor.w3, actor.b3, (const float2 *)eps_pi, cfg->seed, (uint32_t)n_updates, dev_sc, 0u, (float2 *)w.a_pi,
+    if (sde) launch_k(sac_sde_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor.w3, actor.b3, w.sde, cfg->clip_mean, (float2 *)w.a_pi, w.logp,
+                      (float2 *)w.raw_log_std, (float2 *)w.std_eps, w.lp_partial);
+    else launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.a_h2, actor.w3, actor.b3, (const float2 *)eps_pi, cfg->seed, (uint32_t)n_updates, dev_sc, 0u, (float2 *)w.a_pi,
                                              w.logp, (float2 *)w.std_eps, (float2 *)w.raw_log_std, w.lp_partial);
     if (int rc = check_launch("sac_actor_head_kernel")) return rc;
     // one launch when nothing sits between gradient and step; split around the caller's all-reduce of grads[critics .. log_ent_coef] otherwise
     if (int rc = ent_coef(fused_ent ? 3 : 1)) return rc;
     // ---- target (sac.py:245-254): next action from the CURRENT actor (scratch: the dz slabs are free here) ----
     if (int rc = forward_hidden(B, H1, H2, OBS, next_obs, nullptr, actor, 0, 1, w.dz1, w.dz2, w.sc, st)) return rc;
-    launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.dz2, actor.w3, actor.b3, (const float2 *)eps_next, cfg->seed, (uint32_t)n_updates, dev_sc, 1u,
+    if (sde) launch_k(sac_sde_head_kernel, rb, 256, 0, st, B, H2, w.dz2, actor.w3, actor.b3, w.sde, cfg->clip_mean, (float2 *)w.next_act, w.next_logp,
+                      nullptr, nullptr, nullptr);
+    else launch_k(sac_actor_head_kernel, rb, 256, 0, st, B, H2, w.dz2, actor.w3, actor.b3, (const float2 *)eps_next, cfg->seed, (uint32_t)n_updates, dev_sc, 1u,
                                              (float2 *)w.next_act, w.next_logp, nullptr, nullptr, nullptr);
     if (int rc = check_launch("sac_actor_head_kernel<next>")) return rc;
     if (int rc = forward_hidden(B, H1, H2, OBS + ACT, next_obs, w.next_act, critic_t, cz, 2, w.t_h1, w.t_h2, w.sc, st)) return rc;
@@ -1341,6 +1541,16 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
     if (int rc = check_launch("sac_qmin_head_kernel")) return rc;
     if (int rc = backward_dz1(B, H1, H2, critic, cz, 2, w.h1[0], w.dz2, w.dz1, w.sc, st)) return rc;
     // the actor's dz2 / dz1 live in the target-activation slabs (free since the target was formed)
+    FinJobs J{};
+    if (sde) {
+        launch_k(sac_sde_bwd_head_kernel, rb, 256, 0, st, B, H1, H2, w.dz1, (int64_t)B * H1, critic.w1, cz, (const float2 *)w.a_pi,
+                 (const float2 *)w.raw_log_std, (const float2 *)w.std_eps, w.scalars, actor.w3, w.sde, cfg->clip_mean, w.a_h2, (float4 *)w.dpre4,
+                 (float2 *)w.dpre, w.t_h2);
+        if (int rc = check_launch("sac_sde_bwd_head_kernel")) return rc;
+        launch_k(sac_sde_wgrad_kernel, (unsigned)((H2 + 31) / 32), 256, 0, st, B, H2, w.a_h2, (const float4 *)w.dpre4, (const float2 *)w.dpre, w.sde,
+                 g_actor.w3, g_actor.b3);
+        if (int rc = check_launch("sac_sde_wgrad_kernel")) return rc;
+    } else {
     launch_k(sac_actor_bwd_head_kernel, rb, 256, 0, st, B, H1, H2, w.dz1, (int64_t)B * H1, critic.w1, cz, (const float2 *)w.a_pi, (const float2 *)w.std_eps,
                                                  (const float2 *)w.raw_log_std, w.scalars, actor.w3, w.a_h2, (float4 *)w.dpre4, w.t_h2);
     if (int rc = check_launch("sac_actor_bwd_head_kernel")) return rc;
@@ -1348,8 +1558,8 @@ int cstr_sac_update(const cstr_sac_config *cfg, const cstr_td3_state *stt, const
     s.X = w.a_h2, s.x_z = 0, s.ldx = H2, s.H = H2, s.B = B;
     s.Y0 = w.dpre4, s.n0 = 2 * ACT, s.ld0 = 2 * ACT, s.Y1 = nullptr, s.n1 = 0, s.ld1 = 0, s.y_z = 0;
     s.out_w = g_actor.w3, s.out_b = g_actor.b3, s.out_z = 0, s.transposed = 1;
-    FinJobs J{};
     if (int rc = launch_skinny<2 * ACT, true>(s, 1, w.sc.skinny + 2 * w.sc.skinny_region, st, "td3_skinny_wgrad_kernel<sac head>", J)) return rc;
+    }
     if (int rc = backward_hidden(B, H1, H2, td3_src(obs, nullptr, OBS), nullptr, actor, g_actor, 0, 1, w.a_h1, w.t_h2, w.t_h1, w.sc, J, st)) return rc;
     }  // ACTOR_GRAD
     if (phases & CSTR_TD3_ACTOR_APPLY) {

@@ -29,7 +29,7 @@ def actor_shape_error(H1: int, H2: int, actor_mode: str) -> Optional[str]:
     if H1 % 16 or H1 > 1024:
         return f"H1={H1}: the tensor-core actor needs H1 a multiple of 16 and <= 1024"
     # the size query of the W2 packer reads the shape only (W2 need not point anywhere) and returns <= 0 for a shape it rejects
-    probe = _lib.ActorF32(W1=None, b1=None, W2=1, b2=None, W3=None, b3=None, H1=H1, H2=H2, kind=_lib.ACTOR_TANH, reserved=0)
+    probe = _lib.ActorF32(W1=None, b1=None, W2=1, b2=None, W3=None, b3=None, H1=H1, H2=H2, kind=_lib.ACTOR_TANH)
     if _lib.load().cstr_actor_pack_bf16(byref(probe), None, None) <= 0:
         return (f"H1={H1}, H2={H2}: the tensor-core actor needs H2 rounded up to 16 plus two layer-1 K-chunks within 512 TMEM columns "
                 "(H2 <= 480) and its operand buffers within 227 KB of shared memory")
@@ -43,13 +43,19 @@ class ActorWeights:
                         ``Actor`` (core/td3/policies.py:20-83); W3 is (2,H2).
     ``kind="gaussian"`` SAC: ``tanh(mu + exp(clamp(log_std,-20,2)) * eps)`` on the trunk ``latent_pi`` with heads ``mu`` and
                         ``log_std`` (core/sac/policies.py:25-178); W3 is (4,H2) = rows [mu_0, mu_1, log_std_0, log_std_1].
+    ``kind="sde"``      SAC with gSDE (``use_sde=True``): ``tanh(hardtanh(W3 latent + b3, clip_mean) + latent @ E_i)`` with reactor i's
+                        exploration matrix ``E_i = exp(log_std) * N(0,1)`` (StateDependentNoiseDistribution, full_std, no expln,
+                        core/common/distributions.py); W3 is ``mu``'s (2,H2), ``log_std`` the (H2,2) parameter the matrices are drawn
+                        from (:meth:`FusedRollout.reset_noise`), ``clip_mean <= 0`` means no Hardtanh.
     """
 
-    def __init__(self, W1, b1, W2, b2, W3, b3, device="cuda", kind: str = "tanh"):
+    def __init__(self, W1, b1, W2, b2, W3, b3, device="cuda", kind: str = "tanh", log_std=None, clip_mean: float = 0.0):
         torch = _lib.require_cuda()
         dev = torch.device(device)
-        if kind not in ("tanh", "gaussian"):
-            raise ValueError("kind must be 'tanh' or 'gaussian'")
+        if kind not in ("tanh", "gaussian", "sde"):
+            raise ValueError("kind must be 'tanh', 'gaussian' or 'sde'")
+        if (log_std is not None) != (kind == "sde"):
+            raise ValueError("log_std (H2, 2) is given for kind='sde' and only for it")
 
         def put(x):
             return torch.as_tensor(x).detach().to(device=dev, dtype=torch.float32).contiguous()
@@ -57,17 +63,22 @@ class ActorWeights:
         self.W1, self.b1, self.W2, self.b2, self.W3, self.b3 = (put(x) for x in (W1, b1, W2, b2, W3, b3))
         self.H1, self.H2 = int(self.W1.shape[0]), int(self.W2.shape[0])
         self.kind = kind
-        n_out = 2 if kind == "tanh" else 4
+        self.log_std = put(log_std) if kind == "sde" else None
+        self.clip_mean = float(clip_mean) if kind == "sde" else 0.0
+        n_out = 4 if kind == "gaussian" else 2
         if (tuple(self.W1.shape) != (self.H1, 4) or tuple(self.W2.shape) != (self.H2, self.H1) or tuple(self.W3.shape) != (n_out, self.H2)
                 or tuple(self.b3.shape) != (n_out,)):
             raise ValueError(f"actor must be 4 -> H1 -> H2 -> {n_out}")
+        if self.log_std is not None and tuple(self.log_std.shape) != (self.H2, 2):
+            raise ValueError(f"log_std must be (H2, 2) = ({self.H2}, 2), got {tuple(self.log_std.shape)}")
         if self.H1 % 4:
             raise ValueError("H1 must be a multiple of 4")
         self.device = dev
         self.packed_bf16 = None
         self._struct = _lib.ActorF32(W1=self.W1.data_ptr(), b1=self.b1.data_ptr(), W2=self.W2.data_ptr(), b2=self.b2.data_ptr(),
                                      W3=self.W3.data_ptr(), b3=self.b3.data_ptr(), H1=self.H1, H2=self.H2,
-                                     kind=_lib.ACTOR_TANH if kind == "tanh" else _lib.ACTOR_GAUSSIAN, reserved=0)
+                                     kind={"tanh": _lib.ACTOR_TANH, "gaussian": _lib.ACTOR_GAUSSIAN, "sde": _lib.ACTOR_SDE}[kind],
+                                     clip_mean=self.clip_mean)
 
     @staticmethod
     def _linears(module):
@@ -83,14 +94,25 @@ class ActorWeights:
 
     @classmethod
     def from_sac_actor(cls, latent_pi, mu, log_std, device="cuda") -> "ActorWeights":
-        """From the reference SAC ``Actor``: ``actor.latent_pi`` (Linear, ReLU, Linear, ReLU), ``actor.mu``, ``actor.log_std``."""
+        """From the reference SAC ``Actor``: ``actor.latent_pi`` (Linear, ReLU, Linear, ReLU), ``actor.mu``, ``actor.log_std``.  With
+        gSDE (``use_sde=True``) ``log_std`` is the (H2,2) parameter and ``mu`` a Linear or ``Sequential(Linear, Hardtanh)``: the
+        result is ``kind="sde"``."""
         torch = _lib.require_cuda()
         lin = cls._linears(latent_pi)
         if len(lin) != 2:
             raise ValueError("expected a two-layer trunk")
+        if isinstance(log_std, torch.Tensor):
+            head = sde_mean_head(mu)
+            if head is None:
+                raise ValueError("the gSDE actor's mu must be a Linear or Sequential(Linear, Hardtanh(-c, c))")
+            return cls(lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias, head[0].weight, head[0].bias, device=device, kind="sde",
+                       log_std=log_std, clip_mean=head[1])
         W3 = torch.cat([mu.weight.detach(), log_std.weight.detach()], 0)
         b3 = torch.cat([mu.bias.detach(), log_std.bias.detach()], 0)
         return cls(lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias, W3, b3, device=device, kind="gaussian")
+
+    def _targets(self):
+        return (self.W1, self.b1, self.W2, self.b2, self.W3, self.b3) + ((self.log_std,) if self.kind == "sde" else ())
 
     def _sources(self, *modules):
         torch = _lib.require_cuda()
@@ -99,21 +121,25 @@ class ActorWeights:
             return [lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias, lin[2].weight, lin[2].bias]
         latent_pi, mu, log_std = modules
         lin = self._linears(latent_pi)
+        if self.kind == "sde":
+            head = sde_mean_head(mu)[0]
+            return [lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias, head.weight, head.bias, log_std]
         return [lin[0].weight, lin[0].bias, lin[1].weight, lin[1].bias, torch.cat([mu.weight.detach(), log_std.weight.detach()], 0),
                 torch.cat([mu.bias.detach(), log_std.bias.detach()], 0)]
 
     def refresh_from_module(self, *modules) -> None:
         """Copy updated parameters in place (device-to-device) after an optimiser step: ``refresh_from_module(actor.mu)``
-        for TD3, ``refresh_from_module(actor.latent_pi, actor.mu, actor.log_std)`` for SAC."""
-        for dst, src in zip((self.W1, self.b1, self.W2, self.b2, self.W3, self.b3), self._sources(*modules)):
+        for TD3, ``refresh_from_module(actor.latent_pi, actor.mu, actor.log_std)`` for SAC (with gSDE ``log_std`` too; exploration
+        matrices already drawn keep the std they were drawn with, as the reference's do)."""
+        for dst, src in zip(self._targets(), self._sources(*modules)):
             dst.copy_(src.detach(), non_blocking=True)
         if self.packed_bf16 is not None:
             self.pack_bf16()
 
     def refresh_from_tensors(self, tensors) -> None:
         """Same, from six tensors ``W1, b1, W2, b2, W3, b3`` — e.g. ``FusedTD3Update.views("params")["actor"]`` (for SAC the head is
-        already the stacked [mu; log_std] matrix)."""
-        for dst, src in zip((self.W1, self.b1, self.W2, self.b2, self.W3, self.b3), tensors):
+        already the stacked [mu; log_std] matrix); a ``kind="sde"`` actor takes ``log_std`` as a seventh."""
+        for dst, src in zip(self._targets(), tensors):
             dst.copy_(src.detach(), non_blocking=True)
         if self.packed_bf16 is not None:
             self.pack_bf16()
@@ -135,6 +161,20 @@ class ActorWeights:
             if rc < 0:
                 _lib.check(int(rc), "cstr_actor_pack_bf16")
         return self.packed_bf16
+
+
+def sde_mean_head(mu):
+    """(Linear, clip_mean) of a gSDE actor's ``mu`` — a Linear (clip_mean 0: no Hardtanh) or ``Sequential(Linear, Hardtanh(-c, c))``
+    (SAC ``Actor`` with ``clip_mean = c > 0``, core/sac/policies.py) — or None for any other module."""
+    import torch.nn as nn
+
+    if type(mu) is nn.Linear:
+        return mu, 0.0
+    if type(mu) is nn.Sequential and len(mu) == 2 and type(mu[0]) is nn.Linear and type(mu[1]) is nn.Hardtanh:
+        lo, hi = float(mu[1].min_val), float(mu[1].max_val)
+        if hi > 0.0 and lo == -hi:
+            return mu[0], hi
+    return None
 
 
 class AgentActorWeights:
@@ -164,7 +204,7 @@ class AgentActorWeights:
         self._structs = (_lib.ActorF32 * 2)()
         for i, t in enumerate(self._tensors):
             self._structs[i] = _lib.ActorF32(W1=t["W1"].data_ptr(), b1=t["b1"].data_ptr(), W2=t["W2"].data_ptr(), b2=t["b2"].data_ptr(), W3=t["W3"].data_ptr(),
-                                             b3=t["b3"].data_ptr(), H1=self.H1, H2=self.H2, kind=_lib.ACTOR_TANH, reserved=0)
+                                             b3=t["b3"].data_ptr(), H1=self.H1, H2=self.H2, kind=_lib.ACTOR_TANH)
         self.refresh_from_modules(agent_modules)
 
     def refresh_from_modules(self, agent_modules) -> None:
@@ -214,6 +254,10 @@ class FusedRollout:
     :param vec_normalize: a :class:`GpuVecNormalize` wrapping ``env``: the actor then reads normalised observations and every step advances
         the wrapper's statistics and returns on the device (``cstr_rollout_fused_norm``, one kernel launch per step); the buffer keeps the
         original observations, as the reference's ``_store_transition`` does.
+
+    A ``kind="sde"`` (gSDE) actor runs on ``actor_mode="fp32"`` without ``vec_normalize``.  Its per-reactor exploration matrices live in
+    :attr:`explore`, ``(num_envs, H2, 2)`` float32 — 2 GiB at 1,048,576 reactors and H2 = 256, the same object the reference keeps as
+    ``exploration_matrices`` — and stay fixed until the next :meth:`reset_noise`.
     """
 
     def __init__(self, env: GpuCSTRVecEnv, buffer: GpuReplayBuffer, actor: Optional[ActorWeights] = None, sigma: float = 0.1,
@@ -248,8 +292,28 @@ class FusedRollout:
             if nbytes < 0:
                 _lib.check(int(nbytes), "cstr_rollout_norm_workspace_bytes")
             self._norm_workspace = env._torch.zeros(nbytes, dtype=env._torch.uint8, device=env.device)  # zeroed once; calls leave it zeroed
+        if getattr(actor, "kind", None) == "sde" and (actor_mode != "fp32" or vec_normalize is not None):
+            raise ValueError("the gSDE actor runs on the float32 kernel (actor_mode='fp32') without vec_normalize")
+        self.explore = None  # gSDE: (num_envs, H2, 2), allocated by the first reset_noise()
+        self.sde_epoch = 0   # gSDE: Philox counter of the next reset_noise()
         if actor_mode == "tc" and actor is not None and actor.packed_bf16 is None:
             actor.pack_bf16()
+
+    def reset_noise(self) -> None:
+        """gSDE: draw every reactor's exploration matrix ``explore[i] = exp(log_std) * N(0,1)`` from the actor's current ``log_std``
+        (``cstr_sde_sample``) and advance :attr:`sde_epoch` — the reference's ``actor.reset_noise(n_envs)``.  Row i depends on the env's
+        seed, the reactor's global id and the epoch only, so a sharded run draws the rows a single-GPU run would."""
+        env, actor = self.env, self.actor
+        if getattr(actor, "kind", None) != "sde":
+            raise ValueError("reset_noise draws the exploration matrices of a kind='sde' actor")
+        torch = env._torch
+        if self.explore is None:
+            self.explore = torch.zeros((env.num_envs, actor.H2, 2), dtype=torch.float32, device=env.device)
+        with torch.cuda.device(env.device):
+            rc = self._lib.cstr_sde_sample(actor.log_std.data_ptr(), actor.H2, env.num_envs, env._params.env_offset, env._params.seed,
+                                           self.sde_epoch & 0xFFFFFFFF, self.explore.data_ptr(), env._stream())
+        _lib.check(rc, "cstr_sde_sample")
+        self.sde_epoch += 1
 
     def collect(self, K: int, warmup: bool = False, noise=None, reward_sum=None, stats: Optional[EpisodeStats] = None) -> None:
         """K env steps for every reactor; K ring rows are appended to the buffer.
@@ -280,6 +344,10 @@ class FusedRollout:
             self.t += K
             buf.advance(K)
             return
+        if getattr(self.actor, "kind", None) == "sde" and not warmup:
+            if self.explore is None:
+                raise ValueError("call reset_noise() before the gSDE actor's first collect")
+            self.actor._struct.explore = self.explore.data_ptr()
         packed = None
         if self.actor_mode == "tc" and not warmup:
             packed = self.actor.packed_bf16 if self.actor.packed_bf16 is not None else self.actor.pack_bf16()
@@ -339,8 +407,9 @@ def _leaf_types(module):
 
 
 def _actor_unsupported(actor, actor_mode: str) -> Optional[str]:
-    """Why the rollout kernels cannot evaluate this actor (the kernels are ReLU, ReLU, then a tanh or squashed-Gaussian head on a flat
-    4-value observation) — or None when they can."""
+    """Why the rollout kernels cannot evaluate this actor (the kernels are ReLU, ReLU, then a tanh, squashed-Gaussian or gSDE head on a
+    flat 4-value observation) — or None when they can."""
+    import torch
     import torch.nn as nn
 
     relu_trunk = [nn.Linear, nn.ReLU, nn.Linear, nn.ReLU]
@@ -358,7 +427,18 @@ def _actor_unsupported(actor, actor_mode: str) -> Optional[str]:
         return actor_shape_error(*shapes.pop(), "fp32")
     if type(getattr(actor, "features_extractor", None)).__name__ != "FlattenExtractor":
         return f"features extractor {type(getattr(actor, 'features_extractor', None)).__name__} (the kernels read the raw observation)"
-    if hasattr(actor, "latent_pi"):  # SAC
+    if hasattr(actor, "latent_pi") and getattr(actor, "use_sde", False):  # SAC with gSDE
+        if _leaf_types(actor.latent_pi) != relu_trunk:
+            return f"actor.latent_pi is not Linear, ReLU, Linear, ReLU: {[t.__name__ for t in _leaf_types(actor.latent_pi)]}"
+        head = sde_mean_head(getattr(actor, "mu", None))
+        if head is None:
+            return f"use_sde with an actor.mu that is not Linear or Linear + Hardtanh(-c, c): {[t.__name__ for t in _leaf_types(actor.mu)]}"
+        lin = [m for m in actor.latent_pi.modules() if type(m) is nn.Linear] + [head[0]]
+        outs = (head[0].out_features,)
+        log_std = getattr(actor, "log_std", None)
+        if not isinstance(log_std, torch.Tensor) or tuple(log_std.shape) != (head[0].in_features, 2):
+            return "use_sde with an actor.log_std that is not an (H2, 2) parameter"
+    elif hasattr(actor, "latent_pi"):  # SAC
         if _leaf_types(actor.latent_pi) != relu_trunk:
             return f"actor.latent_pi is not Linear, ReLU, Linear, ReLU: {[t.__name__ for t in _leaf_types(actor.latent_pi)]}"
         if type(getattr(actor, "mu", None)) is not nn.Linear or type(getattr(actor, "log_std", None)) is not nn.Linear:
@@ -376,11 +456,30 @@ def _actor_unsupported(actor, actor_mode: str) -> Optional[str]:
     return actor_shape_error(H1, H2, actor_mode)
 
 
+def _sde_unsupported(actor, actor_mode: str, normalized: bool) -> Optional[str]:
+    """Why the gSDE options of this model are not the ones the SDE kernel implements (StateDependentNoiseDistribution with
+    full_std=True, use_expln=False, on the float32 actor without VecNormalize) — or None."""
+    dist = getattr(actor, "action_dist", None)
+    if getattr(actor, "use_expln", getattr(dist, "use_expln", False)):
+        return "use_sde with use_expln=True (the kernel's std is exp(log_std))"
+    if not getattr(actor, "full_std", getattr(dist, "full_std", True)):
+        return "use_sde with full_std=False (the kernel draws one std per latent unit and action)"
+    if actor_mode == "tc":
+        return "use_sde with actor_mode='tc' (the gSDE actor runs on the float32 kernel)"
+    if normalized:
+        return "use_sde under GpuVecNormalize (the VecNormalize rollout has no gSDE actor)"
+    return None
+
+
 def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_noise, actor_mode: str = "fp32") -> Optional[str]:
     """Why ``cstr_rollout_fused`` can NOT stand in for this ``collect_rollouts`` call — or None when it can.  ``actor_mode`` is the
     kernel that would run the actor (``"fp32"`` or ``"tc"``; the two-agent actors always run on ``"fp32"``).  ``env`` may be a
     :class:`GpuVecNormalize` around the env when it is the model's own ``_vec_normalize_env``."""
     vec_normalize = getattr(model, "_vec_normalize_env", None)
+    if getattr(model, "use_sde", False):
+        why = _sde_unsupported(getattr(model, "actor", None), actor_mode, isinstance(env, GpuVecNormalize))
+        if why:
+            return why
     if isinstance(env, GpuVecNormalize):
         if vec_normalize is not env:
             return "the GpuVecNormalize the rollout steps through is not the model's _vec_normalize_env"
@@ -398,8 +497,6 @@ def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_nois
         return "replay buffer is not a GpuReplayBuffer on the env's device with n_envs == env.num_envs"
     if getattr(train_freq.unit, "value", train_freq.unit) != "step":
         return "train_freq counts episodes (one kernel launch collects a fixed number of steps)"
-    if getattr(model, "use_sde", False):
-        return "use_sde (state-dependent exploration matrices)"
     actor = getattr(model, "actor", None)
     if actor is not None and hasattr(actor, "mu_list"):  # multi-agent (MADDPG / IDDPG): any noise object is ignored by the reference itself (Q5)
         splits = ([list(s) for s in getattr(model, "observation_splits", [])], [list(s) for s in getattr(model, "action_splits", [])])
@@ -413,6 +510,30 @@ def fused_rollout_unsupported(model, env, replay_buffer, train_freq, action_nois
     return _actor_unsupported(actor, actor_mode)
 
 
+def launch_plan(K: int, n_envs: int, num_timesteps: int, learning_starts: int, sde_sample_freq: Optional[int] = None,
+                use_sde_at_warmup: bool = False):
+    """The kernel launches of one fused ``collect_rollouts`` call of ``K`` steps: a list of ``(steps, warmup, noise_resets)``.
+
+    A launch ends where the reference changes what ``_sample_action`` does (off_policy_algorithm.py:364-411, collect_rollouts :510-605):
+    at ``learning_starts`` (tested before every step) and, under gSDE (``sde_sample_freq`` not None), before every within-call step that
+    is a multiple of ``sde_sample_freq > 0``.  ``noise_resets`` counts the reference's ``actor.reset_noise`` calls before the launch: one
+    at the start of the call and one at every such multiple, step 0 included.  ``use_sde_at_warmup`` runs the actor during warm-up."""
+    plan, s, t = [], 0, num_timesteps
+    while s < K:
+        warm = t < learning_starts and not use_sde_at_warmup
+        k = min(K - s, -(-(learning_starts - t) // n_envs)) if warm else K - s
+        resets = 0
+        if sde_sample_freq is not None:
+            resets = int(s == 0)
+            if sde_sample_freq > 0:
+                resets += int(s % sde_sample_freq == 0)
+                k = min(k, sde_sample_freq - s % sde_sample_freq)
+        plan.append((k, warm, resets))
+        s += k
+        t += n_envs * k
+    return plan
+
+
 def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
     """Return a subclass of a reference off-policy algorithm (``core.TD3 / DDPG / SAC``, or what ``bind_td3_class`` / ``bind_sac_class``
     returned) whose ``collect_rollouts`` (core/common/off_policy_algorithm.py:510-605) is ONE ``cstr_rollout_fused`` launch per call:
@@ -420,6 +541,9 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
     ``ReplayBuffer.add`` for every reactor, with the bookkeeping the rest of ``learn()`` (:309-355) relies on kept intact:
 
     * ``num_timesteps += n_envs`` per step, the warm-up switch at ``learning_starts`` (a launch that straddles it is split there),
+    * gSDE (``use_sde=True``): ``reset_noise`` at the start of every call and, with ``sde_sample_freq > 0``, before every within-call
+      step that is a multiple of it (launches are split there, see :func:`launch_plan`); ``use_sde_at_warmup`` runs the actor during
+      warm-up;
       ``_update_current_progress_remaining``, ``_on_step``;
     * finished episodes come from the device-side Monitor (:class:`EpisodeStats`) into ``ep_info_buffer`` (``rollout/ep_rew_mean`` /
       ``ep_len_mean``), ``_episode_num`` advances by their number, ``_dump_logs`` runs when it crosses a multiple of ``log_interval``;
@@ -501,20 +625,22 @@ def bind_offpolicy_rollout(algo_base: type, actor_mode: str = "fp32") -> type:
             n_envs, K = env.num_envs, int(train_freq.frequency)
             roll = self._fused_rollout_engine(env, replay_buffer, _noise_sigma(noise) or 0.0)
             stats = self._fused_stats
+            sde = bool(getattr(self, "use_sde", False))
+            plan = launch_plan(K, n_envs, self.num_timesteps, learning_starts, int(getattr(self, "sde_sample_freq", -1)) if sde else None,
+                               sde and bool(getattr(self, "use_sde_at_warmup", False)))
             callback.on_rollout_start()
-            remaining = K
-            while remaining > 0:
-                warm = self.num_timesteps < learning_starts  # the reference tests this before every step (:386)
-                k = min(remaining, -(-(learning_starts - self.num_timesteps) // n_envs)) if warm else remaining
-                if not warm:  # the optimiser moved the weights since the last launch: refresh the kernel's copy (device to device)
+            for k, warm, resets in plan:
+                if not warm or resets:  # the optimiser moved the weights since the last launch: refresh the kernel's copy (device to device)
                     if isinstance(roll.actor, AgentActorWeights):
                         roll.actor.refresh_from_modules(self._fused_actor_modules()[1][0])
                     else:
                         roll.actor.refresh_from_module(*self._fused_actor_modules()[1])
+                if resets:  # the first of two draws at the start of a call is never used: only its epoch is spent
+                    roll.sde_epoch += resets - 1
+                    roll.reset_noise()
                 roll.collect(k, warmup=warm, stats=stats)
                 self.fused_rollout_launches += 1
                 self.num_timesteps += n_envs * k
-                remaining -= k
             num_collected_steps = K
             callback.update_locals(locals())
             if not callback.on_step():

@@ -620,7 +620,11 @@ class FusedSACUpdate(_FusedEngine):
     """SAC gradient steps on the device: one iteration of the loop body of ``SAC.train`` (``core/sac/sac.py:213-288``) per ``update()``
     through ``cstr_sac_update`` — squashed-Gaussian actor sample and log-prob, automatic entropy coefficient, soft twin-min target,
     critics, actor (backward through both critics and the tanh-Gaussian), polyak.  Same flat-block design as :class:`FusedTD3Update`;
-    the actor head is ONE (4, h2) matrix [mu; log_std], ``log_ent_coef`` lives in a slot after the three nets."""
+    the actor head is ONE (4, h2) matrix [mu; log_std], ``log_ent_coef`` lives in a slot after the three nets.
+
+    ``sde=True``: the gSDE actor (``use_sde=True`` with ``full_std=True``, ``use_expln=False``): the head slot holds ``[mu.weight (2, h2) |
+    log_std (h2, 2)]`` (see :meth:`sde_views`), ``clip_mean`` is the Hardtanh bound of the mean (<= 0: none), and every update draws one
+    exploration matrix ``exp(log_std) * eps`` from the un-rank-keyed ``seed``, so data-parallel ranks share it."""
 
     NETS = NET_NAMES
     TARGET_NETS = NET_NAMES[1:]  # SAC has no target actor
@@ -628,9 +632,11 @@ class FusedSACUpdate(_FusedEngine):
 
     def __init__(self, net_arch: Sequence[int] = (256, 256), batch_size: int = 256, device: Any = "cuda", gamma: float = 0.99, tau: float = 0.005,
                  learning_rate: float = 3e-4, target_entropy: float = -2.0, ent_coef_init: float = 1.0, target_update_interval: int = 1,
-                 betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", dp_rank: int = 0):
+                 betas=(0.9, 0.999), eps: float = 1e-8, seed: int = 0, gemm: str = "fp32", dp_rank: int = 0, sde: bool = False,
+                 clip_mean: float = 2.0):
         super().__init__(device, gamma, tau, learning_rate, 1, betas, eps, seed, gemm, dp_rank)
         self._two_hidden(net_arch)
+        self.sde, self.clip_mean = bool(sde), float(clip_mean)
         self.target_entropy, self.target_update_interval = float(target_entropy), int(target_update_interval)
         offs = (c_int64 * 20)()
         _lib.check(self._libc.cstr_sac_layout(self.h1, self.h2, offs), "cstr_sac_layout")
@@ -644,6 +650,11 @@ class FusedSACUpdate(_FusedEngine):
     def _dims(self, net: str):
         return (4, self.h1, self.h2, 4) if net == "actor" else (6, self.h1, self.h2, 1)
 
+    def sde_views(self, block: str = "params"):
+        """gSDE: (mu.weight (2, h2), log_std (h2, 2), mu.bias (2,)) as views of ``block``'s actor head slots."""
+        w, b = self.views(block)["actor"][4:6]
+        return w[0:2], w[2:4].reshape(self.h2, 2), b[0:2]
+
     @property
     def log_ent_coef(self):
         return self.params[self._ent_offset:self._ent_offset + 1]
@@ -651,17 +662,30 @@ class FusedSACUpdate(_FusedEngine):
     def _sac_config(self, batch: int) -> "_lib.SacConfig":
         return _lib.SacConfig(h1=self.h1, h2=self.h2, batch=batch, target_update_interval=self.target_update_interval, gamma=self.gamma, tau=self.tau,
                               lr=self.learning_rate, beta1=self.betas[0], beta2=self.betas[1], eps=self.eps, target_entropy=self.target_entropy,
-                              seed=self._keyed_seed(), gemm_mode=_GEMM_MODES[self.gemm])
+                              seed=self._keyed_seed(), gemm_mode=_GEMM_MODES[self.gemm], sde=int(self.sde), clip_mean=self.clip_mean,
+                              sde_seed=self.seed & (2**64 - 1))
 
     def _workspace_bytes(self, batch: int) -> int:
         return int(self._libc.cstr_sac_workspace_bytes(byref(self._sac_config(batch))))
 
     def adopt_policy(self, policy) -> None:
-        """The reference's ``SACPolicy`` (core/sac/policies.py): ``actor.latent_pi`` + ``actor.mu`` + ``actor.log_std``, twin critics."""
+        """The reference's ``SACPolicy`` (core/sac/policies.py): ``actor.latent_pi`` + ``actor.mu`` + ``actor.log_std``, twin critics.  With gSDE
+        ``mu`` is a Linear or ``Sequential(Linear, Hardtanh)`` and ``log_std`` the (h2, 2) parameter (the first of ``actor.parameters()``):
+        parameters are mapped to their slots by identity, so their Adam moments follow them whatever the optimiser's order."""
         a, v, t = policy.actor, self.views("params"), self.views("targets")
         head_w, head_b = v["actor"][4], v["actor"][5]
-        online = list(zip(v["actor"][:4], a.latent_pi.parameters())) + [(head_w[0:2], a.mu.weight), (head_w[2:4], a.log_std.weight),
-                                                                        (head_b[0:2], a.mu.bias), (head_b[2:4], a.log_std.bias)]
+        if self.sde:
+            from .rollout import sde_mean_head
+
+            lin = sde_mean_head(a.mu)
+            if lin is None or not isinstance(a.log_std, self._torch.Tensor):
+                raise ValueError("the gSDE actor needs mu = Linear or Sequential(Linear, Hardtanh(-c, c)) and an (h2, 2) log_std parameter")
+            w_mu, w_ls, b_mu = self.sde_views("params")
+            online = list(zip(v["actor"][:4], a.latent_pi.parameters())) + [(w_mu, lin[0].weight), (w_ls, a.log_std), (b_mu, lin[0].bias)]
+            head_b[2:4].zero_()
+        else:
+            online = list(zip(v["actor"][:4], a.latent_pi.parameters())) + [(head_w[0:2], a.mu.weight), (head_w[2:4], a.log_std.weight),
+                                                                            (head_b[0:2], a.mu.bias), (head_b[2:4], a.log_std.bias)]
         targets = []
         for z, q in enumerate(policy.critic.q_networks):
             online += zip(v[f"critic{z}"], q.parameters())
@@ -696,13 +720,22 @@ class FusedSACUpdate(_FusedEngine):
     def update(self, batch, eps_pi=None, eps_next=None, allreduce: Optional[Callable[[Any], None]] = None,
                gradient_step: Optional[int] = None) -> None:
         """One iteration of sac.py:213-288.  ``eps_pi`` / ``eps_next``: explicit standard-normal draws (B,2) of the two rsample() calls
-        (parity tests); default = Philox inside the kernel.  ``allreduce``: called on grads[critics .. log_ent_coef] and on grads[actor]
+        (parity tests); default = Philox inside the kernel.  gSDE engines: ``eps_pi`` is the (h2, 2) standard-normal eps of the update's
+        exploration matrix and ``eps_next`` stays None.  ``allreduce``: called on grads[critics .. log_ent_coef] and on grads[actor]
         between backward and Adam (data-parallel training: every rank ends with the gradient of the global batch).
         ``gradient_step``: the index of this step inside the current ``train()`` call — what the reference's target sync tests
         (``gradient_step % target_update_interval``, sac.py:284); None = the engine's own running count of updates."""
         obs, act, nobs, dones, rew = self._batch_f32(batch)
-        e1 = None if eps_pi is None else self._f32(eps_pi, 2)
-        e2 = None if eps_next is None else self._f32(eps_next, 2)
+        if self.sde:
+            if eps_next is not None:
+                raise ValueError("a gSDE update draws one exploration matrix: pass its (h2, 2) eps as eps_pi, eps_next=None")
+            e1 = None if eps_pi is None else self._torch.as_tensor(eps_pi).to(self.device, self._torch.float32).contiguous()
+            if e1 is not None and tuple(e1.shape) != (self.h2, 2):
+                raise ValueError(f"gSDE eps_pi must be ({self.h2}, 2)")
+            e2 = None
+        else:
+            e1 = None if eps_pi is None else self._f32(eps_pi, 2)
+            e2 = None if eps_next is None else self._f32(eps_next, 2)
         self.n_updates += 1
         self.critic_step += 1
         self.actor_step += 1
@@ -738,8 +771,31 @@ class FusedSACUpdate(_FusedEngine):
             self.update(buffer.sample(bs, env=env), allreduce=allreduce, gradient_step=g)
 
 
+def _sde_update_unsupported(actor) -> Optional[str]:
+    """Why ``cstr_sac_update``'s gSDE mode cannot train this actor — or None when it can."""
+    from .rollout import _sde_unsupported, sde_mean_head
+
+    why = _sde_unsupported(actor, "fp32", False)
+    if why:
+        return why
+    head = sde_mean_head(getattr(actor, "mu", None))
+    if head is None:
+        return "use_sde with an actor.mu that is not Linear or Linear + Hardtanh(-c, c)"
+    log_std = getattr(actor, "log_std", None)
+    if getattr(log_std, "shape", None) is None or tuple(log_std.shape) != (head[0].in_features, 2):
+        return "use_sde with an actor.log_std that is not an (H2, 2) parameter"
+    return None
+
+
+def _sde_clip_mean(actor) -> float:
+    from .rollout import sde_mean_head
+
+    return sde_mean_head(actor.mu)[1]
+
+
 def bind_sac_class(sac_base: type) -> type:
-    """Subclass of the reference's ``SAC`` (``ent_coef="auto"``, no gSDE) whose ``train()`` (core/sac/sac.py:199-296) runs on ``cstr_sac_update``."""
+    """Subclass of the reference's ``SAC`` (``ent_coef="auto"``; gSDE with ``full_std=True``, ``use_expln=False`` and ``mu`` a Linear or
+    Linear + Hardtanh) whose ``train()`` (core/sac/sac.py:199-296) runs on ``cstr_sac_update``."""
 
     class FusedSAC(sac_base):  # type: ignore[misc, valid-type]
         _fused: Optional[FusedSACUpdate] = None
@@ -747,8 +803,8 @@ def bind_sac_class(sac_base: type) -> type:
         def train(self, gradient_steps: int, batch_size: int = 64) -> None:
             why = None
             if self._fused is None:
-                why = ("use_sde" if self.use_sde else "fixed ent_coef" if self.ent_coef_optimizer is None else
-                       "n_critics != 2" if len(self.policy.critic.q_networks) != 2 else fused_update_unsupported(self))
+                why = ("fixed ent_coef" if self.ent_coef_optimizer is None else (_sde_update_unsupported(self.actor) if self.use_sde else None) or
+                       ("n_critics != 2" if len(self.policy.critic.q_networks) != 2 else fused_update_unsupported(self)))
             if why:  # the reference's torch path
                 _fallback_once(self, why)
                 return super().train(gradient_steps, batch_size)
@@ -758,7 +814,8 @@ def bind_sac_class(sac_base: type) -> type:
                 arch = self.policy.net_arch if isinstance(self.policy.net_arch, (list, tuple)) else self.policy.net_arch["pi"]
                 eng = FusedSACUpdate(arch, batch_size, self.device, self.gamma, self.tau, float(self.lr_schedule(self._current_progress_remaining)),
                                      float(self.target_entropy), float(self.log_ent_coef.detach().exp().item()), self.target_update_interval,
-                                     seed=int(self.seed or 0), dp_rank=_dist_rank())
+                                     seed=int(self.seed or 0), dp_rank=_dist_rank(), sde=bool(self.use_sde),
+                                     clip_mean=_sde_clip_mean(self.actor) if self.use_sde else 2.0)
                 eng.adopt_policy(self.policy)
                 self.log_ent_coef.data = eng.log_ent_coef  # shared storage
                 eng.import_optimizer_state(self.actor.optimizer, self.critic.optimizer, self.ent_coef_optimizer)
